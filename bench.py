@@ -16,6 +16,12 @@ value : inputs and outputs resident in HBM, CUDA events on the decoder's stream,
 e2e   : the same decode through the C-ABI call with HOST (pinned) buffers: the
         int16 PCM is copied to the device and digitalized + raster are copied back
         inside the timed region (wall clock between stream syncs, max over ranks).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's recording; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output): start_frame, height, status, low_high,
+peaks and phasing_signals (-1 padded to MAX_PEAKS per recording) whole as float64, and digitalized (the grey levels) and image (the pixels of
+every recording's image, concatenated) as float32, whole up to DUMP_SAMPLE elements, else at DUMP_SAMPLE positions
+drawn with DUMP_SEED.
 """
 from __future__ import annotations
 
@@ -36,6 +42,8 @@ METRIC = "decoded audio Msamples/s"
 UNIT = "Msamples/s"
 ALGO_BYTES_PER_SAMPLE = 7.0      # SURVEY.md §8(d): int16 in + uint8 grey out + x4 uint8 raster out @ 11025 Hz
 HBM_FALLBACK_GBS = 6650.0        # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_SAMPLE = 1 << 22            # --dump-outputs: elements kept of one large output (16 MiB as float32)
+DUMP_SEED = 12345
 
 
 def parse_args():
@@ -72,7 +80,13 @@ def parse_args():
     ap.add_argument("--total", type=int, default=4096, help="with --config: recordings in the whole job")
     ap.add_argument("--repeat", type=int, default=1,
                     help="with --segments: the synthetic recording tiled this many times (a very long recording)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy "
+                         "(see the module docstring)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.segments or args.config):
+        ap.error("--dump-outputs covers the default decode path (also with --batch / --noisy / --sample-rate)")
+    return args
 
 
 def workload_name(args) -> str:
@@ -313,6 +327,45 @@ def stage_bytes(name: str, n: int, half: bool) -> float:
             "grey_raster": n * (4 + 1 + 4.0)}.get(name, 0.0)
 
 
+def sample_index(sizes, stride: int) -> np.ndarray:
+    """Flat indices into a (len(sizes), stride) buffer whose row i holds sizes[i] valid elements: all of them when
+    they number at most DUMP_SAMPLE, else DUMP_SAMPLE positions drawn with DUMP_SEED (sorted), the same in every run
+    whose outputs have the same sizes."""
+    sizes = np.asarray(sizes, dtype=np.int64)
+    total = int(sizes.sum())
+    if total <= DUMP_SAMPLE:
+        g = np.arange(total, dtype=np.int64)
+    else:
+        g = np.sort(np.random.default_rng(DUMP_SEED).integers(0, total, DUMP_SAMPLE))
+    starts = np.cumsum(sizes) - sizes
+    row = np.searchsorted(starts, g, side="right") - 1
+    return row * stride + (g - starts[row])
+
+
+def snapshot_outputs(res) -> dict:
+    """What one decode call with device outputs handed back, copied out of buffers the next call overwrites: the
+    per-recording results whole, the grey levels and the images (the first height x width bytes of each raster row;
+    the rest of the row is not written) whole or sampled by sample_index."""
+    import torch
+    from wefax_b200 import _native as N
+    B = len(res.lpm)
+    out = {}
+    for name, buf, sizes in (("digitalized", res.digitalized, [res.n_out] * B),
+                             ("image", res.raster_flat, [int(h) * int(w) for h, w in zip(res.height, res.width)])):
+        idx = torch.from_numpy(sample_index(sizes, buf.shape[1])).to(buf.device)
+        out[name] = buf.reshape(-1).index_select(0, idx).cpu().numpy().astype(np.float32)
+    for name in ("start_frame", "height", "status", "low_high"):
+        out[name] = np.asarray(getattr(res, name), dtype=np.float64).copy()
+    # ragged per recording: padded with -1 to the MAX_PEAKS slots the decoder fills, so that the shape does not depend
+    # on the results (a recording may have no phasing lines at all)
+    for name in ("peaks", "phasing_signals"):
+        a = np.full((B, N.MAX_PEAKS), -1.0)
+        for i, r in enumerate(getattr(res, name)):
+            a[i, :len(r)] = r
+        out[name] = a
+    return out
+
+
 def run_ours(args, rank: int, world: int, local_rank: int) -> None:
     import torch
     import torch.distributed as dist
@@ -390,6 +443,7 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
     barrier()
     sampler.region(False)
     launches = dec.launch_count - launches0
+    dumped = snapshot_outputs(res) if args.dump_outputs and rank == 0 else None
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     ms_per_step = ms_total / args.steps
     value = world * n / (ms_per_step * 1e-3) / 1e6
@@ -619,6 +673,10 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
                           "start_frame_equal": bool(int(res.start_frame[0]) == int(o.get("start_frame", -1)))}
     else:
         line["cpu_baseline"] = None
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     print(json.dumps(line), file=JSON_OUT, flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -312,6 +312,41 @@ typedef struct {
 int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm, const wefax_fm_params *params,
                     const wefax_fm_out *out);
 
+/* Slant (sample-clock error) correction of the FM decode.  A recording whose sample clock is off by p ppm has lines
+ * of Ls / (1 + p * 1e-6) samples, Ls = 60 / lpm * 11025; ppm below is that p (positive: the recording's clock runs
+ * slow, lines are shorter in samples; for resampled input it is the same as at the input rate). */
+#define WEFAX_FM_SLANT_OFF 0     /* lines of exactly Ls samples: the output of the plain FM decode           */
+#define WEFAX_FM_SLANT_FIXED 1   /* lines of Ls / (1 + ppm * 1e-6) samples, line start from the phasing fold  */
+#define WEFAX_FM_SLANT_AUTO 2    /* line length and first line measured from the white line pulses          */
+
+#define WEFAX_FM_SLANT_OK 0
+#define WEFAX_FM_SLANT_NOT_FOUND 1   /* AUTO: too few pulses (or a fit outside +-max_ppm); the output is OFF's */
+
+typedef struct {
+    int mode;                 /* WEFAX_FM_SLANT_*                                                         */
+    double ppm;               /* FIXED: the clock error, |ppm| <= 2000                                    */
+    double max_ppm;           /* AUTO: largest clock error searched, in (0, 2000]                         */
+    double min_contrast;      /* AUTO: pulse minus guard bands a line must show, (0, 1]; 0 = 0.3          */
+    int min_lines;            /* AUTO: fewest lines with a pulse for a fit, >= 2; 0 = 8                   */
+} wefax_fm_slant;
+
+typedef struct {
+    double line_length;       /* samples (at 11025 Hz) per image line used for the image                  */
+    double ppm;               /* (Ls / line_length - 1) * 1e6                                             */
+    double first_line;        /* fractional sample of the first image line (line_start = its rounding)    */
+    int32_t lines_total;      /* AUTO: lines tracked in the last pass                                     */
+    int32_t lines_used;       /* AUTO: lines whose pulse entered the final fit                            */
+    double residual_rms;      /* AUTO: rms of the final fit's residuals (samples); large: the drift is not linear */
+    int32_t status;           /* WEFAX_FM_SLANT_OK or WEFAX_FM_SLANT_NOT_FOUND                            */
+} wefax_fm_slant_out;
+
+/* The FM decode with slant correction; params / out as for the plain FM decode above, which equals this call with
+ * mode WEFAX_FM_SLANT_OFF.  The image is sized for the shortest line the mode allows (FIXED: its line; AUTO:
+ * Ls / (1 + max_ppm * 1e-6)).  slant_out (HOST pointer) may be NULL. */
+int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                          const wefax_fm_params *params, const wefax_fm_slant *slant, const wefax_fm_out *out,
+                          wefax_fm_slant_out *slant_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -29,7 +29,7 @@ EXPORTED_SYMBOLS = (
     "wefax_ctx_enable_timing", "wefax_ctx_timings", "wefax_tone_scan", "wefax_decode_fm",
     "wefax_segment_envelope", "wefax_segment_histogram", "wefax_segment_quantise", "wefax_segment_sync",
     "wefax_segment_raster", "wefax_sync_pulse_scan", "wefax_segment_select_init", "wefax_segment_histogram_dev",
-    "wefax_segment_select_dev", "wefax_segment_quantise_dev",
+    "wefax_segment_select_dev", "wefax_segment_quantise_dev", "wefax_decode_fm_slant",
 )
 ABI_VERSION = 5
 
@@ -77,6 +77,22 @@ class FmParams(C.Structure):
 class FmOut(C.Structure):
     _fields_ = [("grey", C.c_void_p), ("image", C.c_void_p), ("image_capacity", C.c_longlong),
                 ("rows", C.c_void_p), ("width", C.c_void_p), ("line_start", C.c_void_p)]
+
+
+FM_SLANT_OFF, FM_SLANT_FIXED, FM_SLANT_AUTO = 0, 1, 2
+FM_SLANT_OK, FM_SLANT_NOT_FOUND = 0, 1
+FM_SLANT_MAX_PPM = 2000.0
+
+
+class FmSlant(C.Structure):
+    _fields_ = [("mode", C.c_int), ("ppm", C.c_double), ("max_ppm", C.c_double), ("min_contrast", C.c_double),
+                ("min_lines", C.c_int)]
+
+
+class FmSlantOut(C.Structure):
+    _fields_ = [("line_length", C.c_double), ("ppm", C.c_double), ("first_line", C.c_double),
+                ("lines_total", C.c_int32), ("lines_used", C.c_int32), ("residual_rms", C.c_double),
+                ("status", C.c_int32)]
 
 
 class NativeLibraryMissing(RuntimeError):
@@ -148,6 +164,9 @@ def load():
     lib.wefax_sync_pulse_scan.restype = i
     lib.wefax_decode_fm.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmParams), C.POINTER(FmOut)]
     lib.wefax_decode_fm.restype = i
+    lib.wefax_decode_fm_slant.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmParams), C.POINTER(FmSlant),
+                                          C.POINTER(FmOut), C.POINTER(FmSlantOut)]
+    lib.wefax_decode_fm_slant.restype = i
     lib.wefax_segment_envelope.argtypes = [vp, C.POINTER(BatchDesc), vp, ll, ll, ll, ll]
     lib.wefax_segment_envelope.restype = i
     lib.wefax_segment_histogram.argtypes = [vp, i, C.POINTER(C.c_uint32 * 4), vp]

@@ -311,6 +311,142 @@ bool decode_depth_first(wefax_ctx *ctx, const wefax_batch_desc *desc, const int1
     return true;
 }
 
+// ---- slant search of the FM decode (DESIGN.md §4.7a; float64 restatement: tests/fm_slant_oracle.py) ----
+
+constexpr int kSlantCoarseLines = 1024;
+
+struct SlantGeometry {
+    double Ls;
+    int wb, D, Bn, wbb, R;
+    long long L;   // whole lines in [from, image_end) at the longest allowed line
+    int Lc;        // lines of the coarse stage
+    int J;         // coarse candidates k = 2j, |j| <= J
+};
+
+SlantGeometry slant_geometry(double Ls, long long from, long long image_end, double max_ppm) {
+    SlantGeometry s;
+    s.Ls = Ls;
+    s.wb = std::max(1, (int)llround(0.05 * Ls));
+    s.D = std::max(1, (int)llround(s.wb / 16.0));
+    s.Bn = (int)ceil(Ls / s.D);
+    s.wbb = std::max(1, (int)llround((double)s.wb / s.D));
+    s.R = 5 * s.D;
+    const long long span = image_end - from;
+    s.L = span > 0 ? (long long)floor((double)span / (Ls / (1.0 - max_ppm * 1e-6))) : 0;
+    s.Lc = (int)std::min<long long>(s.L, kSlantCoarseLines);
+    const int K = (int)ceil(max_ppm * 1e-6 * Ls * s.Lc / s.D);
+    s.J = (K + 1) / 2;
+    return s;
+}
+
+struct LineFit {
+    double a = 0.0, s = 0.0, rms = 0.0;
+    int used = 0;
+};
+
+void least_squares(const std::vector<double> &l, const std::vector<double> &y, double &a, double &s) {
+    double ml = 0.0, my = 0.0;
+    for (size_t i = 0; i < l.size(); ++i) {
+        ml += l[i];
+        my += y[i];
+    }
+    ml /= (double)l.size();
+    my /= (double)l.size();
+    double sxy = 0.0, sxx = 0.0;
+    for (size_t i = 0; i < l.size(); ++i) {
+        sxy += (l[i] - ml) * (y[i] - my);
+        sxx += (l[i] - ml) * (l[i] - ml);
+    }
+    s = sxy / sxx;
+    a = my - s * ml;
+}
+
+// least squares of pulse position against line index, then twice: drop |residual| > max(1, 3 * 1.4826 * MAD), refit.
+// false: fewer than min_lines lines at some fit
+bool robust_line_fit(std::vector<double> l, std::vector<double> y, int min_lines, LineFit &fit) {
+    const size_t need = (size_t)std::max(2, min_lines);
+    if (l.size() < need) return false;
+    least_squares(l, y, fit.a, fit.s);
+    for (int pass = 0; pass < 2; ++pass) {
+        std::vector<double> r(l.size());
+        for (size_t i = 0; i < l.size(); ++i) r[i] = fabs(y[i] - (fit.a + fit.s * l[i]));
+        std::vector<double> sorted = r;
+        std::sort(sorted.begin(), sorted.end());
+        const size_t m = sorted.size();
+        const double mad = (m & 1) ? sorted[m / 2] : 0.5 * (sorted[m / 2 - 1] + sorted[m / 2]);
+        const double thr = std::max(1.0, 3.0 * 1.4826 * mad);
+        size_t k = 0;
+        for (size_t i = 0; i < l.size(); ++i)
+            if (r[i] <= thr) {
+                l[k] = l[i];
+                y[k] = y[i];
+                ++k;
+            }
+        l.resize(k);
+        y.resize(k);
+        if (k < need) return false;
+        least_squares(l, y, fit.a, fit.s);
+    }
+    double ss = 0.0;
+    for (size_t i = 0; i < l.size(); ++i) {
+        const double r = y[i] - (fit.a + fit.s * l[i]);
+        ss += r * r;
+    }
+    fit.used = (int)l.size();
+    fit.rms = sqrt(ss / (double)l.size());
+    return true;
+}
+
+// AUTO slant: coarse sheared fold of the first Lc lines, per-line pulse tracking, robust line fit (twice: Lc lines,
+// then all L lines from the first fit).  Fills res (status WEFAX_FM_SLANT_NOT_FOUND when too few pulses are found or
+// the fit leaves +-max_ppm); synchronises the context's stream.
+void slant_search(wefax_ctx *ctx, const float *g, long long n, long long from, const SlantGeometry &sg,
+                  const wefax_fm_slant &prm, wefax_fm_slant_out &res) {
+    res.status = WEFAX_FM_SLANT_NOT_FOUND;
+    res.lines_total = (int)std::min<long long>(sg.L, INT32_MAX);
+    if (sg.L < std::max(2, prm.min_lines) || sg.L > INT32_MAX) return;
+    cudaStream_t st = ctx->stream;
+    const int L = (int)sg.L;
+    const size_t q_bytes = ((size_t)sg.Lc * sg.Bn * sizeof(float) + 255) / 256 * 256;
+    char *scratch = (char *)ctx->work_misc.reserve(q_bytes + 256 + (size_t)L * (sizeof(long long) + sizeof(float)));
+    float *Q = (float *)scratch;
+    unsigned long long *d_best = (unsigned long long *)(scratch + q_bytes);
+    long long *d_pos = (long long *)(scratch + q_bytes + 256);
+    float *d_ctr = (float *)(d_pos + L);
+    launch_fm_slant_profile(ctx, g, n, from, sg.Ls, sg.D, sg.Bn, sg.Lc, Q);
+    launch_fm_slant_fold(ctx, Q, sg.Lc, sg.Bn, sg.wbb, 2 * sg.J + 1, d_best);
+    long long *h = (long long *)pinned(ctx, (size_t)L * sizeof(long long) + 64);
+    CUDA_CHECK(cudaMemcpyAsync(h, d_best, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    const int rank = 0x7fffffff - (int)(unsigned)((unsigned long long)h[0] & 0xffffffffull);
+    const int c = rank / sg.Bn, b = rank % sg.Bn;
+    const int k = c == 0 ? 0 : ((c + 1) / 2) * 2 * ((c & 1) ? -1 : 1);
+    double a = (double)(from + (long long)b * sg.D), s = sg.Ls + (double)k * sg.D / sg.Lc;
+    LineFit fit;
+    for (int lines : {sg.Lc, L}) {
+        launch_fm_slant_track(ctx, g, n, a, s, lines, sg.wb, sg.R, prm.min_contrast, d_pos, d_ctr);
+        CUDA_CHECK(cudaMemcpyAsync(h, d_pos, (size_t)lines * sizeof(long long), cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        std::vector<double> li, yi;
+        for (int i = 0; i < lines; ++i)
+            if (h[i] >= 0) {
+                li.push_back((double)i);
+                yi.push_back((double)h[i]);
+            }
+        if (!robust_line_fit(std::move(li), std::move(yi), prm.min_lines, fit)) return;
+        a = fit.a;
+        s = fit.s;
+    }
+    const double ppm = (sg.Ls / s - 1.0) * 1e6;
+    if (!(fabs(ppm) <= prm.max_ppm)) return;
+    res.status = WEFAX_FM_SLANT_OK;
+    res.line_length = s;
+    res.ppm = ppm;
+    res.first_line = a - floor((a - (double)from) / s) * s;
+    res.lines_used = fit.used;
+    res.residual_rms = fit.rms;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1356,13 +1492,34 @@ int wefax_sync_pulse_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames
 
 int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm, const wefax_fm_params *prm,
                     const wefax_fm_out *out) {
+    wefax_fm_slant off;
+    memset(&off, 0, sizeof(off));
+    off.mode = WEFAX_FM_SLANT_OFF;
+    return wefax_decode_fm_slant(ctx, desc, pcm, prm, &off, out, nullptr);
+}
+
+int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm, const wefax_fm_params *prm,
+                          const wefax_fm_slant *slant, const wefax_fm_out *out, wefax_fm_slant_out *slant_out) {
     if (!ctx) return WEFAX_ERR_INVALID;
     return guarded(ctx, [&] {
-        if (!desc || !pcm || !prm || !out || desc->n_recordings != 1 || desc->n_frames < 64 ||
+        if (!desc || !pcm || !prm || !slant || !out || desc->n_recordings != 1 || desc->n_frames < 64 ||
             (desc->channels != 1 && desc->channels != 2) || desc->sample_rate < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
         if (!(prm->lpm > 0.0) || prm->ioc < 1 || !(prm->white_hz > prm->black_hz) || prm->fold_lines < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
+        wefax_fm_slant sp = *slant;
+        if (sp.mode == WEFAX_FM_SLANT_FIXED) {
+            if (!(fabs(sp.ppm) <= 2000.0)) WEFAX_THROW(WEFAX_ERR_INVALID, "slant ppm must be within +-2000");
+        } else if (sp.mode == WEFAX_FM_SLANT_AUTO) {
+            if (sp.min_contrast == 0.0) sp.min_contrast = 0.3;
+            if (sp.min_lines == 0) sp.min_lines = 8;
+            if (!(sp.max_ppm > 0.0 && sp.max_ppm <= 2000.0))
+                WEFAX_THROW(WEFAX_ERR_INVALID, "max_ppm must be in (0, 2000]");
+            if (!(sp.min_contrast > 0.0 && sp.min_contrast <= 1.0) || sp.min_lines < 2)
+                WEFAX_THROW(WEFAX_ERR_INVALID, "min_contrast must be in (0, 1] and min_lines >= 2");
+        } else if (sp.mode != WEFAX_FM_SLANT_OFF) {
+            WEFAX_THROW(WEFAX_ERR_INVALID, "unknown slant mode %d", sp.mode);
+        }
         use_device(ctx);
         cudaStream_t st = ctx->stream;
         const long long n_in = desc->n_frames;
@@ -1375,7 +1532,10 @@ int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t 
         const int W = (int)llround(M_PI * (double)prm->ioc);
         const long long image_end = (prm->image_end > 0 && prm->image_end <= n) ? prm->image_end : n;
         const long long from = std::max<long long>(0, std::min<long long>(prm->search_from, n - 1));
-        const int rows_max = (int)std::max<long long>(0, (long long)floor((double)(image_end - from) / Ls));
+        // the line length FIXED uses, and the shortest one AUTO may find: it sizes the image
+        const double Ls_fixed = sp.mode == WEFAX_FM_SLANT_FIXED ? Ls / (1.0 + sp.ppm * 1e-6) : Ls;
+        const double Ls_min = sp.mode == WEFAX_FM_SLANT_AUTO ? Ls / (1.0 + sp.max_ppm * 1e-6) : Ls_fixed;
+        const int rows_max = (int)std::max<long long>(0, (long long)floor((double)(image_end - from) / Ls_min));
         if (out->image && (long long)rows_max * W > out->image_capacity)
             WEFAX_THROW(WEFAX_ERR_INVALID, "image_capacity %lld too small (need %lld)", out->image_capacity,
                         (long long)rows_max * W);
@@ -1412,15 +1572,32 @@ int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t 
         // grey stream (in the transform scratch, or straight into the caller's device buffer)
         float *g = (out_dev && out->grey) ? out->grey : (float *)ctx->work_z.reserve((size_t)n * sizeof(float));
         launch_fm_grey(ctx, x, y, g, n, prm->black_hz, prm->white_hz);
-        const int Lc = (int)ceil(Ls);
+        const int Lc = (int)ceil(Ls_fixed);
         char *small = (char *)ctx->out_small.reserve((size_t)Lc * sizeof(float) + 64);
         long long *d_ls = (long long *)small;
         float *P = (float *)(small + 64);
-        launch_fm_phasing(ctx, g, n, from, Ls, prm->fold_lines, P, d_ls);
+
+        wefax_fm_slant_out so;
+        memset(&so, 0, sizeof(so));
+        so.status = WEFAX_FM_SLANT_OK;
+        double line_length = Ls_fixed;
+        bool fitted = false;
+        if (sp.mode == WEFAX_FM_SLANT_AUTO) {
+            slant_search(ctx, g, n, from, slant_geometry(Ls, from, image_end, sp.max_ppm), sp, so);
+            if (so.status == WEFAX_FM_SLANT_OK) {
+                const long long ls = llround(so.first_line);
+                CUDA_CHECK(cudaMemcpyAsync(d_ls, &ls, sizeof(long long), cudaMemcpyHostToDevice, st));
+                line_length = so.line_length;
+                fitted = true;
+            }
+        } else if (sp.mode == WEFAX_FM_SLANT_FIXED) {
+            so.ppm = sp.ppm;
+        }
+        if (!fitted) launch_fm_phasing(ctx, g, n, from, line_length, prm->fold_lines, P, d_ls);
         uint8_t *d_img = nullptr;
         if (out->image && rows_max > 0) {
             d_img = out_dev ? out->image : (uint8_t *)ctx->out_raster.reserve((size_t)rows_max * W);
-            launch_fm_image(ctx, g, n, d_ls, Ls, W, rows_max, image_end, d_img);
+            launch_fm_image(ctx, g, n, d_ls, line_length, W, rows_max, image_end, d_img);
         }
         long long *h_ls = (long long *)pinned(ctx, 64);
         CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, sizeof(long long), cudaMemcpyDeviceToHost, st));
@@ -1428,12 +1605,20 @@ int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t 
             CUDA_CHECK(cudaMemcpyAsync(out->grey, g, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaStreamSynchronize(st));
         const long long line_start = *h_ls;
-        const int rows = (int)std::max<long long>(0, (long long)floor((double)(image_end - line_start) / Ls));
+        const int rows = (int)std::min<long long>(
+            rows_max, std::max<long long>(0, (long long)floor((double)(image_end - line_start) / line_length)));
         if (!out_dev && d_img && rows > 0)
             CUDA_CHECK(cudaMemcpy(out->image, d_img, (size_t)rows * W, cudaMemcpyDeviceToHost));
         if (out->rows) *out->rows = rows;
         if (out->width) *out->width = W;
         if (out->line_start) *out->line_start = line_start;
+        if (slant_out) {
+            if (!fitted) {
+                so.line_length = line_length;
+                so.first_line = (double)line_start;
+            }
+            *slant_out = so;
+        }
     });
 }
 

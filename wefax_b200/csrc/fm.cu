@@ -16,6 +16,8 @@
 //                white pulse, arg max = line start (block-wide reduction)
 //   image        pixel (row, col) = box average of grey over its exact fractional sample span,
 //                one thread per pixel: demod -> grey map -> line resample in one pass over x, y
+//   slant        (optional) the recording's true line length from the white line pulses: sheared folds of a
+//                binned profile, per-line pulse tracking, a line fit on the host (api.cu; DESIGN.md §4.7a)
 #include <cmath>
 #include <vector>
 
@@ -152,6 +154,131 @@ fm_image_kernel(const float *g, long long n, const long long *line_start, double
     img[(size_t)r * W + p] = (uint8_t)fminf(fmaxf(v, 0.f), 255.f);
 }
 
+// ---- slant: the sample-clock error measured from the white line pulses (DESIGN.md §4.7a) ----
+
+// Q[l][b] = mean of clip(grey) over [from + floor(l * Ls) + b * D, +D); samples at or past n count as 0.  One CTA per line.
+__global__ void __launch_bounds__(256)
+fm_slant_profile_kernel(const float *g, long long n, long long from, double Ls, int D, int Bn, float *Q) {
+    const int l = blockIdx.x;
+    const long long base = from + (long long)floor((double)l * Ls);
+    for (int b = threadIdx.x; b < Bn; b += blockDim.x) {
+        const long long i0 = base + (long long)b * D;
+        float acc = 0.f;
+        for (int j = 0; j < D; ++j)
+            if (i0 + j < n) acc += clip01(__ldg(g + i0 + j));
+        Q[(size_t)l * Bn + b] = acc / (float)D;
+    }
+}
+
+__device__ __forceinline__ int floor_div(int a, int b) { return a / b - ((a % b != 0) && ((a < 0) != (b < 0))); }
+
+// One CTA per candidate c of the total shift k over `lines` lines (c = 0, 1, 2, 3, 4, ... -> k = 0, -2, +2, -4, +4, ...):
+// S_k[b] = sum_l Q[l][(b + round(l * k / lines)) mod Bn], circular boxcar of wbb bins, arg max over (c, b) into *best as
+// (score bits << 32) | (0x7fffffff - (c * Bn + b)): the highest score wins, then the smallest |k|, then the smallest b.
+__global__ void __launch_bounds__(1024)
+fm_slant_fold_kernel(const float *Q, int lines, int Bn, int wbb, unsigned long long *best) {
+    extern __shared__ float S[];
+    __shared__ unsigned long long s_best[32];
+    const int c = blockIdx.x, tid = threadIdx.x;
+    const int k = c == 0 ? 0 : ((c + 1) / 2) * 2 * ((c & 1) ? -1 : 1);
+    for (int b = tid; b < Bn; b += blockDim.x) {
+        float acc = 0.f;
+        for (int l = 0; l < lines; ++l) {
+            const int sh = floor_div(2 * l * k + lines, 2 * lines);
+            const int col = ((b + sh) % Bn + Bn) % Bn;
+            acc += __ldg(Q + (size_t)l * Bn + col);
+        }
+        S[b] = acc;
+    }
+    __syncthreads();
+    unsigned long long key = 0ull;
+    for (int b = tid; b < Bn; b += blockDim.x) {
+        float score = 0.f;
+        for (int j = 0; j < wbb; ++j) score += S[(b + j) % Bn];
+        const unsigned long long kb = ((unsigned long long)__float_as_uint(fmaxf(score, 0.f)) << 32) |
+                                      (unsigned)(0x7fffffff - (c * Bn + b));
+        key = kb > key ? kb : key;
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, d);
+        key = other > key ? other : key;
+    }
+    if ((tid & 31) == 0) s_best[tid >> 5] = key;
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < (int)(blockDim.x + 31) / 32; ++w) key = s_best[w] > key ? s_best[w] : key;
+        atomicMax(best, key);
+    }
+}
+
+// One warp per line l < lines: the pulse is the arg max over x in [c - R, c + R], c = floor(a + l * s + 0.5), of the
+// width-wb boxcar of clip(grey) (smallest x on ties); contrast = boxcar mean - mean of the guard bands [x - wb, x) and
+// [x + wb, x + 2 wb).  pos[l] = x when the contrast reaches min_contrast, else -1 (also when the window leaves the
+// recording).  Boxcars from float64 prefix sums of the window in shared memory.
+__global__ void __launch_bounds__(32)
+fm_slant_track_kernel(const float *g, long long n, double a, double s, int wb, int R, double min_contrast,
+                      long long *pos, float *contrast) {
+    extern __shared__ double pre[];    // pre[i] = sum_{j < i} clip(g[lo + j]), i <= span
+    const int l = blockIdx.x, lane = threadIdx.x;
+    const long long c = (long long)floor(a + (double)l * s + 0.5);
+    const long long lo = c - R - wb;
+    const int span = 2 * R + 3 * wb;
+    if (lo < 0 || lo + span > n) {
+        if (lane == 0) {
+            pos[l] = -1;
+            contrast[l] = 0.f;
+        }
+        return;
+    }
+    for (int i = lane; i < span; i += 32) pre[i + 1] = (double)clip01(__ldg(g + lo + i));
+    if (lane == 0) pre[0] = 0.0;
+    __syncwarp();
+    // in-place scan: each lane sums a contiguous chunk, the lanes scan their totals with shuffles
+    const int chunk = (span + 31) / 32, b = 1 + lane * chunk, e = min(b + chunk, span + 1);
+    double sum = 0.0;
+    for (int i = b; i < e; ++i) sum += pre[i];
+    double incl = sum;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const double v = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += v;
+    }
+    double run = incl - sum;
+    __syncwarp();
+    for (int i = b; i < e; ++i) {
+        run += pre[i];
+        pre[i] = run;
+    }
+    __syncwarp();
+    // x = c - R + t  <->  pre index u = t + wb
+    double best = -1.0;
+    int bt = 0;
+    for (int t = lane; t <= 2 * R; t += 32) {
+        const double box = pre[t + 2 * wb] - pre[t + wb];
+        if (box > best) {
+            best = box;
+            bt = t;
+        }
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        const double ob = __shfl_xor_sync(0xffffffffu, best, d);
+        const int ot = __shfl_xor_sync(0xffffffffu, bt, d);
+        if (ob > best || (ob == best && ot < bt)) {
+            best = ob;
+            bt = ot;
+        }
+    }
+    if (lane == 0) {
+        const int u = bt + wb;
+        const double guard = (pre[u] - pre[u - wb]) + (pre[u + 2 * wb] - pre[u + wb]);
+        const double ctr = best / wb - guard / (2.0 * wb);
+        pos[l] = ctr >= min_contrast ? c - R + bt : -1;
+        contrast[l] = (float)ctr;
+    }
+}
+
 void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, float *g, long long n, double black_hz,
                     double white_hz) {
     StageTimer timer(ctx, "fm_grey");
@@ -186,6 +313,37 @@ void launch_fm_image(wefax_ctx *ctx, const float *g, long long n, const long lon
     StageTimer timer(ctx, "fm_image");
     dim3 grid((W + 255) / 256, rows_max);
     fm_image_kernel<<<grid, 256, 0, ctx->stream>>>(g, n, d_line_start, Ls, W, image_end, img);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+}
+
+void launch_fm_slant_profile(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int D, int Bn,
+                             int lines, float *Q) {
+    StageTimer timer(ctx, "fm_slant_profile");
+    fm_slant_profile_kernel<<<lines, 256, 0, ctx->stream>>>(g, n, from, Ls, D, Bn, Q);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+}
+
+void launch_fm_slant_fold(wefax_ctx *ctx, const float *Q, int lines, int Bn, int wbb, int n_cand,
+                          unsigned long long *d_best) {
+    StageTimer timer(ctx, "fm_slant_fold");
+    if (Bn > 8192 || (long long)n_cand * Bn > 0x7fffffffLL)
+        WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "slant search of %d bins x %d candidates is too large", Bn, n_cand);
+    const int threads = std::min(1024, (Bn + 31) / 32 * 32);
+    CUDA_CHECK(cudaMemsetAsync(d_best, 0, sizeof(unsigned long long), ctx->stream));
+    fm_slant_fold_kernel<<<n_cand, threads, (size_t)Bn * sizeof(float), ctx->stream>>>(Q, lines, Bn, wbb, d_best);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+}
+
+void launch_fm_slant_track(wefax_ctx *ctx, const float *g, long long n, double a, double s, int lines, int wb, int R,
+                           double min_contrast, long long *pos, float *contrast) {
+    if (lines <= 0) return;
+    StageTimer timer(ctx, "fm_slant_track");
+    const size_t smem = (size_t)(2 * R + 3 * wb + 1) * sizeof(double);
+    if (smem > 48 * 1024) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "line pulse of %d samples is too long for the slant search", wb);
+    fm_slant_track_kernel<<<lines, 32, smem, ctx->stream>>>(g, n, a, s, wb, R, min_contrast, pos, contrast);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }

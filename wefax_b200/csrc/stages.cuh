@@ -145,5 +145,14 @@ void launch_fm_phasing(wefax_ctx *ctx, const float *g, long long n, long long fr
                        long long *d_line_start);
 void launch_fm_image(wefax_ctx *ctx, const float *g, long long n, const long long *d_line_start, double Ls, int W,
                      int rows_max, long long image_end, uint8_t *img);
+// slant search (DESIGN.md §4.7a): Q = lines x Bn bin means of D samples from `from` on lines of Ls samples
+void launch_fm_slant_profile(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int D, int Bn,
+                             int lines, float *Q);
+// sheared folds of Q for n_cand candidate total shifts, best (score, candidate, bin) key into d_best (device)
+void launch_fm_slant_fold(wefax_ctx *ctx, const float *Q, int lines, int Bn, int wbb, int n_cand,
+                          unsigned long long *d_best);
+// pulse position (or -1) and contrast of lines [0, lines) around a + l * s, +-R samples, pulse width wb
+void launch_fm_slant_track(wefax_ctx *ctx, const float *g, long long n, double a, double s, int lines, int wb, int R,
+                           double min_contrast, long long *pos, float *contrast);
 
 }  // namespace wefax

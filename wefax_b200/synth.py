@@ -7,7 +7,7 @@ sum of f, amplitude is 0.25 of full scale.  A transmission is
 
     5 s start tone (black/white alternating at 300 Hz for IOC576, 675 Hz for IOC288)
     n_phasing lines: 5 % white, 95 % black
-    image lines:     5 % white, then seeded block-constant greys
+    image lines:     5 % white, then seeded block-constant greys (no white part with line_pulse=False)
     5 s stop tone (450 Hz alternation)
     10 s black
 
@@ -41,8 +41,11 @@ def synth_recording(duration_s: float,
                     drift_ppm: float = 0.0,
                     block: int = 8,
                     amplitude: float = 0.25,
-                    return_grey: bool = False):
-    """One synthetic transmission, ``int(round(duration_s*sample_rate))`` int16 samples."""
+                    return_grey: bool = False,
+                    line_pulse: bool = True):
+    """One synthetic transmission, ``int(round(duration_s*sample_rate))`` int16 samples.
+
+    ``line_pulse=False``: image lines carry no white pulse, only the phasing lines do (as on most real charts)."""
     n = int(round(duration_s * sample_rate))
     rng = np.random.default_rng(seed)
     t = np.arange(n, dtype=np.float64) / sample_rate
@@ -82,7 +85,7 @@ def synth_recording(duration_s: float,
         nblk = idx.size // block + 1
         levels = rng.integers(0, 256, size=nblk).astype(np.float64) / 255.0
         content = np.repeat(levels, block)[: idx.size]
-        grey[idx] = np.where(frac < 0.05, 1.0, content)
+        grey[idx] = np.where(frac < 0.05, 1.0, content) if line_pulse else content
 
     m = (t >= t_stop0) & (t < t_black0)
     grey[m] = (np.floor(2.0 * 450.0 * (t[m] - t_stop0)) % 2 == 0).astype(np.float64)

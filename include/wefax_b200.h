@@ -56,7 +56,7 @@ typedef enum {
 #define WEFAX_F_OUT_ON_DEVICE 2u   /* every non-NULL output points to device mem  */
 #define WEFAX_F_PCM_FLOAT32 4u     /* wefax_decode_batch only: pcm points to float32 mono samples (WAV sample formats
                                       other than 16-bit PCM, converted by the caller as scipy.io.wavfile.read would
-                                      deliver them, wefax.py:349); channels must be 1                              */
+                                      deliver them, wefax.py:349); channels must be 1.  The FM decode rejects it.  */
 
 /* ---- context -------------------------------------------------------------- */
 
@@ -308,7 +308,9 @@ typedef struct {
 } wefax_fm_out;
 
 /* One recording (desc->n_recordings must be 1); desc->flags as for wefax_decode_batch (grey / image
- * follow WEFAX_F_OUT_ON_DEVICE).  desc->notch_* are ignored. */
+ * follow WEFAX_F_OUT_ON_DEVICE), except that pcm is always int16: WEFAX_F_PCM_FLOAT32 is rejected
+ * (WEFAX_ERR_INVALID).  desc->notch_* are ignored.  The image has floor((image_end - line_start) / line
+ * length) rows, computed in float64 without contraction, and every one of them is written. */
 int wefax_decode_fm(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm, const wefax_fm_params *params,
                     const wefax_fm_out *out);
 

@@ -8,15 +8,55 @@ truth of the synthetic generator.
 
 Definition:  x = zero-phase FIR band-pass of the samples (taps applied forwards and backwards
 with the edge treatment of the notch kernel: odd extension by 9, steady-state constants),
-z = x + i*Hilbert(x), grey[i] = (arg(z[i] conj z[i-1]) * sr / 2pi - black) / (white - black),
-line start = search_from + argmax_o boxcar_{5 % of a line}(sum over lines of clip(grey) folded at
-the exact line length), pixel = box average of clip(grey) over its exact sample span.
+z = x + i*Hilbert(x) where the transform runs on x zero-padded to npad = 2 * next_smooth_length(
+(n + 1) / 2) samples and the first n are kept, grey[i] = (arg(z[i] conj z[i-1]) * sr / 2pi - black) /
+(white - black) with grey[0] repeating the first step, line start = search_from + argmax_o
+boxcar_{5 % of a line}(sum over lines l of clip(grey[search_from + floor(l * Ls + o)]), l * Ls and the
+sum each rounded to float64), rows = floor((image_end - line_start) / Ls) in float64, pixel = box
+average of clip(grey) over its exact sample span.
 """
 from __future__ import annotations
 
 import numpy as np
 
 TARGET_RATE = 11025
+
+
+def next_smooth_length(m: int) -> int:
+    """The smallest 2^a 3^b 5^c 7^d >= m that the library's transform can plan (csrc/fft_plan.cu:
+    next_smooth_length): for every odd part 3^b 5^c 7^d < 2m, the least power-of-two multiple >= m.
+    -1 when none can be planned.  The planning test is the library's own (host only, no device)."""
+    from wefax_b200 import _native as N
+
+    def can_plan(v: int) -> bool:
+        try:
+            return N.fft_plan_describe(v)[1] == 0
+        except ValueError:
+            return False
+
+    cands = set()
+    p7 = 1
+    while p7 < 2 * m:
+        p5 = p7
+        while p5 < 2 * m:
+            p3 = p5
+            while p3 < 2 * m:
+                v = p3
+                while v < m:
+                    v *= 2
+                cands.add(v)
+                p3 *= 3
+            p5 *= 5
+        p7 *= 7
+    for v in sorted(cands):
+        if can_plan(v):
+            return v
+    return -1
+
+
+def transform_length(n: int) -> int:
+    """npad: the even length the FM decode's Hilbert transform runs on (csrc/api.cu, wefax_decode_fm_slant)."""
+    return 2 * next_smooth_length((n + 1) // 2)
 
 
 def bandpass_taps(lo_hz: float, hi_hz: float, fs: float, taps: int) -> np.ndarray:
@@ -62,10 +102,25 @@ def hilbert_imag(x: np.ndarray) -> np.ndarray:
     return np.fft.ifft(X * hmask).imag
 
 
-def grey_stream(pcm: np.ndarray, lo_hz=1200.0, hi_hz=2600.0, taps=63, black_hz=1500.0, white_hz=2300.0):
+def analytic(pcm: np.ndarray, lo_hz=1200.0, hi_hz=2600.0, taps=63, padded: bool = True) -> np.ndarray:
+    """z = x + i Hilbert(x) of the band-passed mono samples at 11025 Hz.  ``padded`` takes the transform
+    at the decoder's zero-padded length (transform_length) and keeps the first n; False takes it at n."""
     x = fir_filtfilt(bandpass_taps(lo_hz, hi_hz, TARGET_RATE, taps), pcm)
-    y = hilbert_imag(x)
-    z = x + 1j * y
+    n = x.shape[0]
+    if padded:
+        y = hilbert_imag(np.concatenate([x, np.zeros(transform_length(n) - n)]))[:n]
+    else:
+        y = hilbert_imag(x)
+    return x + 1j * y
+
+
+def grey_stream(pcm: np.ndarray, lo_hz=1200.0, hi_hz=2600.0, taps=63, black_hz=1500.0, white_hz=2300.0,
+                padded: bool = True):
+    """Per-sample grey of mono samples at 11025 Hz (``padded`` as for analytic())."""
+    return grey_of(analytic(pcm, lo_hz, hi_hz, taps, padded), black_hz, white_hz)
+
+
+def grey_of(z: np.ndarray, black_hz=1500.0, white_hz=2300.0) -> np.ndarray:
     step = z[1:] * np.conj(z[:-1])
     d = np.angle(step)
     d = np.concatenate([d[:1], d])
@@ -73,28 +128,42 @@ def grey_stream(pcm: np.ndarray, lo_hz=1200.0, hi_hz=2600.0, taps=63, black_hz=1
     return (f - black_hz) / (white_hz - black_hz)
 
 
-def line_start(grey: np.ndarray, search_from: int, lpm: float, fold_lines: int) -> int:
-    Ls = 60.0 / lpm * TARGET_RATE
+def _line_length(lpm, line_length):
+    return 60.0 / lpm * TARGET_RATE if line_length is None else float(line_length)
+
+
+def phasing_scores(grey: np.ndarray, search_from: int, lpm: float | None, fold_lines: int,
+                   line_length: float | None = None) -> np.ndarray:
+    """The phasing search's score for every offset o < ceil(Ls) (float32, as the device keeps it)."""
+    Ls = _line_length(lpm, line_length)
     Lc = int(np.ceil(Ls))
     wb = max(1, int(round(0.05 * Ls)))
     g = np.clip(grey, 0.0, 1.0).astype(np.float32)
     P = np.zeros(Lc, dtype=np.float32)
     o = np.arange(Lc)
     for l in range(fold_lines):
-        idx = search_from + np.floor(l * Ls + o).astype(np.int64)
+        idx = search_from + np.floor(l * Ls + o).astype(np.int64)    # l * Ls rounded, then + o rounded
         ok = idx < g.shape[0]
         P[ok] += g[idx[ok]]
     pre = np.concatenate([[0.0], np.cumsum(np.concatenate([P, P]).astype(np.float64))])
-    score = (pre[o + wb] - pre[o]).astype(np.float32)
+    return (pre[o + wb] - pre[o]).astype(np.float32)
+
+
+def line_start(grey: np.ndarray, search_from: int, lpm: float | None, fold_lines: int,
+               line_length: float | None = None) -> int:
+    """Phasing-pulse line start; lines of ``line_length`` samples when given, else of 60 / lpm s."""
+    score = phasing_scores(grey, search_from, lpm, fold_lines, line_length)
     return search_from + int(np.argmax(score))          # first maximum = smallest offset on ties
 
 
-def image(grey: np.ndarray, start: int, lpm: float, ioc: int, image_end: int | None = None) -> np.ndarray:
-    Ls = 60.0 / lpm * TARGET_RATE
+def image(grey: np.ndarray, start: int, lpm: float | None, ioc: int, image_end: int | None = None,
+          line_length: float | None = None) -> np.ndarray:
+    """The picture from ``start``; lines of ``line_length`` samples when given, else of 60 / lpm s."""
+    Ls = _line_length(lpm, line_length)
     W = int(round(np.pi * ioc))
     end = grey.shape[0] if image_end is None else image_end
     rows = max(0, int(np.floor((end - start) / Ls)))
-    g = np.clip(grey, 0.0, 1.0)
+    g = np.clip(np.asarray(grey, dtype=np.float64), 0.0, 1.0)     # float64 sums also for the decoder's float32 grey
     cs = np.concatenate([[0.0], np.cumsum(g)])           # integral of the piecewise-constant grey
     n = g.shape[0]
 

@@ -13,9 +13,9 @@ TARGET_RATE = F.TARGET_RATE
 
 
 def image(grey: np.ndarray, start: float, line_length: float, ioc: int, image_end: int | None = None) -> np.ndarray:
-    """oracle/fm_oracle.py image() with lines of `line_length` samples instead of 60 / lpm s (the round trip through
-    lpm changes the line length by an ulp at most)."""
-    return F.image(grey, start, 60.0 * TARGET_RATE / line_length, ioc, image_end)
+    """oracle/fm_oracle.py image() with lines of exactly `line_length` samples (not a round trip through lpm, which
+    can move the line length by an ulp, and an ulp can decide the row count)."""
+    return F.image(grey, start, None, ioc, image_end, line_length=line_length)
 
 
 SLANT_OK, SLANT_NOT_FOUND = 0, 1

@@ -3,7 +3,11 @@
 There is NO reference parity for this mode (the reference only describes it, README.md:85-101).
 Two checks instead:
   * CUDA (fp32) against oracle/fm_oracle.py (numpy float64 of the same definition): per-sample grey
-    within 2e-3 of the 0..1 range, line start within +-1 sample, >= 99.9 % of pixels within +-1;
+    within 2e-3 of the 0..1 range away from the ends, line start within +-1 sample, >= 99.9 % of pixels within +-1.
+    The definition (DESIGN.md §4.7): the Hilbert transform runs on the samples zero-padded to
+    npad = 2 * next_smooth_length((n + 1) / 2); the fold reads sample search_from + floor(l * Ls + o), with l * Ls
+    and the sum each rounded; the image has floor((image_end - line_start) / Ls) rows, every one written.
+    tests/test_gpu_fm_stages.py holds each stage to it on identical input, ends included;
   * both against the GROUND TRUTH of the synthetic generator (the grey levels that were transmitted,
     box-averaged over the same pixel spans): mean absolute error and fraction within +-16 levels,
     bounds set ~1.5x above what the float64 oracle itself achieves (a discriminator behind a

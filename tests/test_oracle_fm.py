@@ -1,6 +1,8 @@
 """CPU tests of the FM-extension oracle (oracle/fm_oracle.py; SURVEY.md §8(f) N4) and its host logic.
 No reference parity exists for this mode; the oracle is pinned to scipy for its filter / Hilbert pieces
 and to the ground truth of the synthetic generator for the whole definition."""
+from fractions import Fraction
+
 import numpy as np
 
 from oracle import fm_oracle as F
@@ -55,3 +57,62 @@ def test_image_span_from_tone_flags():
     stop[45:50] = True
     assert image_span(start, stop) == (5 * SR, 45 * SR)
     assert image_span(np.zeros(10, dtype=bool), np.zeros(10, dtype=bool)) == (0, 10 * SR)
+
+
+def _smooth7(v):
+    for p in (2, 3, 5, 7):
+        while v % p == 0:
+            v //= p
+    return v == 1
+
+
+def test_next_smooth_length_is_the_librarys():
+    """The restatement of csrc/fft_plan.cu next_smooth_length against a brute-force search with the library's own
+    planning test: primes, numbers just above a 7-smooth one, powers of two and small m."""
+    from wefax_b200 import _native as N
+
+    def can_plan(v):
+        try:
+            return N.fft_plan_describe(v)[1] == 0
+        except ValueError:
+            return False
+
+    def brute(m):
+        v = m
+        while not (_smooth7(v) and can_plan(v)):
+            v += 1
+        return v
+
+    primes = [p for p in range(2, 6000) if all(p % q for q in range(2, int(p ** 0.5) + 1))]
+    smooth = [v for v in range(2, 400_000) if _smooth7(v)]
+    ms = list(range(1, 70)) + primes[::8] + [v + 1 for v in smooth[::6]] + [2 ** k for k in range(1, 19)]
+    ms += [330750, 330751, 1_000_003, 2_205_000 + 1]        # 60 s and 400 s at 11025 Hz halved; a large prime
+    assert len(ms) >= 300
+    for m in ms:
+        assert F.next_smooth_length(m) == brute(m), m
+
+
+def test_padded_and_unpadded_grey_agree_when_nothing_is_padded():
+    pcm, _ = synth.synth_recording(10.0, seed=3, block=64, return_grey=True)
+    for n in (1000, 5000, 66150):                 # halves 500, 2500, 33075 = 3^3 5^2 7^2: npad == n
+        assert F.transform_length(n) == n
+        a, b = F.grey_stream(pcm[:n]), F.grey_stream(pcm[:n], padded=False)
+        assert np.array_equal(a, b)
+    # 11027: padded to 2 * 5600.  The transforms differ mostly at the ends, by several grey ranges at the last
+    # samples, which is why the restatement must pad as the decoder does
+    n = 11027
+    assert F.transform_length(n) == 2 * F.next_smooth_length(5514) == 11200
+    d = np.abs(F.grey_stream(pcm[:n]) - F.grey_stream(pcm[:n], padded=False))
+    assert d[1000:-1000].max() < 1e-3 and d[-10:].max() > 1.0
+
+
+def test_oracle_rows_use_the_exact_line_length():
+    """rows = floor((end - start) / Ls) with the caller's Ls.  Here D / Ls rounds to exactly 65 although 65 * Ls is a
+    fraction of an ulp above D: the 65th row ends at image_end and is part of the picture."""
+    ls, ppm, D = 55125, 29.304888055303476, 358302
+    Ls = 5512.5 / (1.0 + ppm * 1e-6)
+    assert D / Ls == 65.0 and Fraction(65) * Fraction(Ls) > D
+    g = np.linspace(0.0, 1.0, ls + D + 100)
+    img = F.image(g, ls, None, 576, ls + D, line_length=Ls)
+    assert img.shape == (65, 1810)
+    assert np.array_equal(img, F.image(g, ls, 120, 576, ls + D, line_length=Ls))    # lpm is ignored

@@ -1505,6 +1505,7 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
         if (!desc || !pcm || !prm || !slant || !out || desc->n_recordings != 1 || desc->n_frames < 64 ||
             (desc->channels != 1 && desc->channels != 2) || desc->sample_rate < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
+        if (desc->flags & WEFAX_F_PCM_FLOAT32) WEFAX_THROW(WEFAX_ERR_INVALID, "the FM decode takes int16 samples only");
         if (!(prm->lpm > 0.0) || prm->ioc < 1 || !(prm->white_hz > prm->black_hz) || prm->fold_lines < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
         wefax_fm_slant sp = *slant;

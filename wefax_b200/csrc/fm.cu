@@ -70,14 +70,15 @@ fm_grey_kernel(const float *x, const float *y, float *g, long long n, float hz_p
 
 __device__ __forceinline__ float clip01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
 
-// P[o] = sum over lines of clip(grey[from + floor(l * Ls + o)]), o < Lc = ceil(Ls)
+// P[o] = sum over lines of clip(grey[from + floor(l * Ls + o)]), o < Lc = ceil(Ls); l * Ls and the sum each rounded
+// (no fused multiply-add: at a line length that is not a binary fraction the fused form can pick the next sample)
 __global__ void __launch_bounds__(256)
 fm_fold_kernel(const float *g, long long n, long long from, double Ls, int lines, int Lc, float *P) {
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= Lc) return;
     float acc = 0.f;
     for (int l = 0; l < lines; ++l) {
-        const long long i = from + (long long)floor((double)l * Ls + (double)o);
+        const long long i = from + (long long)floor(__dadd_rn(__dmul_rn((double)l, Ls), (double)o));
         if (i < n) acc += clip01(__ldg(g + i));
     }
     P[o] = acc;
@@ -133,25 +134,30 @@ fm_phase_kernel(const float *P, int Lc, int wb, long long from, long long *line_
     }
 }
 
-// pixel (r, p): box average of clip(grey) over [a, a + Ls / W), a = line_start + r * Ls + p * Ls / W
+// pixel (r, p): box average of clip(grey) over [a, a + Ls / W), a = line_start + r * Ls + p * Ls / W.
+// rows = min(rows_max, floor((image_end - line_start) / Ls)), the host's expression (wefax_decode_fm_slant), so
+// every row the caller is told about is written; grid.y strides over the rows (it is capped at 65535)
 __global__ void __launch_bounds__(256)
-fm_image_kernel(const float *g, long long n, const long long *line_start, double Ls, int W, long long image_end,
-                uint8_t *img) {
-    const int p = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
-    const double ls = (double)*line_start;
-    // rows = floor((image_end - line_start) / Ls): the host sizes the grid for the largest possible count
-    if (p >= W || ls + (double)(r + 1) * Ls > (double)image_end) return;
+fm_image_kernel(const float *g, long long n, const long long *line_start, double Ls, int W, int rows_max,
+                long long image_end, uint8_t *img) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= W) return;
+    const long long ls_i = *line_start;
+    const double ls = (double)ls_i;
+    const long long rows = min((long long)rows_max, (long long)floor(__ddiv_rn((double)(image_end - ls_i), Ls)));
     const double step = Ls / (double)W;
-    const double a = ls + (double)r * Ls + (double)p * step, b = a + step;
-    const long long i0 = (long long)floor(a), i1 = (long long)ceil(b);
-    float acc = 0.f;
-    for (long long i = i0; i < i1; ++i) {
-        const double lo = fmax(a, (double)i), hi = fmin(b, (double)(i + 1));
-        const float wgt = (float)(hi - lo);
-        if (i >= 0 && i < n && wgt > 0.f) acc = fmaf(wgt, clip01(__ldg(g + i)), acc);
+    for (long long r = blockIdx.y; r < rows; r += gridDim.y) {
+        const double a = ls + (double)r * Ls + (double)p * step, b = a + step;
+        const long long i0 = (long long)floor(a), i1 = (long long)ceil(b);
+        float acc = 0.f;
+        for (long long i = i0; i < i1; ++i) {
+            const double lo = fmax(a, (double)i), hi = fmin(b, (double)(i + 1));
+            const float wgt = (float)(hi - lo);
+            if (i >= 0 && i < n && wgt > 0.f) acc = fmaf(wgt, clip01(__ldg(g + i)), acc);
+        }
+        const float v = rintf(255.f * acc / (float)step);
+        img[(size_t)r * W + p] = (uint8_t)fminf(fmaxf(v, 0.f), 255.f);
     }
-    const float v = rintf(255.f * acc / (float)step);
-    img[(size_t)r * W + p] = (uint8_t)fminf(fmaxf(v, 0.f), 255.f);
 }
 
 // ---- slant: the sample-clock error measured from the white line pulses (DESIGN.md §4.7a) ----
@@ -311,8 +317,8 @@ void launch_fm_image(wefax_ctx *ctx, const float *g, long long n, const long lon
                      int rows_max, long long image_end, uint8_t *img) {
     if (rows_max <= 0) return;
     StageTimer timer(ctx, "fm_image");
-    dim3 grid((W + 255) / 256, rows_max);
-    fm_image_kernel<<<grid, 256, 0, ctx->stream>>>(g, n, d_line_start, Ls, W, image_end, img);
+    dim3 grid((W + 255) / 256, std::min(rows_max, 65535));
+    fm_image_kernel<<<grid, 256, 0, ctx->stream>>>(g, n, d_line_start, Ls, W, rows_max, image_end, img);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }

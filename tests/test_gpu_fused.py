@@ -221,32 +221,6 @@ def test_both_forms_of_the_greedy_picker_agree(monkeypatch):
         assert res.peaks[i] == O.pattern_search(res.digitalized[i].astype(np.int64), consts), i
 
 
-@pytest.mark.parametrize("env", [{"WEFAX_SIDE": 1}, {"WEFAX_L2_HINT": 2}, {"WEFAX_MID_WARP": 0}, {"WEFAX_TMA_ENV": 1},
-                                 {"WEFAX_PCT_COLLECT": "median"}, {"WEFAX_PCT_NCTA": 32}, {"WEFAX_NOTCH_MINB": 5},
-                                 {"WEFAX_TMA_ISSUER_WARP": 0}, {"WEFAX_TMA_PIPE": 0},
-                                 {"WEFAX_TMA_PIPE": 0, "WEFAX_TMA_ISSUER_WARP": 0}])
-def test_measurement_switches_do_not_change_results(monkeypatch, env):
-    """The A/B switches kept in the library (side stream, L2 hints, CTA-tile middle kernel, TMA-fed envelope pass,
-    always-median collection, selection width, notch occupancy, copy-issuing thread) only move work around."""
-    for k in ("WEFAX_SIDE", "WEFAX_L2_HINT", "WEFAX_MID_WARP", "WEFAX_TMA_ENV", "WEFAX_PCT_COLLECT", "WEFAX_PCT_NCTA",
-              "WEFAX_NOTCH_MINB", "WEFAX_TMA_ISSUER_WARP", "WEFAX_TMA_PIPE"):
-        monkeypatch.delenv(k, raising=False)
-    want = ("audio", "demodulated", "digitalized", "raster")
-    # 176 400 samples: half-length transform 225 x 392 (TMA-staged pass, fused middle, TMA / direct envelope pass);
-    # 1 102 500 samples: long enough for the bracketed percentile selection
-    for seconds in (16.0, 100.0):
-        pcm = np.stack([synth.synth_recording(seconds, lpm=120, seed=60 + k, noise_sigma=0.03) for k in range(2)])
-        base = _decoder(monkeypatch)
-        ref = base.decode(pcm, 11025, 120, want=want)
-        base.close()
-        dec = _decoder(monkeypatch, **env)
-        res = dec.decode(pcm, 11025, 120, want=want)
-        dec.close()
-        _same(res, ref, 2)
-        assert np.array_equal(res.audio, ref.audio)
-        assert np.array_equal(res.demodulated, ref.demodulated)
-
-
 def test_repeated_decode_into_the_same_result_takes_the_short_way_and_stays_right(monkeypatch):
     """``decode(..., out=res)`` with the arguments of the call that made ``res`` skips argument checking and allocation
     (Decoder.decode fast path): same object back, updated in place, equal to a fresh decode; anything different (other

@@ -775,7 +775,7 @@ def _two_pass_cases():
 @pytest.mark.parametrize("R,L", _two_pass_cases())
 def test_hilbert_and_fft_on_every_specialised_kernel(dec, R, L):
     """Half-length plans [R, L] with R on fft_fast_strided_kernel<R1, R2> (both store functors) and L on
-    hilbert_mid_kernel<R1, R2>: envelope against numpy's analytic signal, complex DFT against numpy's FFT."""
+    hilbert_mid_warp_kernel<R1, R2>: envelope against numpy's analytic signal, complex DFT against numpy's FFT."""
     m = R * L
     rng = np.random.default_rng(m)
     x = (rng.normal(size=(2, 2 * m)) * 3000).astype(np.float32)

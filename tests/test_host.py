@@ -213,7 +213,7 @@ def test_parallel_png_writer_roundtrip(tmp_path):
 
 def test_fft_plan_prefers_the_specialised_kernels():
     """The half-length transforms of the BASELINE configs run on fft_fast_strided_kernel (strided pass
-    lengths = products of two radices from {12, 14, 15, 16} or 15*7) and hilbert_mid_kernel (last pass
+    lengths = products of two radices from {12, 14, 15, 16} or 15*7) and hilbert_mid_warp_kernel (last pass
     392 / 300 / 210 / 150 / 140): csrc/fft_fast.cuh, csrc/fft_mid.cuh."""
     fast = {a * b for a in (12, 14, 15, 16) for b in (12, 14, 15, 16)} | {105}
     mid = {392, 300, 210, 150, 140}

@@ -24,7 +24,6 @@ int guarded(wefax_ctx *ctx, F &&f, bool touches_scratch = true) {
             // (a call that failed half way: nothing of it may still be running when the caller reuses its buffers)
             if (ctx->stream && cudaStreamQuery(ctx->stream) != cudaErrorStreamCaptureUnsupported) {
                 cudaStreamSynchronize(ctx->stream);
-                if (ctx->side_stream) cudaStreamSynchronize(ctx->side_stream);
                 (void)cudaGetLastError();
             }
         }
@@ -270,7 +269,6 @@ bool decode_depth_first(wefax_ctx *ctx, const wefax_batch_desc *desc, const int1
         wefax_ctx *lane = ctx->lane_ctx[l];
         lane->max_wave = lane_wave;
         lane->use_fused = ctx->use_fused;
-        lane->use_sym_notch = ctx->use_sym_notch;
         threads.emplace_back([=, &rc] {
             cudaSetDevice(lane->device);
             if (cudaStreamWaitEvent(lane->stream, ctx->ev_lane_fork, 0) != cudaSuccess) {
@@ -481,18 +479,10 @@ int wefax_ctx_create(int device, void *stream, wefax_ctx **out) {
             WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "built for sm_100a (Blackwell); device %d is sm_%d%d", device, prop.major,
                         prop.minor);
         ctx->sm_count = prop.multiProcessorCount;
-        const char *tma = getenv("WEFAX_FFT_TMA");
-        ctx->use_tma = !(tma && tma[0] == '0');
-        const char *fastk = getenv("WEFAX_FFT_FAST");
-        ctx->use_fast = !(fastk && fastk[0] == '0');
-        const char *tmaf = getenv("WEFAX_FFT_TMAFAST");
-        ctx->use_tma_fast = !(tmaf && tmaf[0] == '0');
         if (const char *gr = getenv("WEFAX_GRAPH")) ctx->use_graph = gr[0] != '0';
         if (const char *df = getenv("WEFAX_DEPTH_FIRST")) ctx->depth_first = atoi(df) != 0 ? 1 : 0;
         if (const char *ln = getenv("WEFAX_LANES")) ctx->lanes = std::max(1, std::min(8, atoi(ln)));
         if (const char *lw = getenv("WEFAX_LANE_WAVE")) ctx->lane_wave = std::max(1, atoi(lw));
-        const char *symn = getenv("WEFAX_NOTCH_SYM");
-        ctx->use_sym_notch = !(symn && symn[0] == '0');
         const char *fused = getenv("WEFAX_FUSED");   // WEFAX_FUSED=0: separate grey-map and raster kernels
         ctx->use_fused = !(fused && fused[0] == '0');
         int prio_least = 0, prio_greatest = 0;
@@ -500,30 +490,9 @@ int wefax_ctx_create(int device, void *stream, wefax_ctx **out) {
         if (stream) {
             ctx->stream = (cudaStream_t)stream;
         } else {
-            // the main stream outranks the auxiliary one: its small latency-bound kernels get SM slots first
+            // highest priority: its small latency-bound kernels get SM slots before other work on the device
             CUDA_CHECK(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_greatest));
             ctx->own_stream = true;
-        }
-        {
-            // Measured on B200 (60-min recording): without the graph the side stream gains 0.5 % (828 -> 832 us the other
-            // way round), inside the graph it LOSES 2 % (781 -> 797 us: a graph that is one straight chain of kernel nodes
-            // is scheduled tighter than one with forks), and the graph is the default: WEFAX_SIDE=1 to turn it on.
-            const char *sd = getenv("WEFAX_SIDE");
-            if (sd && sd[0] == '1') {
-                CUDA_CHECK(cudaStreamCreateWithPriority(&ctx->side_stream, cudaStreamNonBlocking, prio_greatest));
-                for (int i = 0; i < wefax_ctx::kSideForks; ++i) {
-                    CUDA_CHECK(cudaEventCreateWithFlags(&ctx->ev_side_fork[i], cudaEventDisableTiming));
-                    CUDA_CHECK(cudaEventCreateWithFlags(&ctx->ev_side_join[i], cudaEventDisableTiming));
-                }
-            }
-        }
-        // WEFAX_OVERLAP=1: grey-map tail on a side stream under the phasing search.  Measured on B200: the
-        // search's 1024-thread CTAs starve behind the bulk kernel (search 85 -> 131 us, step -0.5 %), so off by default.
-        const char *ovl = getenv("WEFAX_OVERLAP");
-        if (ovl && ovl[0] == '1') {
-            CUDA_CHECK(cudaStreamCreateWithPriority(&ctx->aux_stream, cudaStreamNonBlocking, prio_least));
-            CUDA_CHECK(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
-            CUDA_CHECK(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
         }
     });
     if (rc != WEFAX_OK) {
@@ -543,20 +512,6 @@ void wefax_ctx_destroy(wefax_ctx *ctx) {
     ctx->lane_ctx.clear();
     if (ctx->ev_lane_fork) cudaEventDestroy(ctx->ev_lane_fork);
     for (cudaEvent_t e : ctx->ev_lane_join) cudaEventDestroy(e);
-    if (ctx->side_stream) {
-        cudaStreamSynchronize(ctx->side_stream);
-        cudaStreamDestroy(ctx->side_stream);
-        for (int i = 0; i < wefax_ctx::kSideForks; ++i) {
-            cudaEventDestroy(ctx->ev_side_fork[i]);
-            cudaEventDestroy(ctx->ev_side_join[i]);
-        }
-    }
-    if (ctx->aux_stream) {
-        cudaStreamSynchronize(ctx->aux_stream);
-        cudaStreamDestroy(ctx->aux_stream);
-        cudaEventDestroy(ctx->ev_fork);
-        cudaEventDestroy(ctx->ev_join);
-    }
     ctx->plans.clear();
     ctx->bluestein.clear();
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
@@ -717,7 +672,7 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
             WEFAX_THROW(WEFAX_ERR_INVALID, "raster_stride %lld too small (need %lld)", rstride_user, ls.raster_need);
 
         // transform scratch per recording
-        FftPlan *half = (n % 2 == 0 && !getenv("WEFAX_NO_REAL_FFT")) ? get_plan(ctx, n / 2) : nullptr;
+        FftPlan *half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
         FftPlan *plan = half ? nullptr : get_plan(ctx, n);
         long long zlen = half ? n / 2 : n;
         if (!plan && !half) {
@@ -760,9 +715,9 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
             CUDA_CHECK(cudaMemcpyAsync(d_lines, h_lines, sizeof(LineDev) * g, cudaMemcpyHostToDevice, st));
             CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult) * g, st));
             const SyncPlan splan = prepare_sync(ctx, lines.data() + w0, g, n);   // (asynchronous upload from pinned staging)
-            // the phasing search's scratch is cleared beside the first kernels instead of between two latency-bound ones
-            SideFork clears(ctx, 1);
-            clear_sync_scratch(ctx, splan, g, clears.stream());
+            // the phasing search's scratch is cleared among the first operations of the wave instead of between two
+            // latency-bound kernels
+            clear_sync_scratch(ctx, splan, g);
 
             float *d_env = (float *)ctx->work_e.reserve((size_t)g * n * sizeof(float));
             uint8_t *d_dig = (out_dev && out->digitalized) ? out->digitalized + (size_t)w0 * n
@@ -819,10 +774,9 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
             if (fused) {
                 // fused demod-to-pixel path: grey levels of the head for the phasing search (wefax.py:218-294),
                 // then ONE sweep over the envelope writes digitalized_data and the raster (wefax.py:296-327)
-                // (the threshold table is first read by the search's sequential fallback: built beside the search,
-                //  unless the percentile stage has left it behind already)
-                SideFork table(ctx, 2);
-                if (!have_table) launch_grey_table(ctx, d_res, d_tab, g, table.stream());
+                // (the threshold table is first read by the search's sequential fallback; the percentile stage may have
+                //  left it behind already)
+                if (!have_table) launch_grey_table(ctx, d_res, d_tab, g);
                 const long long head = sync_head(splan, n);
                 launch_quantise(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, g, d_res, 0, head, st, "quantise_head");
                 LazyGrey lazy;
@@ -830,13 +784,13 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
                 lazy.es = (size_t)n;
                 lazy.tables = d_tab;
                 lazy.valid = head;
-                launch_sync_search(ctx, d_dig, (size_t)n, n, g, d_lines, d_res, min_mind, splan, nullptr, lazy, &clears, &table);
+                launch_sync_search(ctx, d_dig, (size_t)n, n, g, d_lines, d_res, min_mind, splan, lazy);
                 launch_grey_raster(ctx, d_env, (size_t)n, out->digitalized ? d_dig : nullptr, (size_t)n, d_raster, rs, n, g,
                                    d_lines, lines.data() + w0, d_res, d_tab);
             } else {
-                cudaEvent_t tail_done = launch_quantise_split(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, g, d_res, splan);
+                launch_quantise(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, g, d_res, 0, n, st, "quantise");
                 // ---- phasing search (wefax.py:218-294) and raster (wefax.py:296-327) -----
-                launch_sync_search(ctx, d_dig, (size_t)n, n, g, d_lines, d_res, min_mind, splan, tail_done, LazyGrey(), &clears);
+                launch_sync_search(ctx, d_dig, (size_t)n, n, g, d_lines, d_res, min_mind, splan);
                 if (d_raster)
                     launch_raster(ctx, d_dig, (size_t)n, n, g, d_lines, d_res, d_raster, rs, max_width, (int)(n / min_width));
             }
@@ -948,7 +902,7 @@ int wefax_hilbert_envelope(wefax_ctx *ctx, long long n, int batch, const float *
         float *dx = (float *)ctx->work_a.reserve(bytes);
         float *de = (float *)ctx->work_e.reserve(bytes);
         CUDA_CHECK(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        FftPlan *half = (n % 2 == 0 && !getenv("WEFAX_NO_REAL_FFT")) ? get_plan(ctx, n / 2) : nullptr;
+        FftPlan *half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
         FftPlan *plan = half ? nullptr : get_plan(ctx, n);
         if (half) {
             float2 *z = (float2 *)ctx->work_z.reserve((size_t)(n / 2) * batch * sizeof(float2));
@@ -1052,6 +1006,7 @@ int wefax_sync_raster(wefax_ctx *ctx, long long n, int batch, const uint8_t *dig
         CUDA_CHECK(cudaMemcpyAsync(d_lines, ls.lines.data(), sizeof(LineDev) * batch, cudaMemcpyHostToDevice, st));
         CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult) * batch, st));
         const SyncPlan splan = prepare_sync(ctx, ls.lines.data(), batch, n);
+        clear_sync_scratch(ctx, splan, batch);
         launch_sync_search(ctx, dd, (size_t)n, n, batch, d_lines, d_res, ls.min_mind, splan);
         if (d_raster)
             launch_raster(ctx, dd, (size_t)n, n, batch, d_lines, d_res, d_raster, rs, ls.max_width, (int)(n / ls.min_width));
@@ -1260,6 +1215,7 @@ int wefax_segment_sync(wefax_ctx *ctx, double lpm, const wefax_batch_out *out) {
         CUDA_CHECK(cudaMemcpyAsync(d_lines, ls.lines.data(), sizeof(LineDev), cudaMemcpyHostToDevice, st));
         CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult), st));
         const SyncPlan splan = prepare_sync(ctx, ls.lines.data(), 1, n);
+        clear_sync_scratch(ctx, splan, 1);
         launch_sync_search(ctx, ctx->seg.dig.as<uint8_t>(), (size_t)n, n, 1, d_lines, d_res, ls.min_mind, splan);
         CUDA_CHECK(cudaMemcpyAsync(h_res, d_res, sizeof(RecResult), cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaStreamSynchronize(st));

@@ -46,17 +46,6 @@ struct wefax_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     bool own_stream = false;
-    // low-priority side stream for bulk work that may overlap latency-bound kernels of the main stream
-    cudaStream_t aux_stream = nullptr;
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    // Side stream for the small independent pieces of a step (edge tiles of the notch, scratch clears, the grey
-    // threshold table): forked from / joined to the main stream by events, so that they run beside the kernel the main
-    // stream is busy with instead of between two of its latency-bound ones.  Only with WEFAX_SIDE=1 (api.cu has the
-    // measurements), and never while stage timing is on (the per-stage event pairs live on the main stream).
-    cudaStream_t side_stream = nullptr;
-    static constexpr int kSideForks = 4;
-    cudaEvent_t ev_side_fork[kSideForks] = {nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t ev_side_join[kSideForks] = {nullptr, nullptr, nullptr, nullptr};
     std::string last_error;
     long long launches = 0;
     long long workspace_limit = 24ll << 30;
@@ -82,11 +71,7 @@ struct wefax_ctx {
     cudaEvent_t ev_lane_fork = nullptr;
     std::vector<cudaEvent_t> ev_lane_join;
     int sm_count = 148;
-    bool use_tma = true;   // WEFAX_FFT_TMA=0 forces the LDG tile loads
-    bool use_fast = true;  // WEFAX_FFT_FAST=0 keeps every pass on the generic kernel
-    bool use_sym_notch = true;   // WEFAX_NOTCH_SYM=0: every tile of the notch through the two-section kernel
     bool use_fused = true;  // WEFAX_FUSED=0: grey map and raster as two kernels instead of the fused sweep
-    bool use_tma_fast = true;   // WEFAX_FFT_TMAFAST=0: register-direct loads/stores instead of TMA tiles in the strided pass
     std::map<long long, std::unique_ptr<wefax::FftPlan>> plans;
     std::map<long long, std::unique_ptr<wefax::Bluestein>> bluestein;
     std::map<const void *, int> smem_configured;   // kernels whose dynamic-smem limit was raised
@@ -154,35 +139,6 @@ struct StageTimer {
     }
 };
 
-// One fork / join of the side stream (see wefax_ctx::side_stream).  `slot` picks the event pair: forks that are open at
-// the same time use different slots.  When the side stream is not in use everything simply stays on the main stream.
-struct SideFork {
-    wefax_ctx *ctx;
-    int slot;
-    bool on;
-    SideFork(wefax_ctx *c, int slot_) : ctx(c), slot(slot_), on(c->side_stream != nullptr && !c->timing) {
-        if (!on) return;
-        CUDA_CHECK(cudaEventRecord(ctx->ev_side_fork[slot], ctx->stream));
-        CUDA_CHECK(cudaStreamWaitEvent(ctx->side_stream, ctx->ev_side_fork[slot], 0));
-    }
-    ~SideFork() {   // (an exception between fork and join: never leave the side stream dangling)
-        if (!on) return;
-        cudaEventRecord(ctx->ev_side_join[slot], ctx->side_stream);
-        cudaStreamWaitEvent(ctx->stream, ctx->ev_side_join[slot], 0);
-    }
-    SideFork(const SideFork &) = delete;
-    SideFork &operator=(const SideFork &) = delete;
-    cudaStream_t stream() const { return on ? ctx->side_stream : ctx->stream; }
-    // the side work is complete as far as it has been issued: the main stream waits for it here
-    void join() {
-        if (!on) return;
-        CUDA_CHECK(cudaEventRecord(ctx->ev_side_join[slot], ctx->side_stream));
-        CUDA_CHECK(cudaStreamWaitEvent(ctx->stream, ctx->ev_side_join[slot], 0));
-        on = false;
-    }
-};
-
-
 template <class LoadOp, class StoreOp, int MINB>
 void launch_pass_variant(wefax_ctx *ctx, const PassDev &p, const LoadOp &ld, const StoreOp &st, int batch,
                          const CUtensorMap &map, const float2 *base, size_t bstride) {
@@ -217,12 +173,12 @@ void launch_fast_variant(wefax_ctx *ctx, const PassDev &p, const float2 *src, si
     kern<<<grid, K::T, K::SMEM, ctx->stream>>>(p, src, bstride, st, (int)total);
 }
 
-template <int R1, int R2, class Epi = fast::TileOut>
+// The strided pass with its tiles by tensor TMA (fft_fast_tma3_kernel); false when the pass does not fit the boxes
+template <int R1, int R2>
 bool launch_fast_tma(wefax_ctx *ctx, const PassDev &p, const float2 *src, size_t src_bs, float2 *dst, size_t dst_bs,
-                     int batch, const Epi &epi = Epi()) {
+                     int batch) {
     using K = fast::TmaCfg<R1, R2>;
     static_assert(fast::kFastCW == K::C, "tile geometry of the plan");
-    constexpr bool kTileOut = std::is_same<Epi, fast::TileOut>::value;
     int rbox = 0;
     for (int rb = std::min(K::R, 256); rb >= 1; --rb)
         if (K::R % rb == 0) {
@@ -232,12 +188,8 @@ bool launch_fast_tma(wefax_ctx *ctx, const PassDev &p, const float2 *src, size_t
     if (K::R / rbox > 8) return false;
     alignas(64) CUtensorMap in_map, out_map;
     if (!encode_strided_map(p, src, src_bs, batch, K::C, rbox, &in_map)) return false;
-    if (kTileOut) {
-        if (!encode_strided_map(p, dst, dst_bs, batch, K::C, rbox, &out_map)) return false;
-    } else {
-        out_map = in_map;   // (unused: the functor stores)
-    }
-    auto kern = fast::fft_fast_tma_kernel<R1, R2, Epi>;
+    if (!encode_strided_map(p, dst, dst_bs, batch, K::C, rbox, &out_map)) return false;
+    auto kern = fast::fft_fast_tma3_kernel<R1, R2>;
     const void *fn = (const void *)kern;
     if (!ctx->smem_configured.count(fn)) {
         CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM));
@@ -245,31 +197,7 @@ bool launch_fast_tma(wefax_ctx *ctx, const PassDev &p, const float2 *src, size_t
     }
     const long long total = (long long)p.fast_ntiles * batch;
     const int grid = (int)std::min<long long>(total, (long long)ctx->sm_count);
-    static const bool own_warp = [] {
-        const char *e = getenv("WEFAX_TMA_ISSUER_WARP");
-        return !(e && e[0] == '0');
-    }();
-    static const int l2_hint = [] {
-        const char *e = getenv("WEFAX_L2_HINT");
-        return e ? atoi(e) : 0;
-    }();
-    // three tiles in flight (fft_fast_tma3_kernel) for the plain complex pass unless WEFAX_TMA_PIPE=0
-    static const bool pipe3 = [] {
-        const char *e = getenv("WEFAX_TMA_PIPE");
-        return !(e && e[0] == '0');
-    }();
-    if (kTileOut && pipe3) {
-        auto kern3 = fast::fft_fast_tma3_kernel<R1, R2>;
-        const void *fn3 = (const void *)kern3;
-        if (!ctx->smem_configured.count(fn3)) {
-            CUDA_CHECK(cudaFuncSetAttribute(kern3, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM));
-            ctx->smem_configured[fn3] = 1;
-        }
-        kern3<<<grid, K::T + 32, K::SMEM, ctx->stream>>>(p, in_map, out_map, rbox, (int)total);
-        return true;
-    }
-    kern<<<grid, own_warp ? K::T + 32 : K::T, K::SMEM, ctx->stream>>>(p, in_map, out_map, rbox, (int)total, own_warp ? K::T : 0,
-                                                                        l2_hint, epi);
+    kern<<<grid, K::T + 32, K::SMEM, ctx->stream>>>(p, in_map, out_map, rbox, (int)total);   // + the copy warp
     return true;
 }
 
@@ -279,12 +207,12 @@ template <class LoadOp, class StoreOp>
 bool try_launch_fast(wefax_ctx *ctx, const PassDev &p, const LoadOp &ld, const StoreOp &st, int batch) {
     if constexpr (std::is_same<LoadOp, LoadComplex>::value &&
                   (std::is_same<StoreOp, StoreComplex>::value || std::is_same<StoreOp, StoreEnvPairs>::value)) {
-        if (!ctx->use_fast || !p.fast_R1 || p.contiguous || ld.conj) return false;
+        if (!p.fast_R1 || p.contiguous || ld.conj) return false;
         if ((long long)p.fast_ntiles * batch > 0x7fffffffll) return false;
         StageTimer timer(ctx, p.tag);
         if constexpr (std::is_same<StoreOp, StoreComplex>::value) {
             // plain complex in and out: the TMA-staged variant (tile loads and stores by the copy engine)
-            if (ctx->use_tma_fast && st.scale == 1.f && !st.conj) {
+            if (st.scale == 1.f && !st.conj) {
                 bool done = false;
                 switch (p.fast_R1 * 100 + p.fast_R2) {
                     case 1515: done = launch_fast_tma<15, 15>(ctx, p, ld.src, ld.bstride, st.dst, st.bstride, batch); break;
@@ -293,29 +221,6 @@ bool try_launch_fast(wefax_ctx *ctx, const PassDev &p, const LoadOp &ld, const S
                     case 1514: done = launch_fast_tma<15, 14>(ctx, p, ld.src, ld.bstride, st.dst, st.bstride, batch); break;
                     case 1414: done = launch_fast_tma<14, 14>(ctx, p, ld.src, ld.bstride, st.dst, st.bstride, batch); break;
                     case 1507: done = launch_fast_tma<15, 7>(ctx, p, ld.src, ld.bstride, st.dst, st.bstride, batch); break;
-                    default: break;
-                }
-                if (done) {
-                    CUDA_CHECK(cudaGetLastError());
-                    ctx->launches++;
-                    return true;
-                }
-            }
-        }
-        if constexpr (std::is_same<StoreOp, StoreEnvPairs>::value) {
-            // the envelope store of the last inverse pass with its input tile by TMA a whole tile ahead (side input and
-            // results by direct loads / stores): measured SLOWER than the register-direct kernel below (122 us against
-            // 103 us for the 60-min recording: one 544-thread CTA per SM hides the side loads worse than two CTAs of
-            // 480), so it only runs on request (WEFAX_TMA_ENV=1)
-            static const bool tma_env = [] {
-                const char *e = getenv("WEFAX_TMA_ENV");
-                return e && e[0] == '1';
-            }();
-            if (ctx->use_tma_fast && tma_env) {
-                bool done = false;
-                switch (p.fast_R1 * 100 + p.fast_R2) {
-                    case 1515: done = launch_fast_tma<15, 15, StoreEnvPairs>(ctx, p, ld.src, ld.bstride, nullptr, 0, batch, st); break;
-                    case 1616: done = launch_fast_tma<16, 16, StoreEnvPairs>(ctx, p, ld.src, ld.bstride, nullptr, 0, batch, st); break;
                     default: break;
                 }
                 if (done) {
@@ -359,7 +264,7 @@ void launch_pass(wefax_ctx *ctx, const PassDev &p_in, const LoadOp &ld, const St
     const float2 *base = nullptr;
     size_t bstride = 0;
     p.load_mode = 0;
-    if (ctx->use_tma && ld.tma_source(&base, &bstride)) p.load_mode = choose_load_mode(p, base, bstride, batch, &map);
+    if (ld.tma_source(&base, &bstride)) p.load_mode = choose_load_mode(p, base, bstride, batch, &map);
     StageTimer timer(ctx, p.tag);
     // three CTAs of this pass fit one SM (227 KiB shared memory, 1 KiB reserved per CTA)?
     if ((size_t)p.smem_bytes + 1024 <= (size_t)(227 * 1024) / 3)

@@ -395,32 +395,6 @@ __device__ __forceinline__ void tma_load_4d(void *dst, const CUtensorMap *map, u
         ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
         : "memory");
 }
-// L2 eviction policies for the copy engine: a pass reads every element once (evict first: do not let the input
-// push the previous kernel's freshly written output, or this pass's own, out of the 126 MB L2) and writes what the
-// next pass reads first (evict last).  0 = no hint.
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void tma_load_4d_hint(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2,
-                                                 int c3, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-        ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(policy)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_bulk_hint(void *dst, const void *src, uint32_t bytes, uint64_t *bar, uint64_t policy) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-                     smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
-                 : "memory");
-}
 __device__ __forceinline__ void tma_load_bulk(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                      smem_u32(dst)),

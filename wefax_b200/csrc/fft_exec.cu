@@ -340,21 +340,14 @@ static void ensure_mid_tables(wefax_ctx *ctx, FftPlan *half) {
 
 template <int R1, int R2>
 static void launch_mid(wefax_ctx *ctx, FftPlan *half, float2 *z, size_t zs, int batch) {
-    // warp-autonomous form (one row pair per warp) unless WEFAX_MID_WARP=0 asks for the 8-row CTA tile
-    static const bool by_warp = [] {
-        const char *e = getenv("WEFAX_MID_WARP");
-        return !(e && e[0] == '0');
-    }();
-    using K = fast::MidCfg<R1, R2>;
-    using KW = fast::MidWarpCfg<R1, R2>;
-    auto kern = by_warp ? fast::hilbert_mid_warp_kernel<R1, R2> : fast::hilbert_mid_kernel<R1, R2>;
-    const int smem = by_warp ? KW::SMEM : K::SMEM;
+    using K = fast::MidWarpCfg<R1, R2>;
+    auto kern = fast::hilbert_mid_warp_kernel<R1, R2>;
     const void *fn = (const void *)kern;
     auto it = ctx->smem_configured.find(fn);
     int per_sm;
     if (it == ctx->smem_configured.end()) {
-        CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, K::T, smem));
+        CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM));
+        CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, K::T, K::SMEM));
         if (per_sm < 1) per_sm = 1;
         ctx->smem_configured[fn] = per_sm;
     } else {
@@ -369,13 +362,7 @@ static void launch_mid(wefax_ctx *ctx, FftPlan *half, float2 *z, size_t zs, int 
     a.rows = half->mid_tab.as<fast::MidRow>();
     a.twB = (const float2 *)(half->mid_tab.as<char>() + rows_bytes);
     a.npairs = half->mid_npairs;
-    if (by_warp) {
-        a.tiles_per_batch = a.npairs;               // one pair per warp and round
-        a.total_tiles = a.npairs * batch;
-    } else {
-        a.tiles_per_batch = (a.npairs + K::ROWS / 2 - 1) / (K::ROWS / 2);
-        a.total_tiles = a.tiles_per_batch * batch;
-    }
+    a.total_tiles = a.npairs * batch;               // one pair per warp and round
     a.ncols = (int)(half->n / K::R);
     a.twR = pi.twR;
     a.tw2_lo = half->tw2_lo;
@@ -385,15 +372,10 @@ static void launch_mid(wefax_ctx *ctx, FftPlan *half, float2 *z, size_t zs, int 
     a.tw_mode = pi.tw_mode;
     a.ko_R = pi.ko_R;
     a.inv_m = (float)(1.0 / (double)half->n);
-    static const int l2_hint = [] {
-        const char *e = getenv("WEFAX_L2_HINT");
-        return e ? atoi(e) : 0;
-    }();
-    a.l2_hint = l2_hint;
-    const int ctas = by_warp ? (a.total_tiles + KW::WARPS - 1) / KW::WARPS : a.total_tiles;
+    const int ctas = (a.total_tiles + K::WARPS - 1) / K::WARPS;
     const int grid = std::min(ctas, ctx->sm_count * per_sm);
     StageTimer timer(ctx, "hilbert_mid");
-    kern<<<grid, K::T, smem, ctx->stream>>>(a);
+    kern<<<grid, K::T, K::SMEM, ctx->stream>>>(a);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
@@ -406,7 +388,7 @@ void hilbert_envelope_real(wefax_ctx *ctx, FftPlan *half, const float *x, size_t
     const StoreEnvPairs store_env{(float2 *)env, (const float2 *)x, es / 2, xs / 2, want_y ? 1 : 0};
     int R1 = 0, R2 = 0;
     const bool aligned = (reinterpret_cast<uintptr_t>(z) & 15) == 0 && (batch == 1 || (zs & 1) == 0);
-    if (ctx->use_fast && P >= 2 && aligned && (long long)batch * (long long)(M / half->Rs[P - 1]) < (1ll << 30) &&
+    if (P >= 2 && aligned && (long long)batch * (long long)(M / half->Rs[P - 1]) < (1ll << 30) &&
         fast::mid_pair(half->Rs[P - 1], &R1, &R2)) {
         // passes 0 .. P-2 forward, the fused middle, passes P-2 .. 0 inverse
         ensure_mid_tables(ctx, half);
@@ -645,7 +627,7 @@ __global__ void irfft_scatter_kernel(const float2 *X, size_t xs, uint32_t m2, ui
 
 static bool resample_real_fast(wefax_ctx *ctx, long long n, long long num, const float *x, size_t xs, float *y,
                                size_t ys, int batch) {
-    if ((n & 1) || (num & 1) || (xs & 1) || (ys & 1) || !ctx->use_fast) return false;
+    if ((n & 1) || (num & 1) || (xs & 1) || (ys & 1)) return false;
     if ((reinterpret_cast<uintptr_t>(x) & 7) || (reinterpret_cast<uintptr_t>(y) & 7)) return false;
     FftPlan *hin = get_plan(ctx, n / 2), *hout = get_plan(ctx, num / 2);
     if (!hin || !hout) return false;

@@ -388,13 +388,16 @@ fft_fast_strided_kernel(const PassDev p, const float2 *src, size_t src_bstride, 
     }
 }
 
-// ----------------------------- the pass, TMA-staged ------------------------------
-// Same arithmetic, but the 225 x 32 tile travels by tensor TMA in both directions: one elected thread issues
-// a box load into one of two input buffers a whole tile ahead and a box store of the finished tile; the 480
-// worker threads touch only shared memory.  No global-memory instructions or 64-bit address arithmetic in the
-// loop, 256-byte row segments, and the loads / stores of neighbouring tiles overlap both register stages.
-// Plain complex in, plain complex out (scale 1, no conjugation): the three strided passes that are not the
-// envelope store.  One CTA of 512 threads per SM (two 57.6 KB tile buffers + the exchange tile).
+// ----------------------------- the pass, TMA-staged -----------------------------------------------------------------
+// Same arithmetic, but the R x 32 tile travels by tensor TMA in both directions (256-byte row segments, no global-memory
+// instructions or 64-bit address arithmetic in the workers' loop), and the copy engine runs two tiles ahead of the
+// arithmetic.  Both register stages work IN PLACE on the tile buffer (stage 1 reads and writes the same rows of a
+// column; stage 2 reads its R2 rows, meets the other workers at a barrier, and writes the permuted rows), so there is no
+// exchange tile and the shared memory holds three tile buffers: one being computed, one landing, one leaving.  A 17th
+// warp does nothing but drive the copy engine: it learns through an mbarrier that a tile is finished, stores it, waits
+// (alone) until the store has read the buffer, and at once loads the tile three ahead into it.  The 16 worker warps
+// never wait for a store and meet only each other (named barrier), twice a tile.  Plain complex in, plain complex out
+// (scale 1, no conjugation): the strided passes that are not the envelope store.  One CTA of 544 threads per SM.
 __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
     uint32_t ok;
     asm volatile(
@@ -403,12 +406,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
         : "r"(smem_u32(bar)), "r"(parity)
         : "memory");
     return ok != 0;
-}
-__device__ __forceinline__ void tma_store_4d_hint(const CUtensorMap *map, const void *src, int c0, int c1, int c2, int c3,
-                                                  uint64_t policy) {
-    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3, %4, %5}], [%1], %6;" ::"l"(map),
-                 "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(policy)
-                 : "memory");
 }
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap *map, const void *src, int c0, int c1, int c2, int c3) {
     asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(map),
@@ -425,177 +422,6 @@ template <int R1, int R2> struct TmaCfg {
     static_assert(R1 <= 16 && R2 <= 16, "512 threads = 16 rows x 32 columns");
 };
 
-// Epi = TileOut: the finished tile goes back by TMA (plain complex out).  Any other Epi is a store functor of fft.cuh
-// (the envelope store of the last inverse pass): its side input is fetched into registers before the second
-// stage reads the exchange tile, its results leave by direct global stores; only the input tile uses the copy engine.
-struct TileOut {};
-
-template <int R1, int R2, class Epi = TileOut>
-__global__ void __launch_bounds__(512 + 32, 1)
-fft_fast_tma_kernel(const PassDev p, const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap out_map,
-                    int rbox, int total_tiles, int issuer, int l2_hint, const Epi epi = Epi()) {
-    constexpr bool kTileOut = std::is_same<Epi, TileOut>::value;
-    // l2_hint: 0 none, 1 loads evict-first, 2 loads evict-first and stores evict-last (see fft.cuh)
-    const uint64_t pol_ld = l2_hint >= 1 ? l2_policy_evict_first() : 0ull;
-    const uint64_t pol_st = l2_hint >= 2 ? l2_policy_evict_last() : 0ull;
-    // `issuer` = the thread that drives the copy engine: 512 (lane 0 of a 17th warp that does nothing else, so that no
-    // worker waits for a store to drain before the next load can be issued) or 0 (a worker; launched with 512 threads)
-    using K = TmaCfg<R1, R2>;
-    constexpr int R = K::R, C = K::C;
-    extern __shared__ unsigned char tma_smem_raw[];
-    // tile buffers are TMA destinations / sources: 128-byte aligned
-    // (offset arithmetic on the shared array itself: a round trip through uintptr_t would make every tile access a
-    //  generic LD / ST instead of LDS / STS)
-    float2 *A0 = reinterpret_cast<float2 *>(tma_smem_raw + ((1024u - (smem_u32(tma_smem_raw) & 1023u)) & 1023u));
-    float2 *A1 = A0 + K::TILE;
-    float2 *tb = A1 + K::TILE;                 // exchange tile
-    float2 *P = tb + K::TILE;                  // [R2][C]
-    float2 *twQ = P + R2 * C;                  // [q][u]
-    uint64_t *mbar = reinterpret_cast<uint64_t *>(twQ + R);   // two barriers
-
-    const int tid = threadIdx.x;
-    const int cc = tid % C, row = tid / C;
-    for (int i = tid; i < R; i += K::T) {
-        const int q = i / R1, u = i - q * R1;
-        twQ[i] = __ldg(p.twR + q * u);
-    }
-    if (tid == 0) {
-        mbar_init(mbar, 1);
-        mbar_init(mbar + 1, 1);
-    }
-    __syncthreads();
-    const bool act1 = row < R2, act2 = row < R1;
-    constexpr uint32_t kTileBytes = (uint32_t)(K::TILE * sizeof(float2));
-    const int nbox = R / rbox;
-
-    auto issue_load = [&](int tile, float2 *dst, uint64_t *bar) {
-        const int batch = tile / p.fast_ntiles;
-        const int t_in = tile - batch * p.fast_ntiles;
-        const int o = p.fast_divTpo.div(t_in);
-        const int m0 = (t_in - o * p.fast_tiles_per_o) * C;
-        mbar_expect_tx(bar, kTileBytes);
-        for (int b = 0; b < nbox; ++b) {
-            if (l2_hint >= 1) tma_load_4d_hint(dst + (size_t)b * rbox * C, &in_map, bar, 2 * m0, b * rbox, o, batch, pol_ld);
-            else tma_load_4d(dst + (size_t)b * rbox * C, &in_map, bar, 2 * m0, b * rbox, o, batch);
-        }
-    };
-
-    if (tid == issuer && (int)blockIdx.x < total_tiles) issue_load(blockIdx.x, A0, mbar);
-    int it = 0;
-    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
-        float2 *A = (it & 1) ? A1 : A0;
-        float2 *Aoth = (it & 1) ? A0 : A1;
-        const int batch = tile / p.fast_ntiles;
-        const int t_in = tile - batch * p.fast_ntiles;
-        const int o = p.fast_divTpo.div(t_in);
-        const int m0 = (t_in - o * p.fast_tiles_per_o) * C;
-        const uint32_t m = (uint32_t)(m0 + cc);
-        const bool colok = m < (uint32_t)p.S;
-
-        if (tid == issuer) {
-            // the other buffer was the source of the previous tile's store: reuse it for the next tile's load
-            if (kTileOut) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            if (tile + (int)gridDim.x < total_tiles) issue_load(tile + gridDim.x, Aoth, mbar + ((it + 1) & 1));
-        }
-        uint32_t e0 = 0, de = 0;
-        if (p.tw_mode == 1) {
-            de = m;
-        } else if (p.tw_mode == 2) {
-            const uint32_t ko = (uint32_t)o % (uint32_t)p.ko_R;
-            e0 = ko * m;
-            de = ko * (uint32_t)p.S;
-        }
-        if (!colok) e0 = de = 0;
-        float2 Pval = make_float2(1.f, 0.f), Aval = make_float2(1.f, 0.f);
-        if (p.tw_mode != 0) {
-            if (act1) Pval = pass_twiddle(p, (uint32_t)(row * R1) * de);
-            if (act2) Aval = pass_twiddle(p, e0 + (uint32_t)row * de);
-        }
-        if (tid < K::T)
-            while (!mbar_try_wait(mbar + (it & 1), (uint32_t)((it >> 1) & 1))) {
-            }
-        if (act1) {
-            float2 v[R1];
-#pragma unroll
-            for (int t = 0; t < R1; ++t) v[t] = A[(row + R2 * t) * C + cc];
-            Dft<R1>::run(v);
-            if (p.tw_mode != 0) P[row * C + cc] = Pval;
-            const float2 *tq = twQ + row * R1;
-            tb[row * C + cc] = v[0];
-#pragma unroll
-            for (int u = 1; u < R1; ++u) tb[(row + R2 * u) * C + cc] = pcmul3(v[u], tq[u]);
-        }
-        if constexpr (kTileOut) {
-            __syncthreads();
-            if (act2) {
-                float2 y[R2];
-#pragma unroll
-                for (int t = 0; t < R2; ++t) y[t] = tb[(row * R2 + t) * C + cc];
-                Dft<R2>::run(y);
-                const float2 Aa = bc(Aval.x), Ab = make_float2(-Aval.y, Aval.y);
-#pragma unroll
-                for (int k2 = 0; k2 < R2; ++k2) {
-                    float2 val = y[k2];
-                    if (p.tw_mode != 0) {
-                        val = pcmul2(val, Aa, Ab);
-                        if (k2 > 0) val = pcmul3(val, P[k2 * C + cc]);
-                    }
-                    A[(row + R1 * k2) * C + cc] = val;      // natural row order: the tile is stored as it lies
-                }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncthreads();
-            if (tid == issuer) {
-                for (int b = 0; b < nbox; ++b) {
-                    if (l2_hint >= 2) tma_store_4d_hint(&out_map, A + (size_t)b * rbox * C, 2 * m0, b * rbox, o, batch, pol_st);
-                    else tma_store_4d(&out_map, A + (size_t)b * rbox * C, 2 * m0, b * rbox, o, batch);
-                }
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            }
-        } else {
-            // element index of this thread's output row k = row + R1 * k2: base + k2 * step
-            const size_t gbase = (size_t)o * (size_t)R * (size_t)p.S + m + (size_t)row * (size_t)p.S;
-            const size_t gstep = (size_t)R1 * (size_t)p.S;
-            typename Epi::Side side[R2];
-            if (act2 && colok) {
-#pragma unroll
-                for (int k2 = 0; k2 < R2; ++k2) side[k2] = epi.side_load(gbase + k2 * gstep, batch);
-            }
-            __syncthreads();
-            if (act2) {
-                float2 y[R2];
-#pragma unroll
-                for (int t = 0; t < R2; ++t) y[t] = tb[(row * R2 + t) * C + cc];
-                Dft<R2>::run(y);
-                const float2 Aa = bc(Aval.x), Ab = make_float2(-Aval.y, Aval.y);
-                if (colok) {
-#pragma unroll
-                    for (int k2 = 0; k2 < R2; ++k2) {
-                        float2 val = y[k2];
-                        if (p.tw_mode != 0) {
-                            val = pcmul2(val, Aa, Ab);
-                            if (k2 > 0) val = pcmul3(val, P[k2 * C + cc]);
-                        }
-                        epi(gbase + k2 * gstep, batch, val, row + R1 * k2, 0, side[k2]);
-                    }
-                }
-            }
-            // (the exchange tile is read by this iteration's second stage and written by the next one's first: the
-            //  barrier after the next first stage's loads is not enough, so the iterations are separated here)
-            __syncthreads();
-        }
-    }
-    if (kTileOut && tid == issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
-// ----------------------------- the pass, TMA-staged, three tiles in flight -------------------------------------------
-// Same arithmetic and tile as fft_fast_tma_kernel, but the copy engine runs two tiles ahead of the arithmetic instead
-// of one.  Both register stages work IN PLACE on the tile buffer (stage 1 reads and writes the same rows of a column;
-// stage 2 reads its 15 rows, meets the other workers at a barrier, and writes the permuted rows), so there is no
-// exchange tile and the shared memory holds three tile buffers: one being computed, one landing, one leaving.  A
-// 17th warp does nothing but drive the copy engine: it learns through an mbarrier that a tile is finished, stores it,
-// waits (alone) until the store has read the buffer, and at once loads the tile three ahead into it.  The 16 worker
-// warps never wait for a store and meet only each other (named barrier), twice a tile.
 template <int R1, int R2>
 __global__ void __launch_bounds__(512 + 32, 1)
 fft_fast_tma3_kernel(const PassDev p, const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap out_map,

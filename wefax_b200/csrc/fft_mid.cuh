@@ -4,10 +4,12 @@
 //
 // All three work on engine-order rows of R = R1*R2 contiguous elements (fft_exec.cu:
 // hilbert_pairs_kernel explains the pairing: the mirror M-k of frequency k = kb + ncols*j of
-// row o lives in row o2 at j2 = R-1-j).  A CTA takes four (row, mirrored row) pairs: eight
-// bulk TMA copies bring the rows into shared memory, both transforms and the untangling run
-// there, eight bulk TMA stores write them back.  Compared with three separate kernels this
-// removes two full read+write sweeps over the transform buffer.
+// row o lives in row o2 at j2 = R-1-j).  Every warp owns one (row, mirrored row) pair at a
+// time: two bulk TMA copies bring the rows into shared memory, both transforms and the
+// untangling run there, two bulk TMA stores write them back.  Compared with three separate
+// kernels this removes two full read+write sweeps over the transform buffer.  A warp meets
+// nobody (__syncwarp between the phases, no CTA-wide barrier), so the sixteen warps of an SM
+// drift apart and one warp's copies hide behind the arithmetic of the others.
 //
 // Row transform = two register stages (fft_fast.cuh codelets):
 //   stage 1  item (row, q):  R1 elements q + R2*t of the natural-order row -> DFT_R1 ->
@@ -44,8 +46,8 @@ struct MidArgs {
     float2 *z;
     size_t zs;                     // batch stride (complex elements)
     const MidRow *rows;            // npairs entries
-    int npairs, tiles_per_batch;   // tiles_per_batch = ceil(npairs / 4)
-    int total_tiles;
+    int npairs;                    // row pairs per sequence
+    int total_tiles;               // npairs * batch
     int ncols;                     // rows per sequence
     const float2 *twR;             // w_R^e, e < R
     const float2 *twB;             // w_{2R}^j, j < R   (= w_n^(ncols*j), n = 2*ncols*R)
@@ -54,7 +56,6 @@ struct MidArgs {
     int tw_mode;                   // 2 when a pass follows (e = ko*k), 0 when R is the whole transform
     int ko_R;
     float inv_m;
-    int l2_hint;                   // 0 none, >= 1 row loads evict-first (fft.cuh)
 };
 
 __device__ __forceinline__ void tma_store_bulk(void *gdst, const void *ssrc, uint32_t bytes) {
@@ -66,18 +67,19 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <int R1, int R2> struct MidCfg {
+template <int R1, int R2> struct MidWarpCfg {
     static constexpr int R = R1 * R2;
-    static constexpr int ROWS = 8;
-    static constexpr int T = 128;
-    static constexpr int BP = R2 | 1;          // block pitch of the exchange buffer
-    static constexpr int MIDP = R1 * BP;       // row pitch of the exchange buffer
-    static constexpr int SMEM = (ROWS * R + ROWS * MIDP + R + ROWS * R2) * (int)sizeof(float2) + 16;
+    static constexpr int WARPS = 4, T = 32 * WARPS;
+    static constexpr int BP = R2 | 1, MIDP = R1 * BP;            // block and row pitch of the exchange buffer
+    static constexpr int PER_WARP = 2 * R + 2 * MIDP + 2 * R2;   // float2: rows, exchange rows, inter-pass twiddles
+    static constexpr int SMEM = (R + WARPS * PER_WARP) * (int)sizeof(float2) + WARPS * 8 + 16;
+    static_assert(R % 2 == 0 && PER_WARP % 2 == 0, "bulk copies need 16-byte aligned rows");
 };
 
-template <int R1, int R2, int ROWS = 8, int T = 128>
+// ROWS rows (R apart in nat, MIDP apart in mid) shared by T threads
+template <int R1, int R2, int ROWS, int T>
 __device__ __forceinline__ void mid_stage1(const float2 *nat, float2 *mid, const float2 *twQ, int tid) {
-    using K = MidCfg<R1, R2>;   // (row length and exchange pitches only; ROWS / T are this call's own)
+    using K = MidWarpCfg<R1, R2>;
     // G1 lanes per row (power of two >= R2): a half-warp never straddles two rows, so the 64-bit
     // shared-memory accesses stay conflict-free
     constexpr int G1 = R2 <= 16 ? 16 : 32;
@@ -100,10 +102,10 @@ __device__ __forceinline__ void mid_stage1(const float2 *nat, float2 *mid, const
 }
 
 // pre_aval (optional, only when every thread has at most one item): the item's inter-pass twiddle, fetched earlier
-template <int R1, int R2, bool TW, int ROWS = 8, int T = 128>
+template <int R1, int R2, bool TW, int ROWS, int T>
 __device__ __forceinline__ void mid_stage2(const float2 *mid, float2 *nat, const float2 *P, const MidArgs &a,
                                            const int *s_ko, int tid, const float2 *pre_aval = nullptr) {
-    using K = MidCfg<R1, R2>;   // (row length and exchange pitches only; ROWS / T are this call's own)
+    using K = MidWarpCfg<R1, R2>;
     constexpr int G2 = R1 <= 16 ? 16 : 32;
     static_assert(R1 <= 32, "stage-2 lane group");
 #pragma unroll 1
@@ -140,148 +142,6 @@ __device__ __forceinline__ void mid_stage2(const float2 *mid, float2 *nat, const
 
 template <int R1, int R2>
 __global__ void __launch_bounds__(128, 4)
-hilbert_mid_kernel(const MidArgs a) {
-    using K = MidCfg<R1, R2>;
-    constexpr int R = K::R;
-    extern __shared__ __align__(128) unsigned char mid_smem[];
-    float2 *nat = reinterpret_cast<float2 *>(mid_smem);   // [8][R] natural-order rows (TMA source / destination)
-    float2 *mid = nat + K::ROWS * R;                      // [8][R1][BP] exchange buffer
-    float2 *twQ = mid + K::ROWS * K::MIDP;                // [q][u] stage twiddles
-    float2 *P = twQ + R;                                  // [8][R2] w^(ko*R1*k2)
-    uint64_t *mbar = reinterpret_cast<uint64_t *>(P + K::ROWS * R2);
-    __shared__ int s_o[K::ROWS], s_kb[K::ROWS / 2], s_ko[K::ROWS];
-    __shared__ float2 s_wkb[K::ROWS / 2];
-
-    const int tid = threadIdx.x;
-    for (int i = tid; i < R; i += K::T) {
-        const int q = i / R1, u = i - q * R1;
-        twQ[i] = __ldg(a.twR + q * u);
-    }
-    if (tid == 0) mbar_init(mbar, 1);
-    __syncthreads();
-
-    constexpr uint32_t kRowBytes = R * sizeof(float2);
-    int it = 0;
-    for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++it) {
-        const int batch = tile / a.tiles_per_batch;
-        const int p0 = (tile - batch * a.tiles_per_batch) * (K::ROWS / 2);
-        float2 *zb = a.z + (size_t)batch * a.zs;
-        // rows of this tile: slot 2i = row o of pair i, slot 2i+1 = its mirror (-1: nothing to load)
-        if (tid < K::ROWS / 2) {
-            int o = -1, o2 = -1, kb = 0;
-            if (p0 + tid < a.npairs) {
-                const MidRow r = a.rows[p0 + tid];
-                o = r.o;
-                o2 = r.o2 == r.o ? -1 : r.o2;
-                kb = r.kb;
-                const uint32_t e = (uint32_t)kb;
-                const float2 wk = cmul(__ldg(a.tw2_lo + (e & ((1u << kTwLoBits) - 1))), __ldg(a.tw2_hi + (e >> kTwLoBits)));
-                s_wkb[tid] = make_float2(wk.x * (0.5f * a.inv_m), wk.y * (0.5f * a.inv_m));   // scale folded into the twiddle
-            }
-            s_o[2 * tid] = o;
-            s_o[2 * tid + 1] = o2;
-            s_kb[tid] = kb;
-            s_ko[2 * tid] = o >= 0 ? o % a.ko_R : 0;
-            s_ko[2 * tid + 1] = o2 >= 0 ? o2 % a.ko_R : 0;
-        }
-        __syncthreads();
-        if (tid == 0) {
-            uint32_t bytes = 0;
-            for (int s = 0; s < K::ROWS; ++s) bytes += s_o[s] >= 0 ? kRowBytes : 0u;
-            mbar_expect_tx(mbar, bytes);
-            for (int s = 0; s < K::ROWS; ++s)
-                if (s_o[s] >= 0) tma_load_bulk(nat + s * R, zb + (size_t)s_o[s] * R, kRowBytes, mbar);
-        }
-        // rows that are not loaded transform zeros
-        for (int s = 0; s < K::ROWS; ++s)
-            if (s_o[s] < 0)
-                for (int i = tid; i < R; i += K::T) nat[s * R + i] = make_float2(0.f, 0.f);
-        if (a.tw_mode != 0) {
-            for (int i = tid; i < K::ROWS * R2; i += K::T) {
-                const int row = i / R2, k2 = i - row * R2;
-                const uint32_t e = (uint32_t)s_ko[row] * (uint32_t)(R1 * k2);
-                P[i] = cmul(__ldg(a.tw_lo + (e & ((1u << kTwLoBits) - 1))), __ldg(a.tw_hi + (e >> kTwLoBits)));
-            }
-        }
-        __syncthreads();
-        mbar_wait(mbar, it & 1);
-
-        // ---- last forward pass
-        mid_stage1<R1, R2>(nat, mid, twQ, tid);
-        __syncthreads();
-        mid_stage2<R1, R2, false>(mid, nat, P, a, s_ko, tid);
-        __syncthreads();
-
-        // ---- untangle the real-input spectrum, apply -i*sgn, re-tangle, conjugate, scale
-        // With s = zk + conj(zm), d = zk - conj(zm), w = (inv_m / 2) * w_n^k:  a = conj(w) s,  b = w d,
-        //   row[j]   = conj(a - b)            row2[j2] = -(a + b)
-        // (the mirror's products are the conjugates of a and b, so one pair of complex multiplies serves both rows);
-        // the (pair, j) space is walked flat so that the 128 threads stay busy across the four row pairs.
-        {
-            constexpr int NPR = K::ROWS / 2;
-#pragma unroll 2
-            for (int idx = tid; idx < NPR * R; idx += K::T) {
-                const int pr = idx / R, j = idx - pr * R;
-                if (s_o[2 * pr] < 0) continue;
-                const bool self = s_o[2 * pr + 1] < 0;
-                const int kb = s_kb[pr];
-                float2 *row = nat + (2 * pr) * R;
-                float2 *row2 = self ? row : row + R;
-                const int j2 = kb ? R - 1 - j : (j ? R - j : 0);
-                if (self && j2 < j) continue;
-                if (kb == 0 && j == 0) {
-                    row[0] = make_float2(0.f, 0.f);
-                    continue;
-                }
-                const float2 zk = row[j], zm = row2[j2];
-                const float2 w = pcmul3(__ldg(a.twB + j), s_wkb[pr]);                 // (inv_m / 2) * w_n^k, k = kb + ncols*j
-                const float2 sp = pfma(zm, make_float2(1.f, -1.f), zk);                 // zk + conj zm
-                const float2 dm = pfma(zm, make_float2(-1.f, 1.f), zk);                 // zk - conj zm
-                const float2 wa = bc(w.x);
-                const float2 aa = pfma(sp, wa, pmul(swp(sp), make_float2(w.y, -w.y)));  // conj(w) * sp
-                const float2 bb = pfma(dm, wa, pmul(swp(dm), make_float2(-w.y, w.y)));  // w * dm
-                row[j] = pmul(psub(aa, bb), make_float2(1.f, -1.f));
-                if (!(self && j2 == j)) row2[j2] = pmul(padd(aa, bb), make_float2(-1.f, -1.f));
-            }
-        }
-        __syncthreads();
-
-        // ---- first inverse pass (forward kernels on conjugated data)
-        mid_stage1<R1, R2>(nat, mid, twQ, tid);
-        __syncthreads();
-        if (a.tw_mode != 0)
-            mid_stage2<R1, R2, true>(mid, nat, P, a, s_ko, tid);
-        else
-            mid_stage2<R1, R2, false>(mid, nat, P, a, s_ko, tid);
-        fence_async_smem();
-        __syncthreads();
-        if (tid == 0) {
-            for (int s = 0; s < K::ROWS; ++s)
-                if (s_o[s] >= 0) tma_store_bulk(zb + (size_t)s_o[s] * R, nat + s * R, kRowBytes);
-            tma_store_commit();
-            tma_store_wait_read();   // the rows may be overwritten by the next tile's loads
-        }
-        __syncthreads();
-    }
-    if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// The same sandwich with every WARP on its own: a warp owns one (row, mirrored row) pair - its two bulk loads, both
-// transforms, the untangling and its two bulk stores - and meets nobody: __syncwarp between the phases instead of seven
-// CTA-wide barriers per tile, and the sixteen warps of an SM drift apart so that one warp's copies hide behind the
-// arithmetic of the others.  Same shared-memory footprint as the 8-row tile (4 warps x 2 rows + 2 exchange rows).
-template <int R1, int R2> struct MidWarpCfg {
-    static constexpr int R = R1 * R2;
-    static constexpr int WARPS = 4, T = 32 * WARPS;
-    static constexpr int BP = R2 | 1, MIDP = R1 * BP;
-    static constexpr int PER_WARP = 2 * R + 2 * MIDP + 2 * R2;   // float2: rows, exchange rows, inter-pass twiddles
-    static constexpr int SMEM = (R + WARPS * PER_WARP) * (int)sizeof(float2) + WARPS * 8 + 16;
-    static_assert(R % 2 == 0 && PER_WARP % 2 == 0, "bulk copies need 16-byte aligned rows");
-};
-
-template <int R1, int R2>
-__global__ void __launch_bounds__(128, 4)
 hilbert_mid_warp_kernel(const MidArgs a) {
     using K = MidWarpCfg<R1, R2>;
     constexpr int R = K::R;
@@ -311,14 +171,8 @@ hilbert_mid_warp_kernel(const MidArgs a) {
         const bool self = o2 < 0;
         if (lane == 0) {
             mbar_expect_tx(mbar, self ? kRowBytes : 2 * kRowBytes);
-            if (a.l2_hint >= 1) {
-                const uint64_t pol = l2_policy_evict_first();
-                tma_load_bulk_hint(nat, zb + (size_t)o * R, kRowBytes, mbar, pol);
-                if (!self) tma_load_bulk_hint(nat + R, zb + (size_t)o2 * R, kRowBytes, mbar, pol);
-            } else {
-                tma_load_bulk(nat, zb + (size_t)o * R, kRowBytes, mbar);
-                if (!self) tma_load_bulk(nat + R, zb + (size_t)o2 * R, kRowBytes, mbar);
-            }
+            tma_load_bulk(nat, zb + (size_t)o * R, kRowBytes, mbar);
+            if (!self) tma_load_bulk(nat + R, zb + (size_t)o2 * R, kRowBytes, mbar);
             s_ko[warp][0] = o % a.ko_R;
             s_ko[warp][1] = self ? 0 : o2 % a.ko_R;
         }
@@ -358,7 +212,10 @@ hilbert_mid_warp_kernel(const MidArgs a) {
         mid_stage2<R1, R2, false, 2, 32>(mid, nat, P, a, s_ko[warp], lane);
         __syncwarp();
 
-        // ---- untangle, -i*sgn, re-tangle, conjugate, scale (see hilbert_mid_kernel)
+        // ---- untangle the real-input spectrum, apply -i*sgn, re-tangle, conjugate, scale
+        // With s = zk + conj(zm), d = zk - conj(zm), w = (inv_m / 2) * w_n^k:  a = conj(w) s,  b = w d,
+        //   row[j]   = conj(a - b)            row2[j2] = -(a + b)
+        // (the mirror's products are the conjugates of a and b, so one pair of complex multiplies serves both rows)
         {
             float2 *row = nat;
             float2 *row2 = self ? row : row + R;
@@ -371,12 +228,12 @@ hilbert_mid_warp_kernel(const MidArgs a) {
                     continue;
                 }
                 const float2 zk = row[j], zm = row2[j2];
-                const float2 w = pcmul3(__ldg(a.twB + j), wkb);
-                const float2 sp = pfma(zm, make_float2(1.f, -1.f), zk);
-                const float2 dm = pfma(zm, make_float2(-1.f, 1.f), zk);
+                const float2 w = pcmul3(__ldg(a.twB + j), wkb);                       // (inv_m / 2) * w_n^k, k = kb + ncols*j
+                const float2 sp = pfma(zm, make_float2(1.f, -1.f), zk);                 // zk + conj zm
+                const float2 dm = pfma(zm, make_float2(-1.f, 1.f), zk);                 // zk - conj zm
                 const float2 wa = bc(w.x);
-                const float2 aa = pfma(sp, wa, pmul(swp(sp), make_float2(w.y, -w.y)));
-                const float2 bb = pfma(dm, wa, pmul(swp(dm), make_float2(-w.y, w.y)));
+                const float2 aa = pfma(sp, wa, pmul(swp(sp), make_float2(w.y, -w.y)));  // conj(w) * sp
+                const float2 bb = pfma(dm, wa, pmul(swp(dm), make_float2(-w.y, w.y)));  // w * dm
                 row[j] = pmul(psub(aa, bb), make_float2(1.f, -1.f));
                 if (!(self && j2 == j)) row2[j2] = pmul(padd(aa, bb), make_float2(-1.f, -1.f));
             }
@@ -404,7 +261,7 @@ hilbert_mid_warp_kernel(const MidArgs a) {
 }
 
 inline bool mid_pair(int R, int *R1, int *R2) {
-    static const int pairs[][2] = {{14, 28}, {10, 14}, {15, 20}, {10, 15}, {14, 15}};   // keep in step with launch_mid_any
+    static const int pairs[][2] = {{14, 28}, {10, 14}, {15, 20}, {10, 15}, {14, 15}};   // keep in step with hilbert_envelope_real (fft_exec.cu)
     for (auto &pr : pairs)
         if (pr[0] * pr[1] == R) {
             if (R1) *R1 = pr[0];

@@ -15,15 +15,14 @@ namespace wefax {
 
 namespace {
 
-int env_int(const char *name, int dflt) {
-    const char *v = getenv(name);
-    return (v && *v) ? atoi(v) : dflt;
-}
-
 // tile budget in complex elements (64 KiB of float2 => 3 CTAs / SM)
-int tile_max() { return env_int("WEFAX_FFT_TILE", 8192); }
+constexpr int kTileMax = 8192;
 // strided passes keep at least this many adjacent columns per tile (coalescing)
-int min_cols() { return env_int("WEFAX_FFT_MINC", 8); }
+constexpr int kMinCols = 8;
+// ... and at most this many
+constexpr int kMaxCols = 64;
+// the stride-1 pass keeps tile + w_R table + permutation (18 bytes per point) within 227 KiB
+constexpr long long kLastPassMax = 12000;
 
 bool smooth13(long long n) {
     for (int p : {2, 3, 5, 7, 11, 13})
@@ -84,12 +83,10 @@ const StagePlan &stage_plan(int R) {
 // (256-byte row segments); the budget is 8192 complex (64 KiB, 2-3 CTAs per SM) and is
 // raised to 16384 (one CTA per SM) only when that is what it takes to get there.
 int tile_cols(int R, int ncols, bool strided) {
-    const int tmax = tile_max();
-    const int maxc = env_int("WEFAX_FFT_MAXC", 64);
     int C = 1;
-    while (C * 2 * R <= tmax && C * 2 <= maxc) C *= 2;
-    if (strided && C < 32 && !getenv("WEFAX_FFT_TILE") && maxc >= 32)
-        while (C * 2 * R <= 2 * tmax && C < 32) C *= 2;
+    while (C * 2 * R <= kTileMax && C * 2 <= kMaxCols) C *= 2;
+    if (strided && C < 32)
+        while (C * 2 * R <= 2 * kTileMax && C < 32) C *= 2;
     while (C > 1 && C / 2 >= ncols) C /= 2;
     return C;
 }
@@ -101,9 +98,9 @@ double pass_cost(int R, long long n, bool strided) {
     const StagePlan &sp = stage_plan(R);
     if (sp.cost < 0) return -1.0;
     // specialised two-stage kernel (fft_fast.cuh): ~45 instructions per point
-    if (strided && n >= (1 << 16) && env_int("WEFAX_FFT_FAST", 1) && fast::fast_pair(R, nullptr, nullptr)) return 50.0;
+    if (strided && n >= (1 << 16) && fast::fast_pair(R, nullptr, nullptr)) return 50.0;
     // stride-1 pass lengths the fused middle kernel of the real-input Hilbert transform handles (fft_mid.cuh)
-    if (!strided && n >= (1 << 16) && env_int("WEFAX_FFT_FAST", 1) && fast::mid_pair(R, nullptr, nullptr)) return 60.0;
+    if (!strided && n >= (1 << 16) && fast::mid_pair(R, nullptr, nullptr)) return 60.0;
     const int C = tile_cols(R, (int)std::min<long long>(n / R, 1 << 30), strided);
     double c = kPassCost;
     for (int r : sp.radices) {
@@ -173,18 +170,12 @@ bool plan_factors(long long n, std::vector<int> &Rs) {
         return true;
     }
     if (!smooth13(n)) return false;
-    const int tmax = tile_max();
-    // the stride-1 pass keeps tile + w_R table + permutation (18 bytes per point) within 227 KiB
-    const long long cap_l = getenv("WEFAX_FFT_TILE") ? tmax : 12000;
-    const long long cap_s = std::max(2, tmax / min_cols());
-    int forced = env_int("WEFAX_FFT_PASSES", 0);
     double best_cost = 1e300;
     for (int P = 1; P <= kMaxPasses; ++P) {
-        if (forced && P != forced) continue;
         Search s;
         s.n = n;
-        s.cap_s = cap_s;
-        s.cap_l = cap_l;
+        s.cap_s = kTileMax / kMinCols;
+        s.cap_l = kLastPassMax;
         s.min_r = n >= 64 * 64 ? 64 : 2;   // no degenerate passes on long transforms
         s.go(n, P - 1, 2);
         if (!s.best.empty() && s.best_cost < best_cost - 1e-9) {
@@ -296,7 +287,7 @@ std::unique_ptr<FftPlan> make_plan(long long n, cudaStream_t stream) {
             }
         d.nbox = d.rbox ? R / d.rbox : 0;
         if (d.nbox > 16) d.rbox = d.nbox = 0;
-        d.nthreads = std::max(C, env_int("WEFAX_FFT_THREADS", kFftThreads));
+        d.nthreads = std::max(C, kFftThreads);
         d.twR = (const float2 *)(base + o_twR[i]);
         d.perm = (const uint16_t *)(base + o_perm[i]);
         d.smem_bytes = (int)((size_t)C * R * sizeof(float2) + (size_t)R * sizeof(float2) +
@@ -397,7 +388,7 @@ int choose_load_mode(const PassDev &p, const float2 *base, size_t bstride, int b
 }
 
 // 4-D tensor map {2S floats, R, outer, batch} with a box of `cols` complex columns x `rbox` rows for the
-// TMA-staged strided pass (fft_fast.cuh: fft_fast_tma_kernel); false when the geometry cannot be encoded.
+// TMA-staged strided pass (fft_fast.cuh: fft_fast_tma3_kernel); false when the geometry cannot be encoded.
 bool encode_strided_map(const PassDev &p, const float2 *base, size_t bstride, int batch, int cols, int rbox,
                         CUtensorMap *map) {
     if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || (p.S & 1) || rbox < 1 || rbox > 256) return false;

@@ -471,9 +471,9 @@ __global__ void __launch_bounds__(kGrThreads, ALIGN == 0 ? 4 : 5) grey_raster_ke
     }
 }
 
-void launch_grey_table(wefax_ctx *ctx, const RecResult *res, GreyTable *tables, int batch, cudaStream_t stream) {
+void launch_grey_table(wefax_ctx *ctx, const RecResult *res, GreyTable *tables, int batch) {
     StageTimer timer(ctx, "grey_table");
-    grey_table_kernel<<<batch, 256, 0, stream ? stream : ctx->stream>>>(res, tables);
+    grey_table_kernel<<<batch, 256, 0, ctx->stream>>>(res, tables);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }

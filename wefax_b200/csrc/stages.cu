@@ -234,8 +234,12 @@ __device__ __forceinline__ float2 fir_fma2(float c, float2 a, float2 acc) {
 // Interior tiles (further than the filter's memory from both ends of the signal): the two sections are one
 // symmetric FIR, out[i] = g0 x[i] + sum_k g_k (x[i-k] + x[i+k]).  One shared-memory stage instead of two, half the
 // multiplies; mono int16 comes in as one 16-byte load per thread.
-template <int MODE, int KC, int MINB>
-__global__ void __launch_bounds__(kFirThreads, MINB)
+// Persistent CTAs, kNotchSymCtas per SM with the window and both partial sums in registers (62).  Five per SM cap the
+// registers at 48 and spill; they were measured no faster (DESIGN.md 4.1).
+constexpr int kNotchSymCtas = 4;
+
+template <int MODE, int KC>
+__global__ void __launch_bounds__(kFirThreads, kNotchSymCtas)
 notch_sym_kernel(const void *in, size_t in_stride, float *out, size_t out_stride, float2 *zout, size_t z_stride,
                  long long n, const FirParams fp, int tile0, int ntiles) {
     constexpr int TS = kFirTile;
@@ -363,20 +367,10 @@ notch_sym_kernel(const void *in, size_t in_stride, float *out, size_t out_stride
 template <int MODE, int KC>
 static void launch_notch_sym(wefax_ctx *ctx, const void *in, size_t in_stride, float *out, size_t out_stride, float2 *zout,
                              size_t z_stride, long long n, const FirParams &fp, int batch, int tile0, int ntiles) {
-    // persistent CTAs of 256 threads: 4 per SM with the window and both partial sums in registers (62), or 5 with the
-    // register count capped at 48 (a 16-byte spill); WEFAX_NOTCH_MINB picks (measured: see DESIGN.md 4.1)
-    static const int minb = [] {
-        const char *e = getenv("WEFAX_NOTCH_MINB");
-        return e && atoi(e) == 5 ? 5 : 4;
-    }();
-    const int per_rec = std::max(1, (ctx->sm_count * minb + batch - 1) / batch);
+    const int per_rec = std::max(1, (ctx->sm_count * kNotchSymCtas + batch - 1) / batch);
     dim3 grid((unsigned)std::min(ntiles, per_rec), batch);
-    if (minb == 5)
-        notch_sym_kernel<MODE, KC, 5><<<grid, kFirThreads, 0, ctx->stream>>>(in, in_stride, out, out_stride, zout, z_stride, n,
-                                                                              fp, tile0, ntiles);
-    else
-        notch_sym_kernel<MODE, KC, 4><<<grid, kFirThreads, 0, ctx->stream>>>(in, in_stride, out, out_stride, zout, z_stride, n,
-                                                                              fp, tile0, ntiles);
+    notch_sym_kernel<MODE, KC><<<grid, kFirThreads, 0, ctx->stream>>>(in, in_stride, out, out_stride, zout, z_stride, n, fp,
+                                                                      tile0, ntiles);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
@@ -388,16 +382,12 @@ static void launch_filtfilt_mode(wefax_ctx *ctx, const void *in, size_t in_strid
     const int ntiles = (int)((n + kFirTile - 1) / kFirTile);
     // tiles [ti_lo, ti_hi) are further than the filter's memory from both ends: symmetric single-stage form
     int ti_lo = 0, ti_hi = 0;
-    if (fp.KC > 0 && ctx->use_sym_notch) {
+    if (fp.KC > 0) {
         const long long margin = 2ll * fp.KP + 16;
         ti_lo = (int)((margin + kFirTile - 1) / kFirTile);
         ti_hi = (int)std::max<long long>(0, (n - margin) / kFirTile);
         if (ti_hi <= ti_lo) ti_lo = ti_hi = 0;
     }
-    // the few edge tiles (two-section kernel) write other samples than the interior ones: side by side
-    SideFork edge(ctx, 0);
-    if (ti_hi <= ti_lo) edge.join();   // (nothing to overlap with)
-    cudaStream_t edge_stream = edge.stream();
     if (ti_hi > ti_lo) {
         switch (fp.KC) {
 #define WEFAX_SYM_CASE(KC_) \
@@ -415,11 +405,10 @@ static void launch_filtfilt_mode(wefax_ctx *ctx, const void *in, size_t in_strid
     dim3 grid((unsigned)(ntiles - tiles_skip), batch);
 #define WEFAX_FIR_CASE(KP_)                                                                                   \
     if (fp.KP == KP_) {                                                                                       \
-        filtfilt_kernel<MODE, KP_><<<grid, kFirThreads, 0, edge_stream>>>(in, in_stride, out, out_stride, zout, z_stride, n, fp, \
-                                                                         tiles_first, tiles_skip);          \
+        filtfilt_kernel<MODE, KP_><<<grid, kFirThreads, 0, ctx->stream>>>(in, in_stride, out, out_stride, zout, z_stride, n, fp, \
+                                                                          tiles_first, tiles_skip);         \
         CUDA_CHECK(cudaGetLastError());                                                                       \
         ctx->launches++;                                                                                      \
-        edge.join();                                                                                          \
         return;                                                                                               \
     }
     WEFAX_FIR_CASE(16)
@@ -710,12 +699,11 @@ struct PctGeom {
     uint32_t r[4];                 // wanted ranks: i_lo, i_lo+1, i_hi, i_hi+1 (clipped)
     double t_lo, t_hi;             // numpy lerp weights
     uint32_t cap;                  // capacity of each candidate list
-    int over_mode;                 // PctState.below[1] counts the samples ABOVE the high bracket (pct_collect2_kernel)
 };
 
 struct PctState {                  // per recording, device
     uint32_t key[4];               // bracket keys lo_a, lo_b, hi_a, hi_b
-    unsigned long long below[2];   // elements with key < lo_a / < hi_a
+    unsigned long long below[2];   // elements with key < lo_a / key > hi_b (pct_collect2_kernel)
     uint32_t len[2];               // candidates collected in each list (may exceed cap: overflow)
     int fallback;
     uint32_t out_key[4];           // order statistics found by the two halves of the final selection
@@ -931,74 +919,10 @@ pct_bracket2_kernel(const float *env, size_t es, PctGeom g, PctState *st_all, Pc
 
 constexpr int kPctStage = 1024;   // per-CTA staging of candidates before one global append
 
-__global__ void __launch_bounds__(256)
-pct_collect_kernel(const float *env, size_t es, PctGeom g, PctState *st_all, float *lists, size_t ls) {
-    __shared__ unsigned long long s_below[2];
-    __shared__ float s_cand[2][kPctStage];
-    __shared__ uint32_t s_cnt[2], s_base[2];
-    PctState *st = st_all + blockIdx.y;
-    const float *e = env + (size_t)blockIdx.y * es;
-    float *list[2] = {lists + (size_t)blockIdx.y * ls, lists + (size_t)blockIdx.y * ls + g.cap};
-    const uint32_t k0 = st->key[0], k1 = st->key[1], k2 = st->key[2], k3 = st->key[3];
-    if (threadIdx.x < 2) {
-        s_below[threadIdx.x] = 0;
-        s_cnt[threadIdx.x] = 0;
-    }
-    __syncthreads();
-    auto append = [&](int h, float v) {
-        const uint32_t slot = atomicAdd(&s_cnt[h], 1u);
-        if (slot < kPctStage) {
-            s_cand[h][slot] = v;
-        } else {                                    // staging full (pathological data): append directly
-            const uint32_t gslot = atomicAdd(&st->len[h], 1u);
-            if (gslot < g.cap) list[h][gslot] = v;
-        }
-    };
-    uint32_t below0 = 0, below1 = 0;
-    const long long stride = 8ll * blockDim.x * gridDim.x;
-    for (long long i0 = 8 * ((long long)blockIdx.x * blockDim.x + threadIdx.x); i0 < g.n; i0 += stride) {
-        float m[8];
-        load_med8(e, i0, g.n, m);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            if (i0 + j >= g.n) break;
-            const uint32_t key = __float_as_uint(m[j]);
-            below0 += key < k0;
-            below1 += key < k2;
-            if (key >= k0 && key <= k1) append(0, m[j]);
-            if (key >= k2 && key <= k3) append(1, m[j]);
-        }
-    }
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-        below0 += __shfl_xor_sync(0xFFFFFFFFu, below0, d);
-        below1 += __shfl_xor_sync(0xFFFFFFFFu, below1, d);
-    }
-    if ((threadIdx.x & 31) == 0) {
-        atomicAdd(&s_below[0], (unsigned long long)below0);
-        atomicAdd(&s_below[1], (unsigned long long)below1);
-    }
-    __syncthreads();
-    if (threadIdx.x < 2) {
-        atomicAdd(&st->below[threadIdx.x], s_below[threadIdx.x]);
-        const uint32_t c = min(s_cnt[threadIdx.x], (uint32_t)kPctStage);
-        s_cnt[threadIdx.x] = c;
-        s_base[threadIdx.x] = c ? atomicAdd(&st->len[threadIdx.x], c) : 0u;
-    }
-    __syncthreads();
-    for (int h = 0; h < 2; ++h)
-        for (uint32_t i = threadIdx.x; i < s_cnt[h]; i += blockDim.x)
-            if (s_base[h] + i < g.cap) list[h][s_base[h] + i] = s_cand[h][i];
-}
-
-// Lean form of pct_collect_kernel: the samples outside the two brackets' span (99 % of them lie strictly
-// between the brackets) cost one subtract, one compare and one warp vote each; only warps that hold a sample
-// in a tail or a bracket enter the classification.  Counts: below[0] = samples under the low bracket,
+// Candidates of both brackets into their lists.  The samples outside the two brackets' span (99 % of them lie
+// strictly between the brackets) cost one subtract, one compare and one warp vote each; only warps that hold a
+// sample in a tail or a bracket enter the classification.  Counts: below[0] = samples under the low bracket,
 // below[1] = samples ABOVE the high bracket (the final selection derives its rank offset from it).
-// PRE = true: the flags-first form described above.  PRE = false: always the 8 medians (their shared min / max tree
-// costs 8.5 instructions a sample), two instructions a sample to test them against the middle, ONE vote per thread
-// and round: data-independent, but measured slower on the 60-min recording (75 us against 61 us), kept for A/B runs.
-template <bool PRE>
 __global__ void __launch_bounds__(256)
 pct_collect2_kernel(const float *env, size_t es, PctGeom g, PctState *st_all, float *lists, size_t ls) {
     __shared__ unsigned long long s_cnt_out[2];
@@ -1048,19 +972,15 @@ pct_collect2_kernel(const float *env, size_t es, PctGeom g, PctState *st_all, fl
                 // A median of 5 lies outside the middle only if at least 3 of its 5 values do: fewer than 3 such
                 // values among the 12 this thread's 8 windows cover settles all 8 at once (the usual case: 99 % of
                 // the samples are in the middle), without a single median.
-                if (PRE) {
-                    int outside = 0;
+                int outside = 0;
 #pragma unroll
-                    for (int j = 2; j < 14; ++j) outside += (__float_as_uint(f[j]) - mid_lo >= mid_span) ? 1 : 0;
-                    need = outside >= 3;
-                } else {
-                    need = true;
-                }
+                for (int j = 2; j < 14; ++j) outside += (__float_as_uint(f[j]) - mid_lo >= mid_span) ? 1 : 0;
+                need = outside >= 3;
             } else {
                 need = true;
             }
         }
-        if (PRE && !__any_sync(0xFFFFFFFFu, need)) continue;
+        if (!__any_sync(0xFFFFFFFFu, need)) continue;
         if (i0 < n) {
             if (fast) med8_from16<2>(f, m);
             else load_med8(e, i0, n, m);
@@ -1068,33 +988,12 @@ pct_collect2_kernel(const float *env, size_t es, PctGeom g, PctState *st_all, fl
 #pragma unroll
             for (int j = 0; j < 8; ++j) m[j] = 0.f;
         }
-        if (PRE) {
 #pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const uint32_t key = __float_as_uint(m[j]);
-                const bool out_mid = (key - mid_lo >= mid_span) && j < nvalid;
-                if (__any_sync(0xFFFFFFFFu, out_mid)) {
-                    if (out_mid) {
-                        if (key <= k1) {
-                            if (key < k0) n_under++;
-                            else append(0, m[j]);
-                        }
-                        if (key >= k2) {
-                            if (key > k3) n_over++;
-                            else append(1, m[j]);
-                        }
-                    }
-                }
-            }
-        } else {
-            bool any_out = false;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) any_out |= (__float_as_uint(m[j]) - mid_lo >= mid_span) && j < nvalid;
-            if (__any_sync(0xFFFFFFFFu, any_out) && any_out) {
-#pragma unroll 1
-                for (int j = 0; j < nvalid; ++j) {
-                    const uint32_t key = __float_as_uint(m[j]);
-                    if (key - mid_lo < mid_span) continue;
+        for (int j = 0; j < 8; ++j) {
+            const uint32_t key = __float_as_uint(m[j]);
+            const bool out_mid = (key - mid_lo >= mid_span) && j < nvalid;
+            if (__any_sync(0xFFFFFFFFu, out_mid)) {
+                if (out_mid) {
                     if (key <= k1) {
                         if (key < k0) n_under++;
                         else append(0, m[j]);
@@ -1154,8 +1053,7 @@ pct_final_kernel(PctGeom g, PctState *st_all, const float *lists, size_t ls, Rec
     // every CTA of the recording takes the same decision from the same data
     bool ok = st->len[0] <= g.cap && st->len[1] <= g.cap;
     // samples under each bracket
-    const unsigned long long below_of[2] = {
-        st->below[0], g.over_mode ? (unsigned long long)g.n - st->below[1] - st->len[1] : st->below[1]};
+    const unsigned long long below_of[2] = {st->below[0], (unsigned long long)g.n - st->below[1] - st->len[1]};
     for (int h = 0; h < 2 && ok; ++h) {
         const unsigned long long b = below_of[h];
         ok = b <= g.r[2 * h] && (unsigned long long)g.r[2 * h + 1] < b + st->len[h];
@@ -1313,8 +1211,6 @@ bool launch_percentiles(wefax_ctx *ctx, const float *env, size_t es, long long n
     auto sclip = [&](long long r) { return (uint32_t)std::min<long long>(std::max<long long>(r, 0), g.ns - 1); };
     g.s_rank[0] = sclip(a_lo); g.s_rank[1] = sclip(b_lo); g.s_rank[2] = sclip(a_hi); g.s_rank[3] = sclip(b_hi);
     g.cap = (uint32_t)std::min<long long>(n, 4 * (2 * delta + 2) * kPctStride + 4096);
-    const char *pc = getenv("WEFAX_PCT_COLLECT");   // "old": the first collect kernel (A/B measurements)
-    g.over_mode = !(pc && pc[0] == 'o');
     const size_t ss = (size_t)((g.ns + 63) & ~63ll), ls = 2 * (size_t)g.cap;
     char *base = (char *)ctx->pct_buf.reserve((ss + ls) * sizeof(float) * batch +
                                               (sizeof(PctState) + sizeof(PctCoop)) * batch + 512);
@@ -1324,20 +1220,14 @@ bool launch_percentiles(wefax_ctx *ctx, const float *env, size_t es, long long n
     PctCoop *coop = (PctCoop *)(((uintptr_t)(pst + batch) + 255) & ~(uintptr_t)255);
     CUDA_CHECK(cudaMemsetAsync(coop, 0, sizeof(PctCoop) * batch, st));
     // CTAs of one recording spin at a barrier, so all of them must be resident at once:
-    // 1024-thread CTAs, two per SM
-    // (WEFAX_PCT_NCTA: CTAs per recording, default up to 128: 41 -> 31 us for the bracket kernel against 32 CTAs,
-    //  whose latency-bound sample read gets four times shorter)
-    static const int ncta_cap = [] {
-        const char *e = getenv("WEFAX_PCT_NCTA");
-        const int v = e ? atoi(e) : 0;
-        return v >= 1 && v <= 148 ? v : 128;
-    }();
-    const int ncta = std::max(1, std::min(ncta_cap, ctx->sm_count / batch));
+    // 1024-thread CTAs, two per SM.  Up to 128 CTAs per recording: 41 -> 31 us for the bracket kernel against 32 CTAs,
+    // whose latency-bound sample read gets four times shorter.
+    const int ncta = std::max(1, std::min(128, ctx->sm_count / batch));
 
     const int per = (int)((g.ns + ncta - 1) / ncta);
     const size_t fused_smem = ((size_t)4 * 2048 + (size_t)per) * sizeof(uint32_t);
-    const char *pb = getenv("WEFAX_PCT_BRACKET");   // "old": separate sample + bracket kernels (A/B measurements)
-    if (fused_smem <= 200 * 1024 && !(pb && pb[0] == 'o')) {
+    // the sample taken in the bracket kernel's shared memory when it fits, else a separate sampling pass
+    if (fused_smem <= 200 * 1024) {
         StageTimer t1(ctx, "pct_bracket");
         const void *fn = (const void *)pct_bracket2_kernel;
         if (!ctx->smem_configured.count(fn)) {
@@ -1376,13 +1266,7 @@ bool launch_percentiles(wefax_ctx *ctx, const float *env, size_t es, long long n
     blocks = std::max(1, blocks / std::max(1, std::min(batch, 8)));
     {
         StageTimer t1(ctx, "pct_collect");
-        if (g.over_mode)
-            if (pc && pc[0] == 'm')   // "median": always the 8 medians (measured slower: 75 us against 61 us)
-                pct_collect2_kernel<false><<<dim3(blocks, batch), 256, 0, st>>>(env, es, g, pst, lists, ls);
-            else
-                pct_collect2_kernel<true><<<dim3(blocks, batch), 256, 0, st>>>(env, es, g, pst, lists, ls);
-        else
-            pct_collect_kernel<<<dim3(blocks, batch), 256, 0, st>>>(env, es, g, pst, lists, ls);
+        pct_collect2_kernel<<<dim3(blocks, batch), 256, 0, st>>>(env, es, g, pst, lists, ls);
     }
     {
         StageTimer t1(ctx, "pct_final");
@@ -1994,22 +1878,18 @@ long long sync_head(const SyncPlan &sp, long long n) {
     return sp.any_fast ? std::min(n, ((sp.max_limc + kSyncMaxL + 2047) / 2048) * 2048) : n;
 }
 
-void clear_sync_scratch(wefax_ctx *ctx, const SyncPlan &sp, int batch, cudaStream_t stream) {
-    (void)ctx;
+void clear_sync_scratch(wefax_ctx *ctx, const SyncPlan &sp, int batch) {
     if (!sp.any_fast) return;
-    CUDA_CHECK(cudaMemsetAsync(sp.first_pos, 0x7F, sizeof(int) * batch, stream));   // 0x7F7F7F7F = no positive correlation yet
-    CUDA_CHECK(cudaMemsetAsync(sp.bits, 0, sp.bs * batch * sizeof(uint32_t), stream));
+    CUDA_CHECK(cudaMemsetAsync(sp.first_pos, 0x7F, sizeof(int) * batch, ctx->stream));   // 0x7F7F7F7F = no positive correlation yet
+    CUDA_CHECK(cudaMemsetAsync(sp.bits, 0, sp.bs * batch * sizeof(uint32_t), ctx->stream));
 }
 
 void launch_sync_search(wefax_ctx *ctx, const uint8_t *dig, size_t ds, long long n, int batch, const LineDev *lines,
-                        RecResult *res, int min_mindistance, const SyncPlan &sp, cudaEvent_t all_data_ready,
-                        const LazyGrey &lazy, SideFork *clears, SideFork *table) {
+                        RecResult *res, int min_mindistance, const SyncPlan &sp, const LazyGrey &lazy) {
     StageTimer timer(ctx, "sync_search");
     cudaStream_t st = ctx->stream;
     const char *fs = getenv("WEFAX_SYNC_FORCE_SCAN");
     const int force_scan = fs ? atoi(fs) : 0;
-    if (clears) clears->join();
-    else clear_sync_scratch(ctx, sp, batch, st);
     if (sp.any_fast) {
         dim3 g1((unsigned)std::max<long long>(1, (sp.max_limc + kCorrTile - 1) / kCorrTile), batch);
         {
@@ -2043,9 +1923,6 @@ void launch_sync_search(wefax_ctx *ctx, const uint8_t *dig, size_t ds, long long
     } else {
         CUDA_CHECK(cudaMemsetAsync(sp.need_scan, 1, sizeof(int) * batch, st));
     }
-    // the parallel search above only reads the head of the recording; the sequential fallback may read all of it
-    if (all_data_ready) CUDA_CHECK(cudaStreamWaitEvent(st, all_data_ready, 0));
-    if (table) table->join();
     if (min_mindistance >= 4096)
         sync_search_kernel<4, false><<<batch, kSyncThreads, 0, st>>>(dig, ds, n, lines, res, sp.need_scan, lazy);
     else if (min_mindistance >= 2048)
@@ -2070,21 +1947,6 @@ void launch_packet_pulse_search(wefax_ctx *ctx, const uint8_t *dig, size_t ds, l
         sync_search_kernel<1, true><<<n_packets, kSyncThreads, 0, ctx->stream>>>(dig, ds, n, line, res, nullptr, LazyGrey());
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
-}
-
-cudaEvent_t launch_quantise_split(wefax_ctx *ctx, const float *env, size_t es, uint8_t *dig, size_t ds, long long n,
-                                  int batch, const RecResult *res, const SyncPlan &sp) {
-    const long long head = sync_head(sp, n);
-    if (!ctx->aux_stream || head >= n) {
-        launch_quantise(ctx, env, es, dig, ds, n, batch, res, 0, n, ctx->stream, "quantise");
-        return nullptr;
-    }
-    CUDA_CHECK(cudaEventRecord(ctx->ev_fork, ctx->stream));
-    launch_quantise(ctx, env, es, dig, ds, n, batch, res, 0, head, ctx->stream, "quantise_head");
-    CUDA_CHECK(cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_fork, 0));
-    launch_quantise(ctx, env, es, dig, ds, n, batch, res, head, n, ctx->aux_stream, "quantise");
-    CUDA_CHECK(cudaEventRecord(ctx->ev_join, ctx->aux_stream));
-    return ctx->ev_join;
 }
 
 // ===========================================================================

@@ -89,21 +89,12 @@ bool launch_percentiles(wefax_ctx *ctx, const float *env, size_t es, long long n
 void launch_quantise(wefax_ctx *ctx, const float *env, size_t es, uint8_t *dig, size_t ds, long long n, int batch,
                      const RecResult *res, long long i_begin, long long i_end, cudaStream_t stream, const char *tag,
                      int med = 5, double eps = 0.0);
-// Grey map of the whole recording with the tail (everything the parallel phasing search does not read)
-// on the context's low-priority auxiliary stream, so that it overlaps the latency-bound search kernels.
-// Returns the event the tail signals (nullptr when everything ran on the main stream).
-cudaEvent_t launch_quantise_split(wefax_ctx *ctx, const float *env, size_t es, uint8_t *dig, size_t ds, long long n,
-                                  int batch, const RecResult *res, const SyncPlan &sp);
-// min_mindistance: smallest LineDev.mindistance of the batch (sizes the scan chunk; must be >= 1024)
-// all_data_ready (may be null): event to wait for before the sequential fallback scan, which reads all of dig
-struct SideFork;
-// clears: fork whose side work is clear_sync_scratch() (joined before the first kernel; nullptr: cleared here);
-// table: fork whose side work produces what `lazy` reads (joined before the sequential fallback, the only reader)
+// min_mindistance: smallest LineDev.mindistance of the batch (sizes the scan chunk; must be >= 1024).
+// Expects the scratch cleared by clear_sync_scratch() earlier on the context's stream.
 void launch_sync_search(wefax_ctx *ctx, const uint8_t *dig, size_t ds, long long n, int batch, const LineDev *lines,
-                        RecResult *res, int min_mindistance, const SyncPlan &sp, cudaEvent_t all_data_ready = nullptr,
-                        const LazyGrey &lazy = LazyGrey(), SideFork *clears = nullptr, SideFork *table = nullptr);
-// the scratch the parallel search expects cleared (first positive correlation, settled bits), on `stream`
-void clear_sync_scratch(wefax_ctx *ctx, const SyncPlan &sp, int batch, cudaStream_t stream);
+                        RecResult *res, int min_mindistance, const SyncPlan &sp, const LazyGrey &lazy = LazyGrey());
+// the scratch the parallel search expects cleared (first positive correlation, settled bits)
+void clear_sync_scratch(wefax_ctx *ctx, const SyncPlan &sp, int batch);
 void launch_packet_pulse_search(wefax_ctx *ctx, const uint8_t *dig, size_t ds, long long n, int n_packets,
                                 const LineDev *line, RecResult *res, int mindistance);
 // samples the parallel phasing search reads: [0, sync_head(sp, n))
@@ -114,7 +105,7 @@ void launch_raster(wefax_ctx *ctx, const uint8_t *dig, size_t ds, long long n, i
                    const RecResult *res, uint8_t *raster, size_t rs, int max_width, int max_lines);
 // ---- fused median-5 + grey map + raster (greyraster.cu) ----
 // threshold tables of the grey map from RecResult.low/high (one per recording)
-void launch_grey_table(wefax_ctx *ctx, const RecResult *res, GreyTable *tables, int batch, cudaStream_t stream = nullptr);
+void launch_grey_table(wefax_ctx *ctx, const RecResult *res, GreyTable *tables, int batch);
 // envelope -> digitalized (all n samples; dig may be null) + raster (rows of recordings with status OK; raster may
 // be null).  Needs RecResult.start_frame / height / status, i.e. runs after the phasing search.
 void launch_grey_raster(wefax_ctx *ctx, const float *env, size_t es, uint8_t *dig, size_t ds, uint8_t *raster, size_t rs,

@@ -56,7 +56,8 @@ typedef enum {
 #define WEFAX_F_OUT_ON_DEVICE 2u   /* every non-NULL output points to device mem  */
 #define WEFAX_F_PCM_FLOAT32 4u     /* wefax_decode_batch only: pcm points to float32 mono samples (WAV sample formats
                                       other than 16-bit PCM, converted by the caller as scipy.io.wavfile.read would
-                                      deliver them, wefax.py:349); channels must be 1.  The FM decode rejects it.  */
+                                      deliver them, wefax.py:349); channels must be 1.  The other entry points that
+                                      read pcm take int16 only and reject it (WEFAX_ERR_INVALID).  */
 
 /* ---- context -------------------------------------------------------------- */
 
@@ -182,7 +183,7 @@ int wefax_sync_raster(wefax_ctx *ctx, long long n, int batch, const uint8_t *dig
 
 /* ingest (+ resample) + notch + |hilbert| of one extended segment; the envelope stays resident in the
  * context.  desc: n_recordings == 1, n_frames = input frames of the extended segment; pcm as for
- * wefax_decode_batch.  n_resampled = length of the extended segment at 11025 Hz (the planner cuts on
+ * wefax_decode_batch, except that it is always int16: WEFAX_F_PCM_FLOAT32 is rejected (WEFAX_ERR_INVALID).  n_resampled = length of the extended segment at 11025 Hz (the planner cuts on
  * whole 11025-Hz samples, so this is exact; 0 = wefax_resampled_length(n_frames), the reference's float
  * formula for a whole recording).  [core_begin, core_end) = the samples this segment owns.
  * seam (0 = none): the transforms of the reference are circular, so the halo in front of the FIRST segment
@@ -250,7 +251,8 @@ typedef struct {
 /* DataPacket.contain_start_tone() / contain_stop_tone() (data_packet.py:345-406) for every
  * consecutive packet of packet_frames frames of ONE recording: n_packets = n_frames / packet_frames
  * (a trailing partial packet is ignored).  pcm: int16, mono or interleaved stereo (merged as in
- * wefax.py:372), host pointer unless flags has WEFAX_F_PCM_ON_DEVICE.  Outputs are HOST pointers
+ * wefax.py:372), host pointer unless flags has WEFAX_F_PCM_ON_DEVICE; WEFAX_F_PCM_FLOAT32 is rejected
+ * (WEFAX_ERR_INVALID).  Outputs are HOST pointers
  * of n_packets entries each; any may be NULL.  n_*_peaks = number of peaks find_peaks returned
  * (after the distance / height / prominence filters). */
 int wefax_tone_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames, int channels, int sample_rate,
@@ -274,7 +276,8 @@ typedef struct {
  * ONE recording - the phasing gate of the live decoder's state machine (wefax_live.py:187-192): exactly one
  * spectral peak, inside [min_frequency, max_frequency], and at least one pulse from the template search over
  * the packet's own grey levels (data_packet.py:408-465: notch at the packet's rate, |hilbert|, median-3,
- * percentile stretch).  pcm / flags as for wefax_tone_scan.  Outputs are HOST pointers of n_packets entries
+ * percentile stretch).  pcm / flags as for wefax_tone_scan (int16 only: WEFAX_F_PCM_FLOAT32 is rejected with
+ * WEFAX_ERR_INVALID).  Outputs are HOST pointers of n_packets entries
  * (pulses: n_packets x WEFAX_MAX_PULSES, -1 padded; samples: n_packets x packet_frames grey levels, host or
  * device per cudaMemcpyDefault); any may be NULL.  last_pulse = peaks_samples[-1] (-1: none): where the live
  * decoder starts the picture inside the packet (wefax_live.py:191). */

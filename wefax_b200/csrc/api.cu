@@ -173,6 +173,67 @@ constexpr long long kSegMinPiece = 64;   // shortest piece either side of a segm
 
 void use_device(wefax_ctx *ctx) { CUDA_CHECK(cudaSetDevice(ctx->device)); }
 
+// The caller's PCM as a device pointer: pcm itself under WEFAX_F_PCM_ON_DEVICE, else a copy of its first `samples`
+// samples staged in ctx->pcm.  Samples are int16, or float32 under WEFAX_F_PCM_FLOAT32, which only the batch decode
+// takes (float_ok).
+const void *upload_pcm(wefax_ctx *ctx, const void *pcm, size_t samples, unsigned flags, bool float_ok) {
+    const bool f32 = flags & WEFAX_F_PCM_FLOAT32;
+    if (f32 && !float_ok)
+        WEFAX_THROW(WEFAX_ERR_INVALID, "WEFAX_F_PCM_FLOAT32: this entry point takes int16 samples only");
+    if (flags & WEFAX_F_PCM_ON_DEVICE) return pcm;
+    const size_t bytes = samples * (f32 ? sizeof(float) : sizeof(int16_t));
+    void *buf = ctx->pcm.reserve(bytes);
+    StageTimer timer(ctx, "h2d_pcm");
+    CUDA_CHECK(cudaMemcpyAsync(buf, pcm, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    return buf;
+}
+
+// What the notch reads: the uploaded PCM as it is, or the resampled float stream for input not at 11025 Hz.
+// stride: samples from one recording to the next.
+struct NotchInput {
+    IngestMode mode;
+    const void *x;
+    size_t stride;
+    // the input from sample i on (a stereo int16 frame and a float sample are 4 bytes each)
+    const void *at(long long i) const { return (const char *)x + (size_t)i * (mode == kInMonoI16 ? 2 : 4); }
+};
+
+// desc: frames, channels, sample rate and sample type of the uploaded d_pcm; n: the length at 11025 Hz.  The
+// resampler reserves work_z: take any scratch from work_z after this call.
+NotchInput notch_input(wefax_ctx *ctx, const wefax_batch_desc &desc, const void *d_pcm, long long n, int batch) {
+    const long long n_in = desc.n_frames;
+    const bool f32 = desc.flags & WEFAX_F_PCM_FLOAT32;
+    if (desc.sample_rate == WEFAX_TARGET_RATE)
+        return NotchInput{f32 ? kInFloat : (desc.channels == 2 ? kInStereoI16 : kInMonoI16), d_pcm, (size_t)n_in};
+    // (wefax.py:60-62)
+    float *xin = (float *)ctx->resample_in.reserve(((size_t)batch * n_in + (size_t)batch * n) * sizeof(float));
+    float *xrs = xin + (size_t)batch * n_in;
+    const float *src = (const float *)d_pcm;   // already float: the resampler reads it in place
+    if (!f32) {
+        launch_ingest_float(ctx, (const int16_t *)d_pcm, (size_t)n_in, desc.channels, xin, (size_t)n_in, n_in, batch);
+        src = xin;
+    }
+    resample_real(ctx, n_in, n, src, (size_t)n_in, xrs, (size_t)n, batch);
+    return NotchInput{kInFloat, xrs, (size_t)n};
+}
+
+// Segment mode: grey map of the resident envelope into seg.dig with the percentiles in d_res, then the core's share of
+// the optional outputs (no synchronisation)
+void segment_grey_map(wefax_ctx *ctx, const RecResult *d_res, uint8_t *digitalized, float *demodulated) {
+    cudaStream_t st = ctx->stream;
+    const long long n = ctx->seg.n, lo = ctx->seg.core_lo, hi = ctx->seg.core_hi;
+    uint8_t *d_dig = (uint8_t *)ctx->seg.dig.reserve((size_t)n);
+    const float *d_env = ctx->seg.env.as<float>() + ctx->seg.base;
+    launch_quantise(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, 1, d_res, 0, n, st, "quantise");
+    if (digitalized && hi > lo)
+        CUDA_CHECK(cudaMemcpyAsync(digitalized, d_dig + lo, (size_t)(hi - lo), cudaMemcpyDefault, st));
+    if (demodulated && hi > lo) {
+        float *d_med = (float *)ctx->work_a.reserve((size_t)(hi - lo) * sizeof(float));
+        launch_segment_median(ctx, d_env, n, lo, hi, d_med);
+        CUDA_CHECK(cudaMemcpyAsync(demodulated, d_med, (size_t)(hi - lo) * sizeof(float), cudaMemcpyDefault, st));
+    }
+}
+
 struct LineSet {
     std::vector<LineDev> lines;
     int max_width = 0, min_width = 1 << 30, min_mind = 1 << 30;
@@ -672,22 +733,15 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
             WEFAX_THROW(WEFAX_ERR_INVALID, "raster_stride %lld too small (need %lld)", rstride_user, ls.raster_need);
 
         // transform scratch per recording
-        FftPlan *half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
-        FftPlan *plan = half ? nullptr : get_plan(ctx, n);
-        long long zlen = half ? n / 2 : n;
-        if (!plan && !half) {
-            std::vector<int> tmp;
-            zlen = next_smooth_length(2 * n - 1);
-            if (zlen <= 0) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
-        }
+        const EnvelopeForm form = envelope_form(ctx, n);
         long long zlen_rs = 0;
         if (resample) {
             std::vector<int> tmp;
             long long a = plan_factors(n_in, tmp) ? n_in : next_smooth_length(2 * n_in - 1);
-            zlen_rs = std::max(a, zlen);
+            zlen_rs = std::max(a, form.zlen);
         }
         const long long per_rec = (pcm_dev ? 0 : n_in * ch * (long long)esz) + (resample ? n_in * 4 + (n_in + n) * 8 : 0) +
-                                  std::max(zlen, zlen_rs) * 8 + n * (4 + 4 + 4 + 1 + 4) + 4096;
+                                  std::max(form.zlen, zlen_rs) * 8 + n * (4 + 4 + 4 + 1 + 4) + 4096;
         int wave = (int)std::max<long long>(1, std::min<long long>(nrec, ctx->workspace_limit / per_rec));
         wave = std::min(wave, 32768);
         if (ctx->max_wave > 0) wave = std::min(wave, ctx->max_wave);
@@ -704,13 +758,8 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
         // everything of one wave up to (not including) the final synchronisation: asynchronous work on `st` only
         auto issue_wave = [&](int w0, int g) {
             // ---- inputs ------------------------------------------------------------
-            const int16_t *d_pcm = (const int16_t *)((const char *)pcm + (size_t)w0 * n_in * ch * esz);
-            if (!pcm_dev) {
-                int16_t *buf = (int16_t *)ctx->pcm.reserve((size_t)g * n_in * ch * esz);
-                StageTimer timer(ctx, "h2d_pcm");
-                CUDA_CHECK(cudaMemcpyAsync(buf, d_pcm, (size_t)g * n_in * ch * esz, cudaMemcpyHostToDevice, st));
-                d_pcm = buf;
-            }
+            const void *d_pcm = upload_pcm(ctx, (const char *)pcm + (size_t)w0 * n_in * ch * esz, (size_t)g * n_in * ch,
+                                           desc->flags, true);
             memcpy(h_lines, lines.data() + w0, sizeof(LineDev) * g);
             CUDA_CHECK(cudaMemcpyAsync(d_lines, h_lines, sizeof(LineDev) * g, cudaMemcpyHostToDevice, st));
             CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult) * g, st));
@@ -728,45 +777,18 @@ int wefax_decode_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16
                 d_raster = out_dev ? out->raster + (size_t)w0 * rs : (uint8_t *)ctx->out_raster.reserve((size_t)g * rs);
 
             // ---- resample (wefax.py:60-62) + zero-phase notch (wefax.py:63-72) -------
-            // Even n: the notch writes the float audio_data and the envelope comes from a
-            // half-length transform of the packed real signal.  Odd n: the notch also writes
-            // the complex copy (x, 0) a full-length transform reads (or Bluestein's real input).
-            float2 *z = nullptr;
-            if (half)
-                z = (float2 *)ctx->work_z.reserve((size_t)g * (n / 2) * sizeof(float2));
-            else if (plan)
-                z = (float2 *)ctx->work_z.reserve((size_t)g * n * sizeof(float2));
-            const bool need_audio = out->audio != nullptr || half || !plan;
+            // The notch writes the float audio_data where the caller wants it or the envelope's form reads it, and
+            // the complex copy (x, 0) where the form is the full-length complex transform.
+            const bool need_audio = out->audio != nullptr || !form.plan;
             float *d_audio = nullptr;
             if (need_audio)
                 d_audio = (out_dev && out->audio) ? out->audio + (size_t)w0 * n
                                                   : (float *)ctx->work_a.reserve((size_t)g * n * sizeof(float));
-            float2 *zcopy = half ? nullptr : z;
-            if (resample) {
-                float *xin = (float *)ctx->resample_in.reserve(((size_t)g * n_in + (size_t)g * n) * sizeof(float));
-                float *xrs = xin + (size_t)g * n_in;
-                if (pcm_f32)
-                    xin = (float *)d_pcm;   // already float: the resampler reads it in place
-                else
-                    launch_ingest_float(ctx, d_pcm, (size_t)n_in, ch, xin, (size_t)n_in, n_in, g);
-                resample_real(ctx, n_in, n, xin, (size_t)n_in, xrs, (size_t)n, g);
-                // the resampler used work_z: take the (possibly re-allocated) buffer again
-                if (half)
-                    z = (float2 *)ctx->work_z.reserve((size_t)g * (n / 2) * sizeof(float2));
-                else if (plan)
-                    z = zcopy = (float2 *)ctx->work_z.reserve((size_t)g * n * sizeof(float2));
-                launch_filtfilt(ctx, kInFloat, xrs, (size_t)n, d_audio, (size_t)n, zcopy, (size_t)n, n, fp, g);
-            } else {
-                launch_filtfilt(ctx, pcm_f32 ? kInFloat : (ch == 2 ? kInStereoI16 : kInMonoI16), d_pcm, (size_t)n_in, d_audio,
-                                (size_t)n, zcopy, (size_t)n, n, fp, g);
-            }
+            const NotchInput in = notch_input(ctx, *desc, d_pcm, n, g);
+            float2 *z = envelope_scratch(ctx, form, g);
+            launch_filtfilt(ctx, in.mode, in.x, in.stride, d_audio, (size_t)n, form.plan ? z : nullptr, (size_t)n, n, fp, g);
             // ---- analytic-signal envelope (wefax.py:174) ------------------------------
-            if (half)
-                hilbert_envelope_real(ctx, half, d_audio, (size_t)n, z, (size_t)(n / 2), d_env, (size_t)n, g);
-            else if (plan)
-                hilbert_envelope(ctx, plan, nullptr, 0, z, (size_t)n, d_env, (size_t)n, g);
-            else
-                hilbert_envelope_bluestein(ctx, n, d_audio, (size_t)n, d_env, (size_t)n, g);
+            launch_envelope(ctx, form, d_audio, (size_t)n, z, d_env, (size_t)n, g);
             // ---- median-5, percentiles, grey map (wefax.py:175,196-200) ---------------
             const bool fused = d_raster && ctx->use_fused;
             GreyTable *d_tab = fused ? (GreyTable *)ctx->grey_tab.reserve(sizeof(GreyTable) * (size_t)g) : nullptr;
@@ -902,17 +924,16 @@ int wefax_hilbert_envelope(wefax_ctx *ctx, long long n, int batch, const float *
         float *dx = (float *)ctx->work_a.reserve(bytes);
         float *de = (float *)ctx->work_e.reserve(bytes);
         CUDA_CHECK(cudaMemcpyAsync(dx, x, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        FftPlan *half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
-        FftPlan *plan = half ? nullptr : get_plan(ctx, n);
-        if (half) {
-            float2 *z = (float2 *)ctx->work_z.reserve((size_t)(n / 2) * batch * sizeof(float2));
-            hilbert_envelope_real(ctx, half, dx, (size_t)n, z, (size_t)(n / 2), de, (size_t)n, batch);
-        } else if (plan) {
-            float2 *z = (float2 *)ctx->work_z.reserve((size_t)n * batch * sizeof(float2));
-            hilbert_envelope(ctx, plan, dx, (size_t)n, z, (size_t)n, de, (size_t)n, batch);
-        } else {
-            hilbert_envelope_bluestein(ctx, n, dx, (size_t)n, de, (size_t)n, batch);
+        const EnvelopeForm form = envelope_form(ctx, n);
+        float2 *z = envelope_scratch(ctx, form, batch);
+        std::vector<float2> xz;
+        if (form.plan) {
+            // the complex form reads (x, 0), as the decode's notch writes it
+            xz.assign((size_t)n * batch, make_float2(0.f, 0.f));
+            for (size_t i = 0; i < xz.size(); ++i) xz[i].x = x[i];
+            CUDA_CHECK(cudaMemcpyAsync(z, xz.data(), xz.size() * sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
         }
+        launch_envelope(ctx, form, dx, (size_t)n, z, de, (size_t)n, batch);
         CUDA_CHECK(cudaMemcpyAsync(env, de, bytes, cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
     });
@@ -1052,44 +1073,18 @@ int wefax_segment_envelope(wefax_ctx *ctx, const wefax_batch_desc *desc, const i
         ctx->seg.have_env = ctx->seg.have_dig = false;
         const FirParams &fp = cached_fir(ctx, (double)(long long)desc->notch_freq, desc->notch_q);
 
-        FftPlan *half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
-        FftPlan *plan = half ? nullptr : get_plan(ctx, n);
-        const int16_t *d_pcm = pcm;
-        if (!(desc->flags & WEFAX_F_PCM_ON_DEVICE)) {
-            int16_t *buf = (int16_t *)ctx->pcm.reserve((size_t)n_in * ch * sizeof(int16_t));
-            StageTimer timer(ctx, "h2d_pcm");
-            CUDA_CHECK(cudaMemcpyAsync(buf, pcm, (size_t)n_in * ch * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-            d_pcm = buf;
-        }
+        const EnvelopeForm form = envelope_form(ctx, n);
+        const void *d_pcm = upload_pcm(ctx, pcm, (size_t)n_in * ch, desc->flags, false);
         float *d_env = (float *)ctx->seg.env.reserve((size_t)n * sizeof(float));
         float *d_audio = (float *)ctx->work_a.reserve((size_t)n * sizeof(float));
-        const size_t zbytes = half ? (size_t)(n / 2) * sizeof(float2) : (plan ? (size_t)n * sizeof(float2) : 0);
-        float2 *z = zbytes ? (float2 *)ctx->work_z.reserve(zbytes) : nullptr;
-        if (resample) {
-            float *xin = (float *)ctx->resample_in.reserve(((size_t)n_in + (size_t)n) * sizeof(float));
-            float *xrs = xin + n_in;
-            launch_ingest_float(ctx, d_pcm, (size_t)n_in, ch, xin, (size_t)n_in, n_in, 1);
-            resample_real(ctx, n_in, n, xin, (size_t)n_in, xrs, (size_t)n, 1);
-            z = zbytes ? (float2 *)ctx->work_z.reserve(zbytes) : nullptr;   // the resampler used work_z
-            float2 *zc = half ? nullptr : z;
-            if (seam > 0)
-                launch_filtfilt(ctx, kInFloat, xrs, (size_t)n, d_audio, (size_t)n, zc, (size_t)n, seam, fp, 1);
-            launch_filtfilt(ctx, kInFloat, xrs + seam, (size_t)n, d_audio + seam, (size_t)n, zc ? zc + seam : nullptr,
-                            (size_t)n, n - seam, fp, 1);
-        } else {
-            const IngestMode mode = ch == 2 ? kInStereoI16 : kInMonoI16;
-            float2 *zc = half ? nullptr : z;
-            if (seam > 0)
-                launch_filtfilt(ctx, mode, d_pcm, (size_t)n_in, d_audio, (size_t)n, zc, (size_t)n, seam, fp, 1);
-            launch_filtfilt(ctx, mode, d_pcm + (size_t)seam * ch, (size_t)n_in, d_audio + seam, (size_t)n,
-                            zc ? zc + seam : nullptr, (size_t)n, n - seam, fp, 1);
-        }
-        if (half)
-            hilbert_envelope_real(ctx, half, d_audio, (size_t)n, z, (size_t)(n / 2), d_env, (size_t)n, 1);
-        else if (plan)
-            hilbert_envelope(ctx, plan, nullptr, 0, z, (size_t)n, d_env, (size_t)n, 1);
-        else
-            hilbert_envelope_bluestein(ctx, n, d_audio, (size_t)n, d_env, (size_t)n, 1);
+        const NotchInput in = notch_input(ctx, *desc, d_pcm, n, 1);
+        float2 *z = envelope_scratch(ctx, form, 1);
+        float2 *zc = form.plan ? z : nullptr;
+        if (seam > 0)
+            launch_filtfilt(ctx, in.mode, in.x, in.stride, d_audio, (size_t)n, zc, (size_t)n, seam, fp, 1);
+        launch_filtfilt(ctx, in.mode, in.at(seam), in.stride, d_audio + seam, (size_t)n, zc ? zc + seam : nullptr,
+                        (size_t)n, n - seam, fp, 1);
+        launch_envelope(ctx, form, d_audio, (size_t)n, z, d_env, (size_t)n, 1);
         CUDA_CHECK(cudaStreamSynchronize(st));
         // only the side of the seam that holds the core is needed from here on
         const bool tail_side = seam > 0 && seam <= core_begin;
@@ -1123,25 +1118,14 @@ int wefax_segment_quantise(wefax_ctx *ctx, double low, double high, uint8_t *dig
     return guarded(ctx, [&] {
         if (!ctx->seg.have_env) WEFAX_THROW(WEFAX_ERR_INVALID, "wefax_segment_envelope has not run on this context");
         use_device(ctx);
-        cudaStream_t st = ctx->stream;
-        const long long n = ctx->seg.n, lo = ctx->seg.core_lo, hi = ctx->seg.core_hi;
         RecResult *d_res = (RecResult *)ctx->out_small.reserve(sizeof(RecResult));
         RecResult *h_res = (RecResult *)pinned(ctx, sizeof(RecResult));
         memset(h_res, 0, sizeof(RecResult));
         h_res->low = low;
         h_res->high = high;
-        CUDA_CHECK(cudaMemcpyAsync(d_res, h_res, sizeof(RecResult), cudaMemcpyHostToDevice, st));
-        uint8_t *d_dig = (uint8_t *)ctx->seg.dig.reserve((size_t)n);
-        const float *d_env = ctx->seg.env.as<float>() + ctx->seg.base;
-        launch_quantise(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, 1, d_res, 0, n, st, "quantise");
-        if (digitalized && hi > lo)
-            CUDA_CHECK(cudaMemcpyAsync(digitalized, d_dig + lo, (size_t)(hi - lo), cudaMemcpyDefault, st));
-        if (demodulated && hi > lo) {
-            float *d_med = (float *)ctx->work_a.reserve((size_t)(hi - lo) * sizeof(float));
-            launch_segment_median(ctx, d_env, n, lo, hi, d_med);
-            CUDA_CHECK(cudaMemcpyAsync(demodulated, d_med, (size_t)(hi - lo) * sizeof(float), cudaMemcpyDefault, st));
-        }
-        CUDA_CHECK(cudaStreamSynchronize(st));
+        CUDA_CHECK(cudaMemcpyAsync(d_res, h_res, sizeof(RecResult), cudaMemcpyHostToDevice, ctx->stream));
+        segment_grey_map(ctx, d_res, digitalized, demodulated);
+        CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
         ctx->seg.have_dig = true;
     });
 }
@@ -1181,21 +1165,10 @@ int wefax_segment_quantise_dev(wefax_ctx *ctx, const uint32_t *state, uint8_t *d
         if (!state) WEFAX_THROW(WEFAX_ERR_INVALID, "null argument");
         if (!ctx->seg.have_env) WEFAX_THROW(WEFAX_ERR_INVALID, "wefax_segment_envelope has not run on this context");
         use_device(ctx);
-        cudaStream_t st = ctx->stream;
-        const long long n = ctx->seg.n, lo = ctx->seg.core_lo, hi = ctx->seg.core_hi;
         RecResult *d_res = (RecResult *)ctx->out_small.reserve(sizeof(RecResult));
-        CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult), st));
+        CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult), ctx->stream));
         launch_segment_state_to_result(ctx, state, d_res);
-        uint8_t *d_dig = (uint8_t *)ctx->seg.dig.reserve((size_t)n);
-        const float *d_env = ctx->seg.env.as<float>() + ctx->seg.base;
-        launch_quantise(ctx, d_env, (size_t)n, d_dig, (size_t)n, n, 1, d_res, 0, n, st, "quantise");
-        if (digitalized && hi > lo)
-            CUDA_CHECK(cudaMemcpyAsync(digitalized, d_dig + lo, (size_t)(hi - lo), cudaMemcpyDefault, st));
-        if (demodulated && hi > lo) {
-            float *d_med = (float *)ctx->work_a.reserve((size_t)(hi - lo) * sizeof(float));
-            launch_segment_median(ctx, d_env, n, lo, hi, d_med);
-            CUDA_CHECK(cudaMemcpyAsync(demodulated, d_med, (size_t)(hi - lo) * sizeof(float), cudaMemcpyDefault, st));
-        }
+        segment_grey_map(ctx, d_res, digitalized, demodulated);
         ctx->seg.have_dig = true;   // (stream-ordered: the search / raster calls that follow run on the same stream)
     });
 }
@@ -1285,7 +1258,6 @@ int wefax_tone_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames, int 
         if (wave < 1) wave = 1;
         if (wave > n_packets) wave = n_packets;
         if (wave > 65535) wave = 65535;   // grid.y of the transform passes
-        const bool on_dev = (flags & WEFAX_F_PCM_ON_DEVICE) != 0;
         const size_t frame_elems = (size_t)channels;
         uint8_t *h_flags = (uint8_t *)pinned(ctx, (size_t)n_packets * (2 + 2 * sizeof(int32_t)) + 16);
         int32_t *h_counts = (int32_t *)(h_flags + (((size_t)n_packets * 2 + 15) & ~(size_t)15));
@@ -1293,13 +1265,8 @@ int wefax_tone_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames, int 
         int32_t *d_counts = (int32_t *)(d_flags + (((size_t)n_packets * 2 + 15) & ~(size_t)15));
         for (long long p0 = 0; p0 < n_packets; p0 += wave) {
             const int np = (int)std::min(wave, n_packets - p0);
-            const int16_t *src = pcm + (size_t)p0 * P * frame_elems;
-            const int16_t *d_pcm = src;
-            if (!on_dev) {
-                int16_t *buf = (int16_t *)ctx->pcm.reserve((size_t)np * P * frame_elems * sizeof(int16_t));
-                CUDA_CHECK(cudaMemcpyAsync(buf, src, (size_t)np * P * frame_elems * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-                d_pcm = buf;
-            }
+            const int16_t *d_pcm =
+                (const int16_t *)upload_pcm(ctx, pcm + (size_t)p0 * P * frame_elems, (size_t)np * P * frame_elems, flags, false);
             float *x = (float *)ctx->work_a.reserve((size_t)np * P * sizeof(float));
             float2 *X = (float2 *)ctx->work_e.reserve((size_t)np * half * sizeof(float2));
             launch_ingest_float(ctx, d_pcm, P, channels, x, P, (long long)P, np);   // stride in frames
@@ -1354,18 +1321,11 @@ int wefax_sync_pulse_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames
         ts.max_frequency = settings->max_frequency;
         ts.min_amount = ts.max_amount = 1;
 
-        FftPlan *halfp = (P % 2 == 0) ? get_plan(ctx, P / 2) : nullptr;
-        FftPlan *plan = halfp ? nullptr : get_plan(ctx, P);
-        long long zlen = halfp ? P / 2 : P;
-        if (!plan && !halfp) {
-            zlen = next_smooth_length(2 * P - 1);
-            if (zlen <= 0) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for packets of %lld frames", P);
-        }
+        const EnvelopeForm form = envelope_form(ctx, P);
         const size_t per_packet = (size_t)P * (sizeof(float) * 3 + sizeof(float2) * 4 + 1) + (size_t)half_bins * sizeof(float2) +
-                                  (size_t)zlen * sizeof(float2) + sizeof(RecResult) + sizeof(SelState);
+                                  (size_t)form.zlen * sizeof(float2) + sizeof(RecResult) + sizeof(SelState);
         long long wave = (long long)((size_t)ctx->workspace_limit / per_packet);
         wave = std::max<long long>(1, std::min<long long>(std::min<long long>(wave, n_packets), 32768));
-        const bool on_dev = (flags & WEFAX_F_PCM_ON_DEVICE) != 0;
 
         LineDev line;
         memset(&line, 0, sizeof(line));
@@ -1391,13 +1351,8 @@ int wefax_sync_pulse_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames
 
         for (long long p0 = 0; p0 < n_packets; p0 += wave) {
             const int np = (int)std::min(wave, n_packets - p0);
-            const int16_t *src = pcm + (size_t)p0 * P * channels;
-            const int16_t *d_pcm = src;
-            if (!on_dev) {
-                int16_t *buf = (int16_t *)ctx->pcm.reserve((size_t)np * P * channels * sizeof(int16_t));
-                CUDA_CHECK(cudaMemcpyAsync(buf, src, (size_t)np * P * channels * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-                d_pcm = buf;
-            }
+            const int16_t *d_pcm =
+                (const int16_t *)upload_pcm(ctx, pcm + (size_t)p0 * P * channels, (size_t)np * P * channels, flags, false);
             // ---- the spectral test on the raw samples (data_packet.py:302-311) -----------------------------
             float *x = (float *)ctx->resample_in.reserve((size_t)np * P * sizeof(float));
             float2 *X = (float2 *)ctx->work_misc.reserve((size_t)np * half_bins * sizeof(float2));
@@ -1408,18 +1363,9 @@ int wefax_sync_pulse_scan(wefax_ctx *ctx, const int16_t *pcm, long long n_frames
             float *d_audio = (float *)ctx->work_a.reserve((size_t)np * P * sizeof(float));
             float *d_env = (float *)ctx->work_e.reserve((size_t)np * P * sizeof(float));
             uint8_t *d_dig = (uint8_t *)ctx->out_dig.reserve((size_t)np * P);
-            float2 *z = nullptr;
-            if (halfp)
-                z = (float2 *)ctx->work_z.reserve((size_t)np * (P / 2) * sizeof(float2));
-            else if (plan)
-                z = (float2 *)ctx->work_z.reserve((size_t)np * P * sizeof(float2));
-            launch_filtfilt(ctx, kInFloat, x, (size_t)P, d_audio, (size_t)P, halfp ? nullptr : z, (size_t)P, P, fp, np);
-            if (halfp)
-                hilbert_envelope_real(ctx, halfp, d_audio, (size_t)P, z, (size_t)(P / 2), d_env, (size_t)P, np);
-            else if (plan)
-                hilbert_envelope(ctx, plan, nullptr, 0, z, (size_t)P, d_env, (size_t)P, np);
-            else
-                hilbert_envelope_bluestein(ctx, P, d_audio, (size_t)P, d_env, (size_t)P, np);
+            float2 *z = envelope_scratch(ctx, form, np);
+            launch_filtfilt(ctx, kInFloat, x, (size_t)P, d_audio, (size_t)P, form.plan ? z : nullptr, (size_t)P, P, fp, np);
+            launch_envelope(ctx, form, d_audio, (size_t)P, z, d_env, (size_t)P, np);
             CUDA_CHECK(cudaMemsetAsync(d_res, 0, sizeof(RecResult) * np, st));
             launch_percentiles(ctx, d_env, (size_t)P, P, np, d_sel, d_res, 3);
             launch_quantise(ctx, d_env, (size_t)P, d_dig, (size_t)P, P, np, d_res, 0, P, st, "packet_quantise", 3, 0.000001);
@@ -1461,7 +1407,6 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
         if (!desc || !pcm || !prm || !slant || !out || desc->n_recordings != 1 || desc->n_frames < 64 ||
             (desc->channels != 1 && desc->channels != 2) || desc->sample_rate < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
-        if (desc->flags & WEFAX_F_PCM_FLOAT32) WEFAX_THROW(WEFAX_ERR_INVALID, "the FM decode takes int16 samples only");
         if (!(prm->lpm > 0.0) || prm->ioc < 1 || !(prm->white_hz > prm->black_hz) || prm->fold_lines < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
         wefax_fm_slant sp = *slant;
@@ -1484,7 +1429,7 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
         const bool resample = desc->sample_rate != WEFAX_TARGET_RATE;
         const long long n = resample ? wefax_resampled_length(n_in, desc->sample_rate) : n_in;
         if (n < 64) WEFAX_THROW(WEFAX_ERR_INVALID, "recording too short");
-        const bool pcm_dev = desc->flags & WEFAX_F_PCM_ON_DEVICE, out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE;
+        const bool out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE;
         const double Ls = 60.0 / prm->lpm * (double)WEFAX_TARGET_RATE;   // exact (fractional) samples per line
         const int W = (int)llround(M_PI * (double)prm->ioc);
         const long long image_end = (prm->image_end > 0 && prm->image_end <= n) ? prm->image_end : n;
@@ -1504,25 +1449,12 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
         if (!half) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
         const long long npad = 2 * half_len;
 
-        const int16_t *d_pcm = pcm;
-        if (!pcm_dev) {
-            int16_t *buf = (int16_t *)ctx->pcm.reserve((size_t)n_in * ch * sizeof(int16_t));
-            CUDA_CHECK(cudaMemcpyAsync(buf, pcm, (size_t)n_in * ch * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-            d_pcm = buf;
-        }
+        const void *d_pcm = upload_pcm(ctx, pcm, (size_t)n_in * ch, desc->flags, false);
         float *x = (float *)ctx->work_a.reserve((size_t)npad * sizeof(float));
         float *y = (float *)ctx->work_e.reserve((size_t)npad * sizeof(float));
         if (npad > n) CUDA_CHECK(cudaMemsetAsync(x + n, 0, (size_t)(npad - n) * sizeof(float), st));
-        if (resample) {
-            float *xin = (float *)ctx->resample_in.reserve(((size_t)n_in + (size_t)n) * sizeof(float));
-            float *xrs = xin + n_in;
-            launch_ingest_float(ctx, d_pcm, (size_t)n_in, ch, xin, (size_t)n_in, n_in, 1);
-            resample_real(ctx, n_in, n, xin, (size_t)n_in, xrs, (size_t)n, 1);
-            launch_filtfilt(ctx, kInFloat, xrs, (size_t)n, x, (size_t)npad, nullptr, 0, n, fp, 1);
-        } else {
-            launch_filtfilt(ctx, ch == 2 ? kInStereoI16 : kInMonoI16, d_pcm, (size_t)n_in, x, (size_t)npad, nullptr, 0, n,
-                            fp, 1);
-        }
+        const NotchInput in = notch_input(ctx, *desc, d_pcm, n, 1);
+        launch_filtfilt(ctx, in.mode, in.x, in.stride, x, (size_t)npad, nullptr, 0, n, fp, 1);
         float2 *z = (float2 *)ctx->work_z.reserve((size_t)half_len * sizeof(float2));
         hilbert_envelope_real(ctx, half, x, (size_t)npad, z, (size_t)half_len, y, (size_t)npad, 1, /*want_y=*/true);
 

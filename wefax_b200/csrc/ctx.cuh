@@ -275,25 +275,32 @@ void launch_pass(wefax_ctx *ctx, const PassDev &p_in, const LoadOp &ld, const St
     ctx->launches++;
 }
 
-// |hilbert(x)| for `batch` real sequences of length plan->n (no median filter).
-// x: real input (stride xs) or nullptr when z already holds (x, 0); z: complex scratch
-// (stride zs >= n); env: output (stride es).
-void hilbert_envelope(wefax_ctx *ctx, FftPlan *plan, const float *x, size_t xs, float2 *z, size_t zs,
-                      float *env, size_t es, int batch);
-
-// Same result for even n through a half-length transform of the packed real input
+// |hilbert(x)| for even n through a half-length transform of the packed real input
 // (half = plan of n/2; x and env strides even).  x must stay intact until the end.
 // want_y: env receives the Hilbert transform y of x instead of the envelope sqrt(x^2 + y^2)
 void hilbert_envelope_real(wefax_ctx *ctx, FftPlan *half, const float *x, size_t xs, float2 *z, size_t zs, float *env,
                            size_t es, int batch, bool want_y = false);
 
+// How |hilbert(x)| is computed at length n: a half-length transform of the packed real signal (half: even n whose half
+// can be planned), a full-length transform of the complex copy (x, 0) (plan), or Bluestein (neither).
+// zlen: complex scratch per sequence (n / 2, n, or Bluestein's padded length).
+struct EnvelopeForm {
+    FftPlan *half = nullptr, *plan = nullptr;
+    long long n = 0, zlen = 0;
+};
+EnvelopeForm envelope_form(wefax_ctx *ctx, long long n);
+// work_z scratch of `batch` sequences for launch_envelope, and for the complex copy the notch writes (nullptr for
+// Bluestein, which reserves its own).  Take it after anything else that reserves work_z (the resampler): a larger
+// reserve moves the buffer.
+float2 *envelope_scratch(wefax_ctx *ctx, const EnvelopeForm &f, int batch);
+// env = |hilbert(audio)| of `batch` sequences (no median filter).  The complex form reads (audio, 0) from z, where the
+// notch leaves it, and not audio.
+void launch_envelope(wefax_ctx *ctx, const EnvelopeForm &f, const float *audio, size_t as, float2 *z, float *env,
+                     size_t es, int batch);
+
 // natural-order complex DFT (test entry / Bluestein building block)
 void fft_c2c_natural(wefax_ctx *ctx, FftPlan *plan, const float2 *in, float2 *out, float2 *scratch,
                      int batch, bool inverse);
-
-// Bluestein path for lengths with a large prime factor
-void hilbert_envelope_bluestein(wefax_ctx *ctx, long long n, const float *x, size_t xs, float *env,
-                                size_t es, int batch);
 
 // forward DFT of `batch` real sequences of length n (any n), first `keep` bins in natural
 // order into X (stride xs_out); scratch: ctx->work_z

@@ -199,8 +199,11 @@ static void run_inverse(wefax_ctx *ctx, FftPlan *plan, const LoadFirst &ld, cons
     launch_pass(ctx, plan->inv[0], load_c(z, zs), st, batch);
 }
 
-void hilbert_envelope(wefax_ctx *ctx, FftPlan *plan, const float *x, size_t xs, float2 *z, size_t zs, float *env,
-                      size_t es, int batch) {
+// |hilbert(x)| for `batch` real sequences of length plan->n (no median filter).
+// x: real input (stride xs) or nullptr when z already holds (x, 0); z: complex scratch
+// (stride zs >= n); env: output (stride es).
+static void hilbert_envelope(wefax_ctx *ctx, FftPlan *plan, const float *x, size_t xs, float2 *z, size_t zs,
+                             float *env, size_t es, int batch) {
     const size_t n = (size_t)plan->n;
     StoreHilbert sh{z, zs, plan->outer(), (uint32_t)n, (int)(n / plan->Rs[plan->npass - 1]), (float)(1.0 / (double)n)};
     if (x)
@@ -489,8 +492,9 @@ static StoreGeneric sg(int mode, void *dst, const float2 *table, size_t bs, size
     return StoreGeneric{mode, dst, table, bs, n_valid, n, scale, conj};
 }
 
-void hilbert_envelope_bluestein(wefax_ctx *ctx, long long n, const float *x, size_t xs, float *env, size_t es,
-                                int batch) {
+// Bluestein path for lengths with a large prime factor
+static void hilbert_envelope_bluestein(wefax_ctx *ctx, long long n, const float *x, size_t xs, float *env, size_t es,
+                                       int batch) {
     Bluestein *b = get_bluestein(ctx, n);
     const size_t m = (size_t)b->m;
     float2 *z = (float2 *)ctx->work_z.reserve(m * sizeof(float2) * batch);
@@ -503,6 +507,31 @@ void hilbert_envelope_bluestein(wefax_ctx *ctx, long long n, const float *x, siz
                 z, m, batch);
     run_forward(ctx, b->plan, lg(0, z, nullptr, m, m), sg(1, z, vh, m, m, 0, 1.f), z, m, batch);
     run_inverse(ctx, b->plan, lg(0, z, nullptr, m, m), sg(3, env, nullptr, es, (size_t)n, 0, 1.f), z, m, batch);
+}
+
+EnvelopeForm envelope_form(wefax_ctx *ctx, long long n) {
+    EnvelopeForm f;
+    f.n = n;
+    f.half = (n % 2 == 0) ? get_plan(ctx, n / 2) : nullptr;
+    f.plan = f.half ? nullptr : get_plan(ctx, n);
+    f.zlen = f.half ? n / 2 : (f.plan ? n : next_smooth_length(2 * n - 1));
+    if (f.zlen <= 0) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
+    return f;
+}
+
+float2 *envelope_scratch(wefax_ctx *ctx, const EnvelopeForm &f, int batch) {
+    if (!f.half && !f.plan) return nullptr;
+    return (float2 *)ctx->work_z.reserve((size_t)batch * f.zlen * sizeof(float2));
+}
+
+void launch_envelope(wefax_ctx *ctx, const EnvelopeForm &f, const float *audio, size_t as, float2 *z, float *env,
+                     size_t es, int batch) {
+    if (f.half)
+        hilbert_envelope_real(ctx, f.half, audio, as, z, (size_t)f.zlen, env, es, batch);
+    else if (f.plan)
+        hilbert_envelope(ctx, f.plan, nullptr, 0, z, (size_t)f.zlen, env, es, batch);
+    else
+        hilbert_envelope_bluestein(ctx, f.n, audio, as, env, es, batch);
 }
 
 // ----------------------------- resample ------------------------------------

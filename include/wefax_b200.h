@@ -352,6 +352,72 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
                           const wefax_fm_params *params, const wefax_fm_slant *slant, const wefax_fm_out *out,
                           wefax_fm_slant_out *slant_out);
 
+/* ---- every chart of a recording (DESIGN.md 4.7b) --------------------------------------------------------------------
+ * Tone windows: the grey stream is cut into whole windows of WEFAX_FM_TONE_WINDOW samples (0.2 s).  With u = clip(grey,
+ * 0, 1), window mean mu and variance V = mean((u - mu)^2), r_f = 2 |sum_j (u_j - mu) exp(-2 pi i f j / 11025)|^2 /
+ * (T^2 V) is the share of V in the line at f = 300, 450, 675 Hz (1 for a sinusoid, 8 / pi^2 for a square wave; 0 when
+ * V = 0).  A window is START_576 / STOP / START_288 when r_300 / r_450 / r_675 is the largest of the three, that
+ * largest r >= WEFAX_FM_TONE_MIN_RATIO and V >= WEFAX_FM_TONE_MIN_VAR; otherwise NONE.
+ * Charts: a run is >= WEFAX_FM_TONE_MIN_RUN consecutive windows of one class, taken at its full length.  A start run
+ * opens a chart (tone_begin = its first sample, search_from = the sample after it); the chart ends at the first later
+ * STOP run (image_end = its first sample, stop_found = 1), at the next start run (which opens the next chart), or at
+ * the end of the recording.  A STOP run with no chart open is ignored.
+ * LPM: for each candidate c, the phasing fold of fold_lines lines of 60 / c * 11025 samples from search_from (the
+ * index of the plain decode's fold) scores (best circular boxcar of 5 % of a line) / (boxcar width * lines) - (fold
+ * mean) / lines; the highest score wins (the first listed on ties).  Below WEFAX_FM_LPM_MIN_SCORE the chart has status
+ * WEFAX_FM_CHART_NO_LPM and no picture. */
+#define WEFAX_FM_TONE_WINDOW 2205
+#define WEFAX_FM_TONE_MIN_RATIO 0.5
+#define WEFAX_FM_TONE_MIN_VAR 0.01
+#define WEFAX_FM_TONE_MIN_RUN 10
+#define WEFAX_FM_LPM_MIN_SCORE 0.3
+#define WEFAX_FM_MAX_LPM_CANDIDATES 8   /* each within [60, 240] LPM */
+
+#define WEFAX_FM_TONE_NONE 0
+#define WEFAX_FM_TONE_START_576 1
+#define WEFAX_FM_TONE_STOP 2
+#define WEFAX_FM_TONE_START_288 3
+
+#define WEFAX_FM_CHART_OK 0
+#define WEFAX_FM_CHART_NO_LPM 1         /* no candidate reached WEFAX_FM_LPM_MIN_SCORE: reported, not decoded */
+
+typedef struct {
+    wefax_fm_params fm;       /* lpm / ioc: 0 = detect per chart, > 0 = that value for every chart (IOC 576 and 288
+                                 start tones both open charts); search_from / image_end are ignored              */
+    wefax_fm_slant slant;     /* applies to every chart                                                           */
+    int n_lpm_candidates;     /* 0: the standard 60, 90, 100, 120, 180, 240                                       */
+    double lpm_candidates[WEFAX_FM_MAX_LPM_CANDIDATES];
+} wefax_fm_chart_params;
+
+typedef struct {
+    int64_t tone_begin;       /* first sample (at 11025 Hz) of the start tone run                                */
+    int64_t search_from;      /* sample after the start tone run: the phasing search starts here                 */
+    int64_t image_end;        /* first sample of the stop tone run, of the next start tone run, or n_out         */
+    int32_t stop_found;       /* 1: image_end is a stop tone                                                     */
+    int32_t ioc;              /* 576 or 288 from the start tone (or the forced value)                            */
+    double lpm;               /* the best candidate (or the forced value)                                        */
+    double lpm_score;         /* its score (0 when the LPM is forced)                                            */
+    int32_t status;           /* WEFAX_FM_CHART_*                                                                */
+    int32_t rows, width;      /* the picture: rows x width bytes at images + image_offset (rows 0: none)         */
+    int64_t line_start;       /* sample of the first picture line (-1: no picture decoded)                       */
+    int64_t image_offset;
+    wefax_fm_slant_out slant; /* as wefax_decode_fm_slant reports it                                             */
+} wefax_fm_chart;
+
+/* Every chart of one recording, from one band-pass / Hilbert / discriminator pass: tone windows, charts, each
+ * chart's IOC and LPM, then for each of the first max_charts charts (status OK) the picture exactly as
+ * wefax_decode_fm_slant computes it with that chart's lpm, ioc, search_from and image_end.  desc / pcm / flags as for
+ * wefax_decode_fm (WEFAX_F_PCM_FLOAT32 is rejected).  charts: HOST array of max_charts entries; *n_charts (HOST) = the
+ * number of charts found, also when it is above max_charts.  images: the pictures back to back (host, or device under
+ * WEFAX_F_OUT_ON_DEVICE), or NULL for the chart list only (no pictures, line_start -1); image_capacity must hold
+ * sum over the decoded charts of floor((image_end - search_from) / shortest line) * width bytes (the shortest line as
+ * wefax_decode_fm_slant sizes its image), else WEFAX_ERR_INVALID naming the bytes needed.  Optional outputs (host or
+ * device as images): tone_scores, n_out / WEFAX_FM_TONE_WINDOW windows x (r_300, r_450, r_675, V) floats; grey,
+ * n_out floats. */
+int wefax_decode_fm_charts(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                           const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts,
+                           int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores, float *grey);
+
 #ifdef __cplusplus
 }
 #endif

@@ -29,7 +29,7 @@ EXPORTED_SYMBOLS = (
     "wefax_ctx_enable_timing", "wefax_ctx_timings", "wefax_tone_scan", "wefax_decode_fm",
     "wefax_segment_envelope", "wefax_segment_histogram", "wefax_segment_quantise", "wefax_segment_sync",
     "wefax_segment_raster", "wefax_sync_pulse_scan", "wefax_segment_select_init", "wefax_segment_histogram_dev",
-    "wefax_segment_select_dev", "wefax_segment_quantise_dev", "wefax_decode_fm_slant",
+    "wefax_segment_select_dev", "wefax_segment_quantise_dev", "wefax_decode_fm_slant", "wefax_decode_fm_charts",
 )
 ABI_VERSION = 5
 
@@ -93,6 +93,27 @@ class FmSlantOut(C.Structure):
     _fields_ = [("line_length", C.c_double), ("ppm", C.c_double), ("first_line", C.c_double),
                 ("lines_total", C.c_int32), ("lines_used", C.c_int32), ("residual_rms", C.c_double),
                 ("status", C.c_int32)]
+
+
+FM_TONE_WINDOW = 2205
+FM_TONE_MIN_RATIO, FM_TONE_MIN_VAR, FM_TONE_MIN_RUN = 0.5, 0.01, 10
+FM_LPM_MIN_SCORE = 0.3
+FM_MAX_LPM_CANDIDATES = 8
+FM_STANDARD_LPMS = (60.0, 90.0, 100.0, 120.0, 180.0, 240.0)
+FM_TONE_NONE, FM_TONE_START_576, FM_TONE_STOP, FM_TONE_START_288 = 0, 1, 2, 3
+FM_CHART_OK, FM_CHART_NO_LPM = 0, 1
+
+
+class FmChartParams(C.Structure):
+    _fields_ = [("fm", FmParams), ("slant", FmSlant), ("n_lpm_candidates", C.c_int),
+                ("lpm_candidates", C.c_double * FM_MAX_LPM_CANDIDATES)]
+
+
+class FmChart(C.Structure):
+    _fields_ = [("tone_begin", C.c_int64), ("search_from", C.c_int64), ("image_end", C.c_int64),
+                ("stop_found", C.c_int32), ("ioc", C.c_int32), ("lpm", C.c_double), ("lpm_score", C.c_double),
+                ("status", C.c_int32), ("rows", C.c_int32), ("width", C.c_int32), ("line_start", C.c_int64),
+                ("image_offset", C.c_int64), ("slant", FmSlantOut)]
 
 
 class NativeLibraryMissing(RuntimeError):
@@ -167,6 +188,9 @@ def load():
     lib.wefax_decode_fm_slant.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmParams), C.POINTER(FmSlant),
                                           C.POINTER(FmOut), C.POINTER(FmSlantOut)]
     lib.wefax_decode_fm_slant.restype = i
+    lib.wefax_decode_fm_charts.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmChartParams), vp, i,
+                                           C.POINTER(i), vp, ll, vp, vp]
+    lib.wefax_decode_fm_charts.restype = i
     lib.wefax_segment_envelope.argtypes = [vp, C.POINTER(BatchDesc), vp, ll, ll, ll, ll]
     lib.wefax_segment_envelope.restype = i
     lib.wefax_segment_histogram.argtypes = [vp, i, C.POINTER(C.c_uint32 * 4), vp]

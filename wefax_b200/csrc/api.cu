@@ -506,6 +506,159 @@ void slant_search(wefax_ctx *ctx, const float *g, long long n, long long from, c
     res.residual_rms = fit.rms;
 }
 
+// ---- FM decode: the stages every FM entry point shares ----
+
+// the caller's slant parameters with their defaults filled in
+wefax_fm_slant checked_slant(const wefax_fm_slant &slant) {
+    wefax_fm_slant sp = slant;
+    if (sp.mode == WEFAX_FM_SLANT_FIXED) {
+        if (!(fabs(sp.ppm) <= 2000.0)) WEFAX_THROW(WEFAX_ERR_INVALID, "slant ppm must be within +-2000");
+    } else if (sp.mode == WEFAX_FM_SLANT_AUTO) {
+        if (sp.min_contrast == 0.0) sp.min_contrast = 0.3;
+        if (sp.min_lines == 0) sp.min_lines = 8;
+        if (!(sp.max_ppm > 0.0 && sp.max_ppm <= 2000.0))
+            WEFAX_THROW(WEFAX_ERR_INVALID, "max_ppm must be in (0, 2000]");
+        if (!(sp.min_contrast > 0.0 && sp.min_contrast <= 1.0) || sp.min_lines < 2)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "min_contrast must be in (0, 1] and min_lines >= 2");
+    } else if (sp.mode != WEFAX_FM_SLANT_OFF) {
+        WEFAX_THROW(WEFAX_ERR_INVALID, "unknown slant mode %d", sp.mode);
+    }
+    return sp;
+}
+
+// One picture's line lengths: the one FIXED uses (OFF: Ls) and the shortest one the mode may use, which sizes the
+// picture to rows_max rows
+struct FmGeometry {
+    double Ls, Ls_fixed, Ls_min;
+    int W, rows_max;
+};
+
+FmGeometry fm_geometry(double lpm, int ioc, const wefax_fm_slant &sp, long long from, long long image_end) {
+    FmGeometry f;
+    f.Ls = 60.0 / lpm * (double)WEFAX_TARGET_RATE;   // exact (fractional) samples per line
+    f.W = (int)llround(M_PI * (double)ioc);
+    f.Ls_fixed = sp.mode == WEFAX_FM_SLANT_FIXED ? f.Ls / (1.0 + sp.ppm * 1e-6) : f.Ls;
+    f.Ls_min = sp.mode == WEFAX_FM_SLANT_AUTO ? f.Ls / (1.0 + sp.max_ppm * 1e-6) : f.Ls_fixed;
+    f.rows_max = (int)std::max<long long>(0, (long long)floor((double)(image_end - from) / f.Ls_min));
+    return f;
+}
+
+// Band-pass, analytic signal and discriminator of one recording: the grey stream, n samples at 11025 Hz, in g_out
+// when it is not null (a device buffer), else in work_z
+float *fm_front_end(wefax_ctx *ctx, const wefax_batch_desc &desc, const int16_t *pcm, const wefax_fm_params &prm,
+                    long long n, float *g_out) {
+    cudaStream_t st = ctx->stream;
+    const FirParams fp = make_bandpass_fir(prm.band_lo_hz, prm.band_hi_hz, (double)WEFAX_TARGET_RATE, prm.fir_taps);
+    // the transform runs on the next even length whose half is smooth (zero padded)
+    long long half_len = next_smooth_length((n + 1) / 2);
+    FftPlan *half = half_len > 0 ? get_plan(ctx, half_len) : nullptr;
+    if (!half) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
+    const long long npad = 2 * half_len;
+
+    const void *d_pcm = upload_pcm(ctx, pcm, (size_t)desc.n_frames * desc.channels, desc.flags, false);
+    float *x = (float *)ctx->work_a.reserve((size_t)npad * sizeof(float));
+    float *y = (float *)ctx->work_e.reserve((size_t)npad * sizeof(float));
+    if (npad > n) CUDA_CHECK(cudaMemsetAsync(x + n, 0, (size_t)(npad - n) * sizeof(float), st));
+    const NotchInput in = notch_input(ctx, desc, d_pcm, n, 1);
+    launch_filtfilt(ctx, in.mode, in.x, in.stride, x, (size_t)npad, nullptr, 0, n, fp, 1);
+    float2 *z = (float2 *)ctx->work_z.reserve((size_t)half_len * sizeof(float2));
+    hilbert_envelope_real(ctx, half, x, (size_t)npad, z, (size_t)half_len, y, (size_t)npad, 1, /*want_y=*/true);
+    float *g = g_out ? g_out : (float *)ctx->work_z.reserve((size_t)n * sizeof(float));
+    launch_fm_grey(ctx, x, y, g, n, prm.black_hz, prm.white_hz);
+    return g;
+}
+
+// One picture from the grey stream g: line start from the phasing fold (or the slant search), then rows_max rows of
+// fg.W pixels into the device buffer d_img (null: no picture).  Synchronises the context's stream; returns the line
+// start, the rows written (floor((image_end - line_start) / line length), at most rows_max) and the slant report.
+struct FmPicture {
+    long long line_start;
+    int rows;
+    wefax_fm_slant_out so;
+};
+
+FmPicture fm_picture(wefax_ctx *ctx, const float *g, long long n, long long from, long long image_end,
+                     const FmGeometry &fg, int fold_lines, const wefax_fm_slant &sp, uint8_t *d_img) {
+    cudaStream_t st = ctx->stream;
+    const int Lc = (int)ceil(fg.Ls_fixed);
+    char *small = (char *)ctx->out_small.reserve((size_t)Lc * sizeof(float) + 64);
+    long long *d_ls = (long long *)small;
+    float *P = (float *)(small + 64);
+
+    FmPicture pic;
+    wefax_fm_slant_out &so = pic.so;
+    memset(&so, 0, sizeof(so));
+    so.status = WEFAX_FM_SLANT_OK;
+    double line_length = fg.Ls_fixed;
+    bool fitted = false;
+    if (sp.mode == WEFAX_FM_SLANT_AUTO) {
+        slant_search(ctx, g, n, from, slant_geometry(fg.Ls, from, image_end, sp.max_ppm), sp, so);
+        if (so.status == WEFAX_FM_SLANT_OK) {
+            const long long ls = llround(so.first_line);
+            CUDA_CHECK(cudaMemcpyAsync(d_ls, &ls, sizeof(long long), cudaMemcpyHostToDevice, st));
+            line_length = so.line_length;
+            fitted = true;
+        }
+    } else if (sp.mode == WEFAX_FM_SLANT_FIXED) {
+        so.ppm = sp.ppm;
+    }
+    if (!fitted) launch_fm_phasing(ctx, g, n, from, line_length, fold_lines, P, d_ls);
+    if (d_img && fg.rows_max > 0) launch_fm_image(ctx, g, n, d_ls, line_length, fg.W, fg.rows_max, image_end, d_img);
+    long long *h_ls = (long long *)pinned(ctx, 64);
+    CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, sizeof(long long), cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    pic.line_start = *h_ls;
+    pic.rows = (int)std::min<long long>(
+        fg.rows_max, std::max<long long>(0, (long long)floor((double)(image_end - pic.line_start) / line_length)));
+    if (!fitted) {
+        so.line_length = line_length;
+        so.first_line = (double)pic.line_start;
+    }
+    return pic;
+}
+
+// ---- charts of a recording (DESIGN.md §4.7b; float64 restatement: tests/fm_charts_oracle.py) ----
+
+int tone_class(const float *s) {   // s = (r_300, r_450, r_675, V) of one window
+    int k = 0;
+    for (int f = 1; f < 3; ++f)
+        if (s[f] > s[k]) k = f;
+    if (!(s[k] >= WEFAX_FM_TONE_MIN_RATIO && s[3] >= WEFAX_FM_TONE_MIN_VAR)) return WEFAX_FM_TONE_NONE;
+    static const int cls[3] = {WEFAX_FM_TONE_START_576, WEFAX_FM_TONE_STOP, WEFAX_FM_TONE_START_288};
+    return cls[k];
+}
+
+std::vector<wefax_fm_chart> find_charts(const std::vector<int> &cls, long long n) {
+    std::vector<wefax_fm_chart> charts;
+    const long long T = WEFAX_FM_TONE_WINDOW, nw = (long long)cls.size();
+    bool open = false;
+    for (long long k = 0; k < nw;) {
+        long long e = k + 1;
+        while (e < nw && cls[e] == cls[k]) ++e;
+        const int c = cls[k];
+        if (e - k >= WEFAX_FM_TONE_MIN_RUN && c != WEFAX_FM_TONE_NONE) {
+            if (open) {
+                charts.back().image_end = k * T;
+                charts.back().stop_found = c == WEFAX_FM_TONE_STOP;
+                open = false;
+            }
+            if (c != WEFAX_FM_TONE_STOP) {
+                wefax_fm_chart ch;
+                memset(&ch, 0, sizeof(ch));
+                ch.tone_begin = k * T;
+                ch.search_from = e * T;
+                ch.ioc = c == WEFAX_FM_TONE_START_576 ? 576 : 288;
+                ch.line_start = -1;
+                charts.push_back(ch);
+                open = true;
+            }
+        }
+        k = e;
+    }
+    if (open) charts.back().image_end = n;
+    return charts;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1409,105 +1562,151 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
         if (!(prm->lpm > 0.0) || prm->ioc < 1 || !(prm->white_hz > prm->black_hz) || prm->fold_lines < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
-        wefax_fm_slant sp = *slant;
-        if (sp.mode == WEFAX_FM_SLANT_FIXED) {
-            if (!(fabs(sp.ppm) <= 2000.0)) WEFAX_THROW(WEFAX_ERR_INVALID, "slant ppm must be within +-2000");
-        } else if (sp.mode == WEFAX_FM_SLANT_AUTO) {
-            if (sp.min_contrast == 0.0) sp.min_contrast = 0.3;
-            if (sp.min_lines == 0) sp.min_lines = 8;
-            if (!(sp.max_ppm > 0.0 && sp.max_ppm <= 2000.0))
-                WEFAX_THROW(WEFAX_ERR_INVALID, "max_ppm must be in (0, 2000]");
-            if (!(sp.min_contrast > 0.0 && sp.min_contrast <= 1.0) || sp.min_lines < 2)
-                WEFAX_THROW(WEFAX_ERR_INVALID, "min_contrast must be in (0, 1] and min_lines >= 2");
-        } else if (sp.mode != WEFAX_FM_SLANT_OFF) {
-            WEFAX_THROW(WEFAX_ERR_INVALID, "unknown slant mode %d", sp.mode);
-        }
+        const wefax_fm_slant sp = checked_slant(*slant);
         use_device(ctx);
         cudaStream_t st = ctx->stream;
         const long long n_in = desc->n_frames;
-        const int ch = desc->channels;
         const bool resample = desc->sample_rate != WEFAX_TARGET_RATE;
         const long long n = resample ? wefax_resampled_length(n_in, desc->sample_rate) : n_in;
         if (n < 64) WEFAX_THROW(WEFAX_ERR_INVALID, "recording too short");
         const bool out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE;
-        const double Ls = 60.0 / prm->lpm * (double)WEFAX_TARGET_RATE;   // exact (fractional) samples per line
-        const int W = (int)llround(M_PI * (double)prm->ioc);
         const long long image_end = (prm->image_end > 0 && prm->image_end <= n) ? prm->image_end : n;
         const long long from = std::max<long long>(0, std::min<long long>(prm->search_from, n - 1));
-        // the line length FIXED uses, and the shortest one AUTO may find: it sizes the image
-        const double Ls_fixed = sp.mode == WEFAX_FM_SLANT_FIXED ? Ls / (1.0 + sp.ppm * 1e-6) : Ls;
-        const double Ls_min = sp.mode == WEFAX_FM_SLANT_AUTO ? Ls / (1.0 + sp.max_ppm * 1e-6) : Ls_fixed;
-        const int rows_max = (int)std::max<long long>(0, (long long)floor((double)(image_end - from) / Ls_min));
-        if (out->image && (long long)rows_max * W > out->image_capacity)
+        const FmGeometry fg = fm_geometry(prm->lpm, prm->ioc, sp, from, image_end);
+        if (out->image && (long long)fg.rows_max * fg.W > out->image_capacity)
             WEFAX_THROW(WEFAX_ERR_INVALID, "image_capacity %lld too small (need %lld)", out->image_capacity,
-                        (long long)rows_max * W);
-        const FirParams fp = make_bandpass_fir(prm->band_lo_hz, prm->band_hi_hz, (double)WEFAX_TARGET_RATE, prm->fir_taps);
-
-        // the transform runs on the next even length whose half is smooth (zero padded)
-        long long half_len = next_smooth_length((n + 1) / 2);
-        FftPlan *half = half_len > 0 ? get_plan(ctx, half_len) : nullptr;
-        if (!half) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
-        const long long npad = 2 * half_len;
-
-        const void *d_pcm = upload_pcm(ctx, pcm, (size_t)n_in * ch, desc->flags, false);
-        float *x = (float *)ctx->work_a.reserve((size_t)npad * sizeof(float));
-        float *y = (float *)ctx->work_e.reserve((size_t)npad * sizeof(float));
-        if (npad > n) CUDA_CHECK(cudaMemsetAsync(x + n, 0, (size_t)(npad - n) * sizeof(float), st));
-        const NotchInput in = notch_input(ctx, *desc, d_pcm, n, 1);
-        launch_filtfilt(ctx, in.mode, in.x, in.stride, x, (size_t)npad, nullptr, 0, n, fp, 1);
-        float2 *z = (float2 *)ctx->work_z.reserve((size_t)half_len * sizeof(float2));
-        hilbert_envelope_real(ctx, half, x, (size_t)npad, z, (size_t)half_len, y, (size_t)npad, 1, /*want_y=*/true);
+                        (long long)fg.rows_max * fg.W);
 
         // grey stream (in the transform scratch, or straight into the caller's device buffer)
-        float *g = (out_dev && out->grey) ? out->grey : (float *)ctx->work_z.reserve((size_t)n * sizeof(float));
-        launch_fm_grey(ctx, x, y, g, n, prm->black_hz, prm->white_hz);
-        const int Lc = (int)ceil(Ls_fixed);
-        char *small = (char *)ctx->out_small.reserve((size_t)Lc * sizeof(float) + 64);
-        long long *d_ls = (long long *)small;
-        float *P = (float *)(small + 64);
-
-        wefax_fm_slant_out so;
-        memset(&so, 0, sizeof(so));
-        so.status = WEFAX_FM_SLANT_OK;
-        double line_length = Ls_fixed;
-        bool fitted = false;
-        if (sp.mode == WEFAX_FM_SLANT_AUTO) {
-            slant_search(ctx, g, n, from, slant_geometry(Ls, from, image_end, sp.max_ppm), sp, so);
-            if (so.status == WEFAX_FM_SLANT_OK) {
-                const long long ls = llround(so.first_line);
-                CUDA_CHECK(cudaMemcpyAsync(d_ls, &ls, sizeof(long long), cudaMemcpyHostToDevice, st));
-                line_length = so.line_length;
-                fitted = true;
-            }
-        } else if (sp.mode == WEFAX_FM_SLANT_FIXED) {
-            so.ppm = sp.ppm;
-        }
-        if (!fitted) launch_fm_phasing(ctx, g, n, from, line_length, prm->fold_lines, P, d_ls);
-        uint8_t *d_img = nullptr;
-        if (out->image && rows_max > 0) {
-            d_img = out_dev ? out->image : (uint8_t *)ctx->out_raster.reserve((size_t)rows_max * W);
-            launch_fm_image(ctx, g, n, d_ls, line_length, W, rows_max, image_end, d_img);
-        }
-        long long *h_ls = (long long *)pinned(ctx, 64);
-        CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        const float *g = fm_front_end(ctx, *desc, pcm, *prm, n, (out_dev && out->grey) ? out->grey : nullptr);
         if (!out_dev && out->grey)
             CUDA_CHECK(cudaMemcpyAsync(out->grey, g, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-        const long long line_start = *h_ls;
-        const int rows = (int)std::min<long long>(
-            rows_max, std::max<long long>(0, (long long)floor((double)(image_end - line_start) / line_length)));
-        if (!out_dev && d_img && rows > 0)
-            CUDA_CHECK(cudaMemcpy(out->image, d_img, (size_t)rows * W, cudaMemcpyDeviceToHost));
-        if (out->rows) *out->rows = rows;
-        if (out->width) *out->width = W;
-        if (out->line_start) *out->line_start = line_start;
-        if (slant_out) {
-            if (!fitted) {
-                so.line_length = line_length;
-                so.first_line = (double)line_start;
-            }
-            *slant_out = so;
+        uint8_t *d_img = nullptr;
+        if (out->image && fg.rows_max > 0)
+            d_img = out_dev ? out->image : (uint8_t *)ctx->out_raster.reserve((size_t)fg.rows_max * fg.W);
+        const FmPicture pic = fm_picture(ctx, g, n, from, image_end, fg, prm->fold_lines, sp, d_img);
+        if (!out_dev && d_img && pic.rows > 0)
+            CUDA_CHECK(cudaMemcpy(out->image, d_img, (size_t)pic.rows * fg.W, cudaMemcpyDeviceToHost));
+        if (out->rows) *out->rows = pic.rows;
+        if (out->width) *out->width = fg.W;
+        if (out->line_start) *out->line_start = pic.line_start;
+        if (slant_out) *slant_out = pic.so;
+    });
+}
+
+int wefax_decode_fm_charts(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                           const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts, int *n_charts,
+                           uint8_t *images, long long image_capacity, float *tone_scores, float *grey) {
+    if (!ctx) return WEFAX_ERR_INVALID;
+    return guarded(ctx, [&] {
+        if (!desc || !pcm || !params || !n_charts || max_charts < 0 || (max_charts > 0 && !charts) ||
+            desc->n_recordings != 1 || desc->n_frames < 64 || (desc->channels != 1 && desc->channels != 2) ||
+            desc->sample_rate < 1)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
+        const wefax_fm_params &prm = params->fm;
+        if (!(prm.lpm >= 0.0) || prm.ioc < 0 || !(prm.white_hz > prm.black_hz) || prm.fold_lines < 1)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
+        const wefax_fm_slant sp = checked_slant(params->slant);
+        static const double kStandardLpm[] = {60.0, 90.0, 100.0, 120.0, 180.0, 240.0};
+        const int n_cand = params->n_lpm_candidates ? params->n_lpm_candidates : 6;
+        const double *cand_lpm = params->n_lpm_candidates ? params->lpm_candidates : kStandardLpm;
+        if (n_cand < 1 || n_cand > WEFAX_FM_MAX_LPM_CANDIDATES)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "1 to %d LPM candidates, not %d", WEFAX_FM_MAX_LPM_CANDIDATES, n_cand);
+        LpmCandidates cand;
+        memset(&cand, 0, sizeof(cand));
+        cand.n = n_cand;
+        for (int c = 0; c < n_cand; ++c) {
+            if (!(cand_lpm[c] >= 60.0 && cand_lpm[c] <= 240.0))
+                WEFAX_THROW(WEFAX_ERR_INVALID, "LPM candidate %g is outside [60, 240]", cand_lpm[c]);
+            cand.Ls[c] = 60.0 / cand_lpm[c] * (double)WEFAX_TARGET_RATE;
+            cand.Lc[c] = (int)ceil(cand.Ls[c]);
+            cand.wb[c] = std::max(1, (int)llround(0.05 * cand.Ls[c]));
         }
+        use_device(ctx);
+        cudaStream_t st = ctx->stream;
+        const long long n_in = desc->n_frames;
+        const long long n = desc->sample_rate != WEFAX_TARGET_RATE ? wefax_resampled_length(n_in, desc->sample_rate) : n_in;
+        if (n < 64) WEFAX_THROW(WEFAX_ERR_INVALID, "recording too short");
+        const bool out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE;
+        const float *g = fm_front_end(ctx, *desc, pcm, prm, n, (out_dev && grey) ? grey : nullptr);
+        if (!out_dev && grey)
+            CUDA_CHECK(cudaMemcpyAsync(grey, g, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
+
+        // tone windows -> charts
+        const long long nw = n / WEFAX_FM_TONE_WINDOW;
+        const size_t tone_bytes = (size_t)nw * sizeof(float4);
+        float4 *d_tone = (float4 *)ctx->work_misc.reserve(tone_bytes + 16);
+        launch_fm_tone(ctx, g, nw, d_tone);
+        if (out_dev && tone_scores && nw > 0)
+            CUDA_CHECK(cudaMemcpyAsync(tone_scores, d_tone, tone_bytes, cudaMemcpyDeviceToDevice, st));
+        float *h_tone = (float *)pinned(ctx, tone_bytes + 16);
+        if (nw > 0) CUDA_CHECK(cudaMemcpyAsync(h_tone, d_tone, tone_bytes, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        if (!out_dev && tone_scores && nw > 0) memcpy(tone_scores, h_tone, tone_bytes);
+        std::vector<int> cls((size_t)nw);
+        for (long long k = 0; k < nw; ++k) cls[k] = tone_class(h_tone + 4 * k);
+        std::vector<wefax_fm_chart> found = find_charts(cls, n);
+        *n_charts = (int)found.size();
+        const int nc = (int)std::min<long long>((long long)found.size(), max_charts);
+
+        // LPM of each chart from its phasing lines (one launch for all charts and candidates)
+        for (int i = 0; i < nc; ++i) {
+            found[i].lpm = prm.lpm;
+            if (prm.ioc > 0) found[i].ioc = prm.ioc;
+        }
+        if (!(prm.lpm > 0.0) && nc > 0) {
+            std::vector<long long> from(nc);
+            for (int i = 0; i < nc; ++i) from[i] = std::min<long long>(found[i].search_from, n - 1);
+            char *buf = (char *)ctx->work_misc.reserve((size_t)nc * sizeof(long long) + (size_t)nc * n_cand * sizeof(double));
+            long long *d_from = (long long *)buf;
+            double *d_score = (double *)(buf + (size_t)nc * sizeof(long long));
+            CUDA_CHECK(cudaMemcpyAsync(d_from, from.data(), (size_t)nc * sizeof(long long), cudaMemcpyHostToDevice, st));
+            launch_fm_lpm(ctx, g, n, d_from, nc, cand, prm.fold_lines, d_score);
+            double *h_score = (double *)pinned(ctx, (size_t)nc * n_cand * sizeof(double));
+            CUDA_CHECK(cudaMemcpyAsync(h_score, d_score, (size_t)nc * n_cand * sizeof(double), cudaMemcpyDeviceToHost, st));
+            CUDA_CHECK(cudaStreamSynchronize(st));
+            for (int i = 0; i < nc; ++i) {
+                int best = 0;
+                for (int c = 1; c < n_cand; ++c)
+                    if (h_score[(size_t)i * n_cand + c] > h_score[(size_t)i * n_cand + best]) best = c;
+                found[i].lpm = cand_lpm[best];
+                found[i].lpm_score = h_score[(size_t)i * n_cand + best];
+                if (found[i].lpm_score < WEFAX_FM_LPM_MIN_SCORE) found[i].status = WEFAX_FM_CHART_NO_LPM;
+            }
+        }
+
+        // each chart's picture: the tail of the single-picture decode on the shared grey stream
+        std::vector<FmGeometry> geo(nc);
+        long long need = 0;
+        for (int i = 0; i < nc; ++i) {
+            wefax_fm_chart &ch = found[i];
+            const long long from = std::min<long long>(ch.search_from, n - 1);
+            geo[i] = fm_geometry(ch.lpm, ch.ioc, sp, from, ch.image_end);
+            ch.width = geo[i].W;
+            if (ch.status == WEFAX_FM_CHART_OK) need += (long long)geo[i].rows_max * geo[i].W;
+        }
+        if (images && need > image_capacity)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "image_capacity %lld too small (need %lld)", image_capacity, need);
+        long long offset = 0;
+        for (int i = 0; i < nc; ++i) {
+            wefax_fm_chart &ch = found[i];
+            ch.image_offset = offset;
+            if (!images || ch.status != WEFAX_FM_CHART_OK) continue;
+            const FmGeometry &fg = geo[i];
+            uint8_t *d_img = nullptr;
+            if (fg.rows_max > 0)
+                d_img = out_dev ? images + offset : (uint8_t *)ctx->out_raster.reserve((size_t)fg.rows_max * fg.W);
+            const long long from = std::min<long long>(ch.search_from, n - 1);
+            const FmPicture pic = fm_picture(ctx, g, n, from, ch.image_end, fg, prm.fold_lines, sp, d_img);
+            if (!out_dev && d_img && pic.rows > 0)
+                CUDA_CHECK(cudaMemcpy(images + offset, d_img, (size_t)pic.rows * fg.W, cudaMemcpyDeviceToHost));
+            ch.rows = pic.rows;
+            ch.line_start = pic.line_start;
+            ch.slant = pic.so;
+            offset += (long long)pic.rows * fg.W;
+        }
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        for (int i = 0; i < nc; ++i) charts[i] = found[i];
     });
 }
 

@@ -285,6 +285,132 @@ fm_slant_track_kernel(const float *g, long long n, double a, double s, int wb, i
     }
 }
 
+// ---- charts of a recording: tone windows and the LPM from the phasing lines (DESIGN.md §4.7b) ----
+
+// sum of K values over the CTA (every thread gets the totals); s: 32 * K doubles of shared memory
+template <int K>
+__device__ __forceinline__ void block_sum(double (&v)[K], double *s) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = (blockDim.x + 31) / 32;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+        for (int d = 16; d; d >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], d);
+    if (lane == 0)
+#pragma unroll
+        for (int k = 0; k < K; ++k) s[warp * K + k] = v[k];
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        double t = 0.0;
+        for (int w = 0; w < nw; ++w) t += s[w * K + k];
+        v[k] = t;
+    }
+    __syncthreads();
+}
+
+// One CTA per whole window k of T samples: u = clip(grey), mu = mean, V = mean((u - mu)^2),
+// C_f = sum_j (u_j - mu) exp(-2 pi i f j / 11025) for f = 300, 450, 675 Hz with the phase from the exact integer
+// (f * j) mod 11025, r_f = 2 |C_f|^2 / (T^2 V) (0 when V = 0).  out[k] = (r_300, r_450, r_675, V)
+constexpr int kToneThreads = 256;
+__global__ void __launch_bounds__(kToneThreads)
+fm_tone_kernel(const float *g, float4 *out) {
+    constexpr int T = WEFAX_FM_TONE_WINDOW;
+    constexpr int F[3] = {300, 450, 675};
+    __shared__ float u[T];
+    __shared__ double s_red[32 * 7];
+    const float *w = g + (size_t)blockIdx.x * T;
+    double m[1] = {0.0};
+    for (int j = threadIdx.x; j < T; j += blockDim.x) {
+        const float v = clip01(__ldg(w + j));
+        u[j] = v;
+        m[0] += (double)v;
+    }
+    block_sum<1>(m, s_red);    // (its barrier also publishes u)
+    const double mu = m[0] / T;
+    double a[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};   // sum d^2, then (re, im) of C_300, C_450, C_675
+    for (int j = threadIdx.x; j < T; j += blockDim.x) {
+        const double d = (double)u[j] - mu;
+        a[0] += d * d;
+#pragma unroll
+        for (int f = 0; f < 3; ++f) {
+            float sn, cs;
+            sincospif((float)(2 * ((F[f] * j) % WEFAX_TARGET_RATE)) / (float)WEFAX_TARGET_RATE, &sn, &cs);
+            a[1 + 2 * f] += d * (double)cs;
+            a[2 + 2 * f] -= d * (double)sn;
+        }
+    }
+    block_sum<7>(a, s_red);
+    if (threadIdx.x == 0) {
+        float r[3];
+#pragma unroll
+        for (int f = 0; f < 3; ++f)
+            r[f] = a[0] > 0.0 ? (float)(2.0 * (a[1 + 2 * f] * a[1 + 2 * f] + a[2 + 2 * f] * a[2 + 2 * f]) / ((double)T * a[0]))
+                              : 0.f;
+        out[blockIdx.x] = make_float4(r[0], r[1], r[2], (float)(a[0] / T));
+    }
+}
+
+// One CTA per (chart, candidate): the phasing fold of fm_fold_kernel (same index, same float32 sums in line order) for
+// the candidate's line length from the chart's search_from, kept in shared memory, then
+// score = max_o sum_{j < wb} P[(o + j) mod Lc] / (wb * lines) - mean(P) / lines  (boxcar sums in float64)
+__global__ void __launch_bounds__(1024)
+fm_lpm_kernel(const float *g, long long n, const long long *from, LpmCandidates cand, int lines, double *score) {
+    __shared__ float P[kLpmMaxLine];
+    __shared__ double s_red[32 * 2];
+    const int chart = blockIdx.x / cand.n, c = blockIdx.x % cand.n, tid = threadIdx.x, nt = blockDim.x;
+    const double Ls = cand.Ls[c];
+    const int Lc = cand.Lc[c], wb = cand.wb[c];
+    const long long f0 = from[chart];
+    double tot[1] = {0.0};
+    for (int o = tid; o < Lc; o += nt) {
+        float acc = 0.f;
+        for (int l = 0; l < lines; ++l) {
+            const long long i = f0 + (long long)floor(__dadd_rn(__dmul_rn((double)l, Ls), (double)o));
+            if (i < n) acc += clip01(__ldg(g + i));
+        }
+        P[o] = acc;
+        tot[0] += (double)acc;
+    }
+    block_sum<1>(tot, s_red);   // (its barrier also publishes P)
+    // each thread slides the boxcar over a contiguous chunk of offsets
+    const int chunk = (Lc + nt - 1) / nt, b = tid * chunk, e = min(b + chunk, Lc);
+    double best = 0.0;
+    if (b < e) {
+        double box = 0.0;
+        for (int j = 0; j < wb; ++j) box += (double)P[(b + j) % Lc];
+        best = box;
+        for (int o = b + 1; o < e; ++o) {
+            box += (double)P[(o + wb - 1) % Lc] - (double)P[o - 1];
+            best = fmax(best, box);
+        }
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffffu, best, d));
+    if ((tid & 31) == 0) s_red[tid >> 5] = best;
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < (nt + 31) / 32; ++w) best = fmax(best, s_red[w]);
+        score[blockIdx.x] = best / ((double)wb * lines) - tot[0] / Lc / lines;
+    }
+}
+
+void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n_windows, float4 *out) {
+    if (n_windows <= 0) return;
+    StageTimer timer(ctx, "fm_tone");
+    fm_tone_kernel<<<(unsigned)n_windows, kToneThreads, 0, ctx->stream>>>(g, out);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+}
+
+void launch_fm_lpm(wefax_ctx *ctx, const float *g, long long n, const long long *d_from, int n_charts,
+                   const LpmCandidates &cand, int lines, double *d_score) {
+    if (n_charts <= 0) return;
+    StageTimer timer(ctx, "fm_lpm");
+    fm_lpm_kernel<<<(unsigned)(n_charts * cand.n), 1024, 0, ctx->stream>>>(g, n, d_from, cand, lines, d_score);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+}
+
 void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, float *g, long long n, double black_hz,
                     double white_hz) {
     StageTimer timer(ctx, "fm_grey");

@@ -145,5 +145,17 @@ void launch_fm_slant_fold(wefax_ctx *ctx, const float *Q, int lines, int Bn, int
 // pulse position (or -1) and contrast of lines [0, lines) around a + l * s, +-R samples, pulse width wb
 void launch_fm_slant_track(wefax_ctx *ctx, const float *g, long long n, double a, double s, int lines, int wb, int R,
                            double min_contrast, long long *pos, float *contrast);
+// charts (DESIGN.md §4.7b): (r_300, r_450, r_675, V) of each whole WEFAX_FM_TONE_WINDOW window of g into out
+void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n_windows, float4 *out);
+// the LPM candidates' line lengths Ls = 60 / lpm * 11025, Lc = ceil(Ls) <= kLpmMaxLine, boxcars wb = max(1, round(0.05 Ls))
+constexpr int kLpmMaxLine = 11025;
+struct LpmCandidates {
+    int n;
+    double Ls[WEFAX_FM_MAX_LPM_CANDIDATES];
+    int Lc[WEFAX_FM_MAX_LPM_CANDIDATES], wb[WEFAX_FM_MAX_LPM_CANDIDATES];
+};
+// phasing score of every (chart, candidate), chart-major, folding `lines` lines from d_from[chart] (device)
+void launch_fm_lpm(wefax_ctx *ctx, const float *g, long long n, const long long *d_from, int n_charts,
+                   const LpmCandidates &cand, int lines, double *d_score);
 
 }  // namespace wefax

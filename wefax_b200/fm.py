@@ -6,6 +6,11 @@ The reference never implemented what its README describes (README.md:85-101: bla
 (``csrc/fm.cu`` through ``wefax_decode_fm``): band-pass, analytic signal, instantaneous frequency,
 phasing-pulse line start, ``round(pi * IOC)`` pixels per line.  It is off the reference-exact path
 and has no reference parity; see ``oracle/fm_oracle.py`` and ``tests/test_gpu_fm.py``.
+
+:func:`decode_fm` decodes one picture whose LPM and IOC the caller knows.  Its default span comes from the AM path's
+tone test (:func:`image_span`), which finds only the first IOC 576 chart of a recording.  :func:`decode_fm_charts`
+finds every chart of a recording in the FM grey stream itself (start tones at 300 / 675 Hz, stop tone at 450 Hz),
+measures each chart's LPM from its phasing lines and decodes them all from one front end (``wefax_decode_fm_charts``).
 """
 from __future__ import annotations
 
@@ -44,6 +49,31 @@ class FmResult:
     image_end: int
     grey: np.ndarray | None = None     # per-sample grey before clipping (float32), when asked for
     slant: FmSlant | None = None       # with slant="auto" or a ppm value
+
+
+@dataclass
+class FmChart:
+    """One chart of a recording (``wefax_fm_chart``); positions are samples at 11025 Hz."""
+    tone_begin: int            # first sample of the start tone
+    search_from: int           # sample after the start tone: the phasing search starts here
+    image_end: int             # first sample of the stop tone, of the next start tone, or the end of the recording
+    stop_found: bool
+    ioc: int                   # 576 or 288 from the start tone (or the forced value)
+    lpm: float                 # from the phasing lines (or the forced value)
+    lpm_score: float           # the phasing score of that LPM (about 1 on a clean signal; 0 when the LPM is forced)
+    status: int                # N.FM_CHART_OK, or N.FM_CHART_NO_LPM (no LPM scored N.FM_LPM_MIN_SCORE: no picture)
+    width: int                 # round(pi * ioc)
+    line_start: int            # sample of the first picture line (-1: no picture decoded)
+    image: np.ndarray | None   # (rows, width) uint8; None when pictures were not asked for or status is not OK
+    slant: FmSlant | None = None
+
+
+@dataclass
+class FmCharts:
+    charts: list               # FmChart of the first max_charts charts, in recording order
+    n_found: int               # charts found (may exceed len(charts))
+    grey: np.ndarray | None = None          # per-sample grey (float32), when asked for
+    tone_scores: np.ndarray | None = None   # (windows, 4) float32: r_300, r_450, r_675, V per 0.2 s window
 
 
 def image_span(start_flags, stop_flags, sample_rate_out: int = N.TARGET_RATE, packet_seconds: float = 1.0):
@@ -94,7 +124,8 @@ def decode_fm(decoder, pcm, sample_rate: int, lpm: float = 120, ioc: int = 576, 
     """Decode one recording (int16 numpy, mono ``(n,)`` or stereo ``(n, 2)``).
 
     ``search_from`` / ``image_end`` (samples at 11025 Hz) default to what the start / stop tone scan
-    finds (:func:`image_span`).  ``slant`` corrects the recording's sample-clock error: ``"auto"`` measures
+    finds (:func:`image_span`).  That scan is the AM path's packet test: it finds only the first IOC 576 chart of a
+    recording (it misses the 675 Hz start tone); :func:`decode_fm_charts` finds every chart.  ``slant`` corrects the recording's sample-clock error: ``"auto"`` measures
     it from the white line pulses (within +-``max_slant_ppm``), a number is the error in ppm (what
     ``result.slant.ppm`` reported for an earlier decode); None decodes lines of exactly 60 / lpm s."""
     sp = slant_params(slant, max_slant_ppm)
@@ -133,6 +164,78 @@ def decode_fm(decoder, pcm, sample_rate: int, lpm: float = 120, ioc: int = 576, 
                     int(search_from), int(image_end), grey, so)
 
 
+def chart_params(lpm=None, ioc=None, lpm_candidates=None, slant=None, max_slant_ppm: float = 300.0,
+                 fold_lines: int = 20, black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0),
+                 fir_taps: int = 63):
+    """``N.FmChartParams`` for :func:`decode_fm_charts`; ValueError for arguments the library would refuse."""
+    def real(v):
+        return not isinstance(v, bool) and isinstance(v, numbers.Real) and math.isfinite(float(v))
+    if lpm is not None and not (real(lpm) and float(lpm) > 0):
+        raise ValueError(f"lpm must be None (detect) or a positive number, not {lpm!r}")
+    if ioc is not None and not (isinstance(ioc, numbers.Integral) and not isinstance(ioc, bool) and ioc > 0):
+        raise ValueError(f"ioc must be None (detect) or a positive integer, not {ioc!r}")
+    cands = N.FM_STANDARD_LPMS if lpm_candidates is None else tuple(lpm_candidates)
+    if not 1 <= len(cands) <= N.FM_MAX_LPM_CANDIDATES or not all(real(c) and 60 <= float(c) <= 240 for c in cands):
+        raise ValueError(f"lpm_candidates: 1 to {N.FM_MAX_LPM_CANDIDATES} values within [60, 240], not {lpm_candidates!r}")
+    if isinstance(fold_lines, bool) or not isinstance(fold_lines, numbers.Integral) or fold_lines < 1:
+        raise ValueError(f"fold_lines must be a positive integer, not {fold_lines!r}")
+    sp = slant_params(slant, max_slant_ppm) or N.FmSlant(N.FM_SLANT_OFF, 0.0, 0.0, 0.0, 0)
+    prm = N.FmParams(float(lpm or 0.0), int(ioc or 0), float(black_hz), float(white_hz), float(band[0]),
+                     float(band[1]), int(fir_taps), 0, int(fold_lines), 0)
+    arr = (C.c_double * N.FM_MAX_LPM_CANDIDATES)(*[float(c) for c in cands])
+    return N.FmChartParams(prm, sp, len(cands), arr)
+
+
+def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_candidates=None, slant=None,
+                     max_slant_ppm: float = 300.0, max_charts: int = 64, fold_lines: int = 20,
+                     black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0), fir_taps: int = 63,
+                     want_images: bool = True, want_grey: bool = False, want_tone_scores: bool = False,
+                     image_capacity: int | None = None) -> FmCharts:
+    """Find and decode every chart of a recording (int16 numpy, mono ``(n,)`` or stereo ``(n, 2)``).
+
+    Each chart starts at a start tone (300 Hz: IOC 576, 675 Hz: IOC 288) and ends at the stop tone, the next start
+    tone or the end of the recording; its LPM is the candidate (default 60, 90, 100, 120, 180, 240) whose phasing
+    fold shows the sharpest line pulse.  ``lpm`` / ``ioc`` force a value for every chart.  ``slant`` as for
+    :func:`decode_fm`, for every chart.  Each chart's picture equals ``decode_fm`` with that chart's lpm, ioc,
+    search_from and image_end.  ``want_images=False`` returns the chart list only; ``image_capacity`` overrides the
+    size of the picture buffer (bytes; default: enough for any recording of this length)."""
+    prm = chart_params(lpm, ioc, lpm_candidates, slant, max_slant_ppm, fold_lines, black_hz, white_hz, band, fir_taps)
+    if isinstance(max_charts, bool) or not isinstance(max_charts, numbers.Integral) or max_charts < 0:
+        raise ValueError(f"max_charts must be a non-negative integer, not {max_charts!r}")
+    pcm = np.ascontiguousarray(pcm, dtype=np.int16)
+    n_in, ch = int(pcm.shape[0]), (1 if pcm.ndim == 1 else int(pcm.shape[1]))
+    n_out = n_in if sample_rate == N.TARGET_RATE else N.resampled_length(n_in, sample_rate)
+    if image_capacity is None:
+        # the charts' spans are disjoint: ceil(n_out / shortest line) rows of the widest picture hold them all
+        ls_min = 60.0 / (float(lpm) if lpm else max(prm.lpm_candidates[: prm.n_lpm_candidates])) * N.TARGET_RATE
+        sp = prm.slant
+        if sp.mode != N.FM_SLANT_OFF:
+            ls_min = ls_min / (1.0 + (sp.max_ppm if sp.mode == N.FM_SLANT_AUTO else max(sp.ppm, 0.0)) * 1e-6)
+        w_max = int(round(math.pi * (ioc if ioc else 576)))
+        image_capacity = int(math.ceil(n_out / ls_min)) * w_max if want_images else 0
+    img = np.zeros(max(1, image_capacity), dtype=np.uint8) if want_images else None
+    grey = np.zeros(n_out, dtype=np.float32) if want_grey else None
+    tones = np.zeros((n_out // N.FM_TONE_WINDOW, 4), dtype=np.float32) if want_tone_scores else None
+    out = (N.FmChart * max(1, max_charts))()
+    n_found = C.c_int(0)
+    desc = N.BatchDesc(1, n_in, ch, int(sample_rate), 0.0, 0.0, 0)
+    decoder._check(decoder._lib.wefax_decode_fm_charts(
+        decoder._h, C.byref(desc), C.c_void_p(pcm.ctypes.data), C.byref(prm), out, int(max_charts), C.byref(n_found),
+        img.ctypes.data if want_images else None, int(image_capacity),
+        tones.ctypes.data if want_tone_scores else None, grey.ctypes.data if want_grey else None))
+    charts = []
+    for c in out[: min(n_found.value, max_charts)]:
+        picture = None
+        if want_images and c.status == N.FM_CHART_OK:
+            picture = img[c.image_offset: c.image_offset + c.rows * c.width].reshape(c.rows, c.width)
+        so = FmSlant(**{name: getattr(c.slant, name) for name, _ in N.FmSlantOut._fields_}) \
+            if (want_images and c.status == N.FM_CHART_OK and prm.slant.mode != N.FM_SLANT_OFF) else None
+        charts.append(FmChart(int(c.tone_begin), int(c.search_from), int(c.image_end), bool(c.stop_found), int(c.ioc),
+                              float(c.lpm), float(c.lpm_score), int(c.status), int(c.width), int(c.line_start),
+                              picture, so))
+    return FmCharts(charts, int(n_found.value), grey, tones)
+
+
 def _pcm16(data: np.ndarray) -> np.ndarray:
     """int16 samples of what wavio.read returns (uint8, int16, int32 or float PCM)."""
     if data.dtype == np.int16:
@@ -150,9 +253,13 @@ def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="python -m wefax_b200.fm",
                                  description="FM-discriminator WEFAX decode of a WAV recording into a greyscale PNG.")
     ap.add_argument("wav", help="input recording (WAV)")
-    ap.add_argument("png", help="output picture (8-bit greyscale PNG)")
-    ap.add_argument("--lpm", type=float, default=120.0, help="lines per minute (default 120)")
-    ap.add_argument("--ioc", type=int, default=576, help="index of cooperation: 576 or 288 (default 576)")
+    ap.add_argument("png", help="output picture (8-bit greyscale PNG); with --all, OUT-01.png, OUT-02.png, ...")
+    ap.add_argument("--all", action="store_true",
+                    help="find every chart of the recording by its start / stop tones and write one PNG per chart")
+    ap.add_argument("--lpm", type=float, default=None,
+                    help="lines per minute (default 120; with --all: measured per chart from its phasing lines)")
+    ap.add_argument("--ioc", type=int, default=None,
+                    help="index of cooperation: 576 or 288 (default 576; with --all: from each chart's start tone)")
     ap.add_argument("--slant", default=None, metavar="auto|PPM",
                     help="correct the sample-clock error: 'auto' measures it, a number gives it in ppm")
     ap.add_argument("--max-slant-ppm", type=float, default=300.0, help="largest error 'auto' searches (default 300)")
@@ -173,9 +280,11 @@ def main(argv=None) -> int:
     from .decoder import Decoder
 
     sample_rate, data = wavio.read(a.wav)
+    if a.all:
+        return _main_all(a, slant, _pcm16(data), sample_rate, ap)
     with Decoder(a.device) as dec:
-        res = decode_fm(dec, _pcm16(data), sample_rate, lpm=a.lpm, ioc=a.ioc, slant=slant,
-                        max_slant_ppm=a.max_slant_ppm)
+        res = decode_fm(dec, _pcm16(data), sample_rate, lpm=120.0 if a.lpm is None else a.lpm,
+                        ioc=576 if a.ioc is None else a.ioc, slant=slant, max_slant_ppm=a.max_slant_ppm)
     pngio.write_png_gray8(a.png, res.image)
     print(f"{a.png}: {res.image.shape[0]} x {res.image.shape[1]} pixels, first line at sample {res.line_start}")
     if res.slant is not None:
@@ -186,6 +295,38 @@ def main(argv=None) -> int:
                   f"reuse with --slant {s.ppm:.3f}")
         else:
             print("slant: too few line pulses to measure it; the picture is not corrected")
+    return 0
+
+
+def _main_all(a, slant, pcm, sample_rate, ap) -> int:
+    import os
+
+    from . import pngio
+    from .decoder import Decoder
+
+    try:
+        chart_params(a.lpm, a.ioc, slant=slant, max_slant_ppm=a.max_slant_ppm)
+    except ValueError as e:
+        ap.error(str(e))
+    stem, ext = os.path.splitext(a.png)
+    with Decoder(a.device) as dec:
+        res = decode_fm_charts(dec, pcm, sample_rate, lpm=a.lpm, ioc=a.ioc, slant=slant, max_slant_ppm=a.max_slant_ppm)
+    if res.n_found > len(res.charts):
+        print(f"{res.n_found} charts found, the first {len(res.charts)} decoded")
+    for k, c in enumerate(res.charts, 1):
+        t0, t1 = c.tone_begin / N.TARGET_RATE, c.image_end / N.TARGET_RATE
+        where = f"chart {k}: {t0:8.1f} s - {t1:8.1f} s{'' if c.stop_found else ' (no stop tone)'}, IOC {c.ioc}"
+        if c.status != N.FM_CHART_OK:
+            print(f"{where}, no LPM found (best {c.lpm:g}, score {c.lpm_score:.2f}): not decoded")
+            continue
+        path = f"{stem}-{k:02d}{ext or '.png'}"
+        pngio.write_png_gray8(path, c.image)
+        line = f"{where}, LPM {c.lpm:g} (score {c.lpm_score:.2f}), {path}: {c.image.shape[0]} x {c.image.shape[1]}"
+        if c.slant is not None:
+            line += f", slant {c.slant.ppm:+.3f} ppm" if c.slant.found else ", slant not measured"
+        print(line)
+    if not res.n_found:
+        print("no chart found (no start tone of 2 s or more)")
     return 0
 
 

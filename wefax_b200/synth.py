@@ -30,6 +30,23 @@ BATCH_LPMS = (60, 90, 120, 240)
 BATCH_IOCS = (576, 288)
 
 
+def transmission_times(duration_s: float, lpm: float = 120, n_phasing: int = 30):
+    """(phasing start, picture start, stop tone start, black start) in seconds of transmission time."""
+    line_t = 60.0 / lpm
+    start_len, stop_len, black_len = 5.0, 5.0, 10.0
+    tail = stop_len + black_len
+    # keep the structure sensible for very short test clips
+    if duration_s < start_len + tail + (n_phasing + 4) * line_t:
+        scale = duration_s / (start_len + tail + (n_phasing + 4) * line_t)
+        start_len *= scale
+        stop_len *= scale
+        black_len *= scale
+        tail = stop_len + black_len
+        n_phasing = max(2, int(n_phasing * scale))
+    t_phase0 = start_len
+    return t_phase0, t_phase0 + n_phasing * line_t, duration_s - tail, duration_s - black_len
+
+
 def synth_recording(duration_s: float,
                     sample_rate: int = TARGET_RATE,
                     lpm: int = 120,
@@ -53,20 +70,7 @@ def synth_recording(duration_s: float,
         t = t * (1.0 + drift_ppm * 1e-6)
 
     line_t = 60.0 / lpm
-    start_len, stop_len, black_len = 5.0, 5.0, 10.0
-    tail = stop_len + black_len
-    # keep the structure sensible for very short test clips
-    if duration_s < start_len + tail + (n_phasing + 4) * line_t:
-        scale = duration_s / (start_len + tail + (n_phasing + 4) * line_t)
-        start_len *= scale
-        stop_len *= scale
-        black_len *= scale
-        tail = stop_len + black_len
-        n_phasing = max(2, int(n_phasing * scale))
-    t_phase0 = start_len
-    t_img0 = t_phase0 + n_phasing * line_t
-    t_stop0 = duration_s - tail
-    t_black0 = duration_s - black_len
+    t_phase0, t_img0, t_stop0, t_black0 = transmission_times(duration_s, lpm, n_phasing)
 
     grey = np.zeros(n, dtype=np.float64)
 
@@ -102,6 +106,42 @@ def synth_recording(duration_s: float,
     if return_grey:      # the per-sample grey level that was transmitted (ground truth of the FM extension)
         return x.astype(np.int16), grey
     return x.astype(np.int16)
+
+
+def synth_broadcast(charts, sample_rate: int = TARGET_RATE, noise_sigma: float = 0.0, drift_ppm: float = 0.0,
+                    gap_s: float = 0.0, seed: int = 0, return_grey: bool = False):
+    """A broadcast: the transmissions ``charts`` (dicts of synth_recording arguments, at least ``duration_s``; ``lpm``
+    and ``ioc`` default to 120 and 576) back to back, ``gap_s`` seconds of noise only (silence when noise_sigma is 0)
+    before each one after the first.  Every piece shares noise_sigma and drift_ppm and has its own seed (seed + k).
+
+    Returns (pcm, truth): int16 mono PCM and, per piece, dict(tone_begin, search_from, stop_begin, lpm, ioc) in samples
+    at sample_rate (the start tone, the phasing lines and the stop tone as the recording's drifted clock places them);
+    with return_grey, (pcm, truth, grey): the transmitted grey per sample (0 in the gaps)."""
+    rng = np.random.default_rng(seed)
+    pieces, greys, truth, at = [], [], [], 0
+    for k, spec in enumerate(charts):
+        spec = dict(spec)
+        spec.setdefault("lpm", 120)
+        spec.setdefault("ioc", 576)
+        spec.setdefault("seed", seed + 1 + k)
+        if k and gap_s > 0:
+            g = int(round(gap_s * sample_rate))
+            gap = np.round(rng.normal(0.0, noise_sigma, size=g) * 32767.0) if noise_sigma else np.zeros(g)
+            pieces.append(np.clip(gap, -32768, 32767).astype(np.int16))
+            greys.append(np.zeros(g))
+            at += g
+        x, grey = synth_recording(sample_rate=sample_rate, noise_sigma=noise_sigma, drift_ppm=drift_ppm,
+                                  return_grey=True, **spec)
+        t_phase0, _, t_stop0, _ = transmission_times(spec["duration_s"], spec["lpm"], spec.get("n_phasing", 30))
+        clock = sample_rate / (1.0 + drift_ppm * 1e-6)      # samples per second of transmission time
+        truth.append(dict(tone_begin=at, search_from=at + int(round(t_phase0 * clock)),
+                          stop_begin=at + int(round(t_stop0 * clock)), lpm=spec["lpm"], ioc=spec["ioc"]))
+        pieces.append(x)
+        greys.append(grey)
+        at += x.shape[0]
+    if return_grey:
+        return np.concatenate(pieces), truth, np.concatenate(greys)
+    return np.concatenate(pieces), truth
 
 
 def batch_spec(k: int, noisy: bool = False) -> dict:

@@ -418,6 +418,20 @@ int wefax_decode_fm_charts(wefax_ctx *ctx, const wefax_batch_desc *desc, const i
                            const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts,
                            int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores, float *grey);
 
+/* Every chart of desc->n_recordings >= 1 recordings of equal length (int16, host or WEFAX_F_PCM_ON_DEVICE), each
+ * recording's charts and pictures exactly what wefax_decode_fm_charts returns for it alone.  The recordings run in
+ * waves sized by wefax_ctx_set_workspace_limit; each wave takes a fixed number of launches and synchronisations
+ * however many recordings and charts it holds (DESIGN.md 4.7c).  charts: HOST array of n_recordings x max_charts
+ * entries, recording r's at r * max_charts; n_charts: HOST array of one count per recording (the charts found, also
+ * when above max_charts; 0 when none is found, which is not an error).  images: the pictures of every recording back
+ * to back, in recording then chart order, image_offset counted from images; image_capacity covers the whole batch,
+ * else WEFAX_ERR_INVALID naming the bytes needed.  tone_scores: (n_out / WEFAX_FM_TONE_WINDOW) x 4 floats per
+ * recording; grey: n_out floats per recording. */
+int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                                 const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts,
+                                 int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
+                                 float *grey);
+
 #ifdef __cplusplus
 }
 #endif

@@ -30,6 +30,7 @@ EXPORTED_SYMBOLS = (
     "wefax_segment_envelope", "wefax_segment_histogram", "wefax_segment_quantise", "wefax_segment_sync",
     "wefax_segment_raster", "wefax_sync_pulse_scan", "wefax_segment_select_init", "wefax_segment_histogram_dev",
     "wefax_segment_select_dev", "wefax_segment_quantise_dev", "wefax_decode_fm_slant", "wefax_decode_fm_charts",
+    "wefax_decode_fm_charts_batch",
 )
 ABI_VERSION = 5
 
@@ -191,6 +192,9 @@ def load():
     lib.wefax_decode_fm_charts.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmChartParams), vp, i,
                                            C.POINTER(i), vp, ll, vp, vp]
     lib.wefax_decode_fm_charts.restype = i
+    lib.wefax_decode_fm_charts_batch.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmChartParams), vp, i, vp,
+                                                 vp, ll, vp, vp]
+    lib.wefax_decode_fm_charts_batch.restype = i
     lib.wefax_segment_envelope.argtypes = [vp, C.POINTER(BatchDesc), vp, ll, ll, ll, ll]
     lib.wefax_segment_envelope.restype = i
     lib.wefax_segment_histogram.argtypes = [vp, i, C.POINTER(C.c_uint32 * 4), vp]

@@ -456,56 +456,6 @@ bool robust_line_fit(std::vector<double> l, std::vector<double> y, int min_lines
     return true;
 }
 
-// AUTO slant: coarse sheared fold of the first Lc lines, per-line pulse tracking, robust line fit (twice: Lc lines,
-// then all L lines from the first fit).  Fills res (status WEFAX_FM_SLANT_NOT_FOUND when too few pulses are found or
-// the fit leaves +-max_ppm); synchronises the context's stream.
-void slant_search(wefax_ctx *ctx, const float *g, long long n, long long from, const SlantGeometry &sg,
-                  const wefax_fm_slant &prm, wefax_fm_slant_out &res) {
-    res.status = WEFAX_FM_SLANT_NOT_FOUND;
-    res.lines_total = (int)std::min<long long>(sg.L, INT32_MAX);
-    if (sg.L < std::max(2, prm.min_lines) || sg.L > INT32_MAX) return;
-    cudaStream_t st = ctx->stream;
-    const int L = (int)sg.L;
-    const size_t q_bytes = ((size_t)sg.Lc * sg.Bn * sizeof(float) + 255) / 256 * 256;
-    char *scratch = (char *)ctx->work_misc.reserve(q_bytes + 256 + (size_t)L * (sizeof(long long) + sizeof(float)));
-    float *Q = (float *)scratch;
-    unsigned long long *d_best = (unsigned long long *)(scratch + q_bytes);
-    long long *d_pos = (long long *)(scratch + q_bytes + 256);
-    float *d_ctr = (float *)(d_pos + L);
-    launch_fm_slant_profile(ctx, g, n, from, sg.Ls, sg.D, sg.Bn, sg.Lc, Q);
-    launch_fm_slant_fold(ctx, Q, sg.Lc, sg.Bn, sg.wbb, 2 * sg.J + 1, d_best);
-    long long *h = (long long *)pinned(ctx, (size_t)L * sizeof(long long) + 64);
-    CUDA_CHECK(cudaMemcpyAsync(h, d_best, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    const int rank = 0x7fffffff - (int)(unsigned)((unsigned long long)h[0] & 0xffffffffull);
-    const int c = rank / sg.Bn, b = rank % sg.Bn;
-    const int k = c == 0 ? 0 : ((c + 1) / 2) * 2 * ((c & 1) ? -1 : 1);
-    double a = (double)(from + (long long)b * sg.D), s = sg.Ls + (double)k * sg.D / sg.Lc;
-    LineFit fit;
-    for (int lines : {sg.Lc, L}) {
-        launch_fm_slant_track(ctx, g, n, a, s, lines, sg.wb, sg.R, prm.min_contrast, d_pos, d_ctr);
-        CUDA_CHECK(cudaMemcpyAsync(h, d_pos, (size_t)lines * sizeof(long long), cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-        std::vector<double> li, yi;
-        for (int i = 0; i < lines; ++i)
-            if (h[i] >= 0) {
-                li.push_back((double)i);
-                yi.push_back((double)h[i]);
-            }
-        if (!robust_line_fit(std::move(li), std::move(yi), prm.min_lines, fit)) return;
-        a = fit.a;
-        s = fit.s;
-    }
-    const double ppm = (sg.Ls / s - 1.0) * 1e6;
-    if (!(fabs(ppm) <= prm.max_ppm)) return;
-    res.status = WEFAX_FM_SLANT_OK;
-    res.line_length = s;
-    res.ppm = ppm;
-    res.first_line = a - floor((a - (double)from) / s) * s;
-    res.lines_used = fit.used;
-    res.residual_rms = fit.rms;
-}
-
 // ---- FM decode: the stages every FM entry point shares ----
 
 // the caller's slant parameters with their defaults filled in
@@ -543,78 +493,227 @@ FmGeometry fm_geometry(double lpm, int ioc, const wefax_fm_slant &sp, long long 
     return f;
 }
 
-// Band-pass, analytic signal and discriminator of one recording: the grey stream, n samples at 11025 Hz, in g_out
-// when it is not null (a device buffer), else in work_z
-float *fm_front_end(wefax_ctx *ctx, const wefax_batch_desc &desc, const int16_t *pcm, const wefax_fm_params &prm,
-                    long long n, float *g_out) {
+// The FM front end's layout for recordings of n samples at 11025 Hz: the real-input transform runs on the next even
+// length npad = 2 * half_len whose half is smooth (zero padded).  zs, the row stride of the half-length spectrum, is
+// even so that a batch takes the same fused Hilbert middle as one recording.
+struct FmFront {
+    long long n, half_len, npad, zs;
+    FftPlan *half;
+};
+
+FmFront fm_front_plan(wefax_ctx *ctx, long long n) {
+    FmFront f;
+    f.n = n;
+    f.half_len = next_smooth_length((n + 1) / 2);
+    f.half = f.half_len > 0 ? get_plan(ctx, f.half_len) : nullptr;
+    if (!f.half) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
+    f.npad = 2 * f.half_len;
+    f.zs = f.half_len + (f.half_len & 1);
+    return f;
+}
+
+// Band-pass, analytic signal and discriminator of `batch` recordings (d_pcm: their uploaded PCM, desc as the caller's):
+// the grey streams, rows of n samples at 11025 Hz, in g_out when it is not null (a device buffer), else in work_z
+float *fm_front_end(wefax_ctx *ctx, const wefax_batch_desc &desc, const void *d_pcm, const wefax_fm_params &prm,
+                    const FmFront &f, int batch, float *g_out) {
     cudaStream_t st = ctx->stream;
     const FirParams fp = make_bandpass_fir(prm.band_lo_hz, prm.band_hi_hz, (double)WEFAX_TARGET_RATE, prm.fir_taps);
-    // the transform runs on the next even length whose half is smooth (zero padded)
-    long long half_len = next_smooth_length((n + 1) / 2);
-    FftPlan *half = half_len > 0 ? get_plan(ctx, half_len) : nullptr;
-    if (!half) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "no transform length for n=%lld", n);
-    const long long npad = 2 * half_len;
-
-    const void *d_pcm = upload_pcm(ctx, pcm, (size_t)desc.n_frames * desc.channels, desc.flags, false);
-    float *x = (float *)ctx->work_a.reserve((size_t)npad * sizeof(float));
-    float *y = (float *)ctx->work_e.reserve((size_t)npad * sizeof(float));
-    if (npad > n) CUDA_CHECK(cudaMemsetAsync(x + n, 0, (size_t)(npad - n) * sizeof(float), st));
-    const NotchInput in = notch_input(ctx, desc, d_pcm, n, 1);
-    launch_filtfilt(ctx, in.mode, in.x, in.stride, x, (size_t)npad, nullptr, 0, n, fp, 1);
-    float2 *z = (float2 *)ctx->work_z.reserve((size_t)half_len * sizeof(float2));
-    hilbert_envelope_real(ctx, half, x, (size_t)npad, z, (size_t)half_len, y, (size_t)npad, 1, /*want_y=*/true);
-    float *g = g_out ? g_out : (float *)ctx->work_z.reserve((size_t)n * sizeof(float));
-    launch_fm_grey(ctx, x, y, g, n, prm.black_hz, prm.white_hz);
+    const long long n = f.n, npad = f.npad;
+    float *x = (float *)ctx->work_a.reserve((size_t)batch * npad * sizeof(float));
+    float *y = (float *)ctx->work_e.reserve((size_t)batch * npad * sizeof(float));
+    if (npad > n)
+        CUDA_CHECK(cudaMemset2DAsync(x + n, (size_t)npad * sizeof(float), 0, (size_t)(npad - n) * sizeof(float), batch, st));
+    const NotchInput in = notch_input(ctx, desc, d_pcm, n, batch);
+    launch_filtfilt(ctx, in.mode, in.x, in.stride, x, (size_t)npad, nullptr, 0, n, fp, batch);
+    float2 *z = (float2 *)ctx->work_z.reserve((size_t)batch * f.zs * sizeof(float2));
+    hilbert_envelope_real(ctx, f.half, x, (size_t)npad, z, (size_t)f.zs, y, (size_t)npad, batch, /*want_y=*/true);
+    float *g = g_out ? g_out : (float *)ctx->work_z.reserve((size_t)batch * n * sizeof(float));
+    launch_fm_grey(ctx, x, y, (size_t)npad, g, n, batch, prm.black_hz, prm.white_hz);
     return g;
 }
 
-// One picture from the grey stream g: line start from the phasing fold (or the slant search), then rows_max rows of
-// fg.W pixels into the device buffer d_img (null: no picture).  Synchronises the context's stream; returns the line
-// start, the rows written (floor((image_end - line_start) / line length), at most rows_max) and the slant report.
-struct FmPicture {
-    long long line_start;
-    int rows;
+// One chart of the picture stage: its recording's grey stream and its span in; its line start, rows, slant report and
+// picture offset out
+struct FmTail {
+    const float *g;
+    long long n, from, image_end;
+    FmGeometry fg;
+    bool picture;              // write its picture (rows_max rows at most)
+    long long line_start = 0;
+    int rows = 0;
+    long long offset = 0;      // of its picture from d_img (fm_tail)
     wefax_fm_slant_out so;
 };
 
-FmPicture fm_picture(wefax_ctx *ctx, const float *g, long long n, long long from, long long image_end,
-                     const FmGeometry &fg, int fold_lines, const wefax_fm_slant &sp, uint8_t *d_img) {
+// The picture stage of every chart in cs, each launch once over one chart table (DESIGN.md §4.7c):
+//   AUTO: coarse sheared fold of each chart's first Lc lines, per-line pulse tracking, robust line fit (twice: Lc
+//         lines, then all L lines from the first fit), three synchronisations for all charts together; a chart whose
+//         search finds too few pulses or leaves +-max_ppm keeps its phasing line start (status NOT_FOUND);
+//   the phasing fold of every chart without a fitted line; one synchronisation for all line starts;
+//   packed picture offsets from d_img on (rows * W bytes each); one image launch.
+// Returns the bytes of pictures written to d_img (device); the image launch may still be running.
+long long fm_tail(wefax_ctx *ctx, std::vector<FmTail> &cs, int fold_lines, const wefax_fm_slant &sp, uint8_t *d_img) {
     cudaStream_t st = ctx->stream;
-    const int Lc = (int)ceil(fg.Ls_fixed);
-    char *small = (char *)ctx->out_small.reserve((size_t)Lc * sizeof(float) + 64);
-    long long *d_ls = (long long *)small;
-    float *P = (float *)(small + 64);
+    const int nc = (int)cs.size();
+    if (nc == 0) return 0;
+    std::vector<FmChartJob> tab(nc);
+    int max_lc = 0;
+    for (int i = 0; i < nc; ++i) {
+        FmTail &c = cs[i];
+        FmChartJob &j = tab[i];
+        memset(&j, 0, sizeof(j));
+        j.g = c.g;
+        j.n = c.n;
+        j.from = c.from;
+        j.image_end = c.image_end;
+        j.Ls = c.fg.Ls_fixed;
+        j.phase = 1;
+        j.W = c.fg.W;
+        max_lc = std::max(max_lc, (int)ceil(j.Ls));
+        memset(&c.so, 0, sizeof(c.so));
+        c.so.status = WEFAX_FM_SLANT_OK;
+        if (sp.mode == WEFAX_FM_SLANT_FIXED) c.so.ppm = sp.ppm;
+    }
+    const size_t tab_bytes = ((size_t)nc * sizeof(FmChartJob) + 255) / 256 * 256;
+    const size_t key_bytes = ((size_t)nc * sizeof(long long) + 255) / 256 * 256;
+    char *dev = (char *)ctx->out_small.reserve(tab_bytes + 2 * key_bytes + (size_t)nc * max_lc * sizeof(float));
+    FmChartJob *d_tab = (FmChartJob *)dev;
+    long long *d_ls = (long long *)(dev + tab_bytes);
+    unsigned long long *d_best = (unsigned long long *)(dev + tab_bytes + key_bytes);
+    float *P = (float *)(dev + tab_bytes + 2 * key_bytes);
+    // (pageable source: the copy is staged before the call returns, so the host table may change right after it)
+    auto upload = [&] {
+        CUDA_CHECK(cudaMemcpyAsync(d_tab, tab.data(), (size_t)nc * sizeof(FmChartJob), cudaMemcpyHostToDevice, st));
+    };
+    std::vector<long long> ls0(nc, 0);
 
-    FmPicture pic;
-    wefax_fm_slant_out &so = pic.so;
-    memset(&so, 0, sizeof(so));
-    so.status = WEFAX_FM_SLANT_OK;
-    double line_length = fg.Ls_fixed;
-    bool fitted = false;
     if (sp.mode == WEFAX_FM_SLANT_AUTO) {
-        slant_search(ctx, g, n, from, slant_geometry(fg.Ls, from, image_end, sp.max_ppm), sp, so);
-        if (so.status == WEFAX_FM_SLANT_OK) {
-            const long long ls = llround(so.first_line);
-            CUDA_CHECK(cudaMemcpyAsync(d_ls, &ls, sizeof(long long), cudaMemcpyHostToDevice, st));
-            line_length = so.line_length;
-            fitted = true;
+        std::vector<SlantGeometry> sg(nc);
+        std::vector<char> alive(nc, 0);
+        long long q_total = 0, pos_total = 0;
+        for (int i = 0; i < nc; ++i) {
+            FmTail &c = cs[i];
+            sg[i] = slant_geometry(c.fg.Ls, c.from, c.image_end, sp.max_ppm);
+            c.so.status = WEFAX_FM_SLANT_NOT_FOUND;
+            c.so.lines_total = (int)std::min<long long>(sg[i].L, INT32_MAX);
+            if (sg[i].L < std::max(2, sp.min_lines) || sg[i].L > INT32_MAX) continue;
+            alive[i] = 1;
+            FmChartJob &j = tab[i];
+            j.sLs = sg[i].Ls;
+            j.D = sg[i].D;
+            j.Bn = sg[i].Bn;
+            j.wbb = sg[i].wbb;
+            j.R = sg[i].R;
+            j.swb = sg[i].wb;
+            j.q_lines = sg[i].Lc;
+            j.n_cand = 2 * sg[i].J + 1;
+            j.q_off = q_total;
+            j.pos_off = pos_total;
+            q_total += (long long)sg[i].Lc * sg[i].Bn;
+            pos_total += sg[i].L;
         }
-    } else if (sp.mode == WEFAX_FM_SLANT_FIXED) {
-        so.ppm = sp.ppm;
+        if (pos_total > 0) {
+            const size_t q_bytes = ((size_t)q_total * sizeof(float) + 255) / 256 * 256;
+            char *scratch = (char *)ctx->work_misc.reserve(q_bytes + (size_t)pos_total * (sizeof(long long) + sizeof(float)));
+            float *Q = (float *)scratch;
+            long long *d_pos = (long long *)(scratch + q_bytes);
+            float *d_ctr = (float *)(d_pos + pos_total);
+            upload();
+            launch_fm_slant_profile(ctx, d_tab, tab.data(), nc, Q);
+            launch_fm_slant_fold(ctx, d_tab, tab.data(), nc, Q, d_best);
+            long long *h = (long long *)pinned(ctx, (size_t)std::max<long long>(nc, pos_total) * sizeof(long long) + 64);
+            CUDA_CHECK(cudaMemcpyAsync(h, d_best, (size_t)nc * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            CUDA_CHECK(cudaStreamSynchronize(st));
+            std::vector<double> a(nc, 0.0), s(nc, 0.0);
+            std::vector<LineFit> fit(nc);
+            for (int i = 0; i < nc; ++i) {
+                if (!alive[i]) continue;
+                const int rank = 0x7fffffff - (int)(unsigned)((unsigned long long)h[i] & 0xffffffffull);
+                const int c = rank / sg[i].Bn, b = rank % sg[i].Bn;
+                const int k = c == 0 ? 0 : ((c + 1) / 2) * 2 * ((c & 1) ? -1 : 1);
+                a[i] = (double)(cs[i].from + (long long)b * sg[i].D);
+                s[i] = sg[i].Ls + (double)k * sg[i].D / sg[i].Lc;
+            }
+            for (int pass = 0; pass < 2; ++pass) {
+                for (int i = 0; i < nc; ++i) {
+                    tab[i].track_lines = alive[i] ? (pass == 0 ? sg[i].Lc : (int)sg[i].L) : 0;
+                    tab[i].a = a[i];
+                    tab[i].s = s[i];
+                }
+                upload();
+                launch_fm_slant_track(ctx, d_tab, tab.data(), nc, sp.min_contrast, d_pos, d_ctr);
+                CUDA_CHECK(cudaMemcpyAsync(h, d_pos, (size_t)pos_total * sizeof(long long), cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaStreamSynchronize(st));
+                for (int i = 0; i < nc; ++i) {
+                    if (!alive[i]) continue;
+                    std::vector<double> li, yi;
+                    const long long *hp = h + tab[i].pos_off;
+                    for (int l = 0; l < tab[i].track_lines; ++l)
+                        if (hp[l] >= 0) {
+                            li.push_back((double)l);
+                            yi.push_back((double)hp[l]);
+                        }
+                    if (!robust_line_fit(std::move(li), std::move(yi), sp.min_lines, fit[i])) {
+                        alive[i] = 0;
+                        continue;
+                    }
+                    a[i] = fit[i].a;
+                    s[i] = fit[i].s;
+                }
+            }
+            for (int i = 0; i < nc; ++i) {
+                tab[i].q_lines = tab[i].track_lines = 0;
+                if (!alive[i]) continue;
+                const double ppm = (sg[i].Ls / s[i] - 1.0) * 1e6;
+                if (!(fabs(ppm) <= sp.max_ppm)) continue;
+                wefax_fm_slant_out &so = cs[i].so;
+                so.status = WEFAX_FM_SLANT_OK;
+                so.line_length = s[i];
+                so.ppm = ppm;
+                so.first_line = a[i] - floor((a[i] - (double)cs[i].from) / s[i]) * s[i];
+                so.lines_used = fit[i].used;
+                so.residual_rms = fit[i].rms;
+                ls0[i] = llround(so.first_line);
+                tab[i].Ls = so.line_length;
+                tab[i].phase = 0;
+            }
+        }
     }
-    if (!fitted) launch_fm_phasing(ctx, g, n, from, line_length, fold_lines, P, d_ls);
-    if (d_img && fg.rows_max > 0) launch_fm_image(ctx, g, n, d_ls, line_length, fg.W, fg.rows_max, image_end, d_img);
-    long long *h_ls = (long long *)pinned(ctx, 64);
-    CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, sizeof(long long), cudaMemcpyDeviceToHost, st));
+    for (int i = 0; i < nc; ++i) {
+        tab[i].Lc = (int)ceil(tab[i].Ls);
+        tab[i].wb = std::max(1, (int)llround(0.05 * tab[i].Ls));
+    }
+
+    // line starts: the fitted ones as given, the others from the phasing fold
+    upload();
+    CUDA_CHECK(cudaMemcpyAsync(d_ls, ls0.data(), (size_t)nc * sizeof(long long), cudaMemcpyHostToDevice, st));
+    launch_fm_phasing(ctx, d_tab, tab.data(), nc, fold_lines, P, d_ls);
+    long long *h_ls = (long long *)pinned(ctx, (size_t)nc * sizeof(long long) + 64);
+    CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, (size_t)nc * sizeof(long long), cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaStreamSynchronize(st));
-    pic.line_start = *h_ls;
-    pic.rows = (int)std::min<long long>(
-        fg.rows_max, std::max<long long>(0, (long long)floor((double)(image_end - pic.line_start) / line_length)));
-    if (!fitted) {
-        so.line_length = line_length;
-        so.first_line = (double)pic.line_start;
+
+    // rows and packed offsets, then every picture in one launch
+    long long off = 0;
+    for (int i = 0; i < nc; ++i) {
+        FmTail &c = cs[i];
+        const double line_length = tab[i].Ls;
+        c.line_start = h_ls[i];
+        c.rows = (int)std::min<long long>(
+            c.fg.rows_max, std::max<long long>(0, (long long)floor((double)(c.image_end - c.line_start) / line_length)));
+        if (tab[i].phase) {
+            c.so.line_length = line_length;
+            c.so.first_line = (double)c.line_start;
+        }
+        c.offset = off;
+        tab[i].out = off;
+        tab[i].rows_max = (d_img && c.picture) ? c.fg.rows_max : 0;
+        if (tab[i].rows_max > 0) off += (long long)c.rows * c.fg.W;
     }
-    return pic;
+    if (off > 0) {
+        upload();
+        launch_fm_image(ctx, d_tab, tab.data(), nc, d_ls, d_img);
+    }
+    return off;
 }
 
 // ---- charts of a recording (DESIGN.md §4.7b; float64 restatement: tests/fm_charts_oracle.py) ----
@@ -1578,29 +1677,50 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
                         (long long)fg.rows_max * fg.W);
 
         // grey stream (in the transform scratch, or straight into the caller's device buffer)
-        const float *g = fm_front_end(ctx, *desc, pcm, *prm, n, (out_dev && out->grey) ? out->grey : nullptr);
+        const FmFront ff = fm_front_plan(ctx, n);
+        const void *d_pcm = upload_pcm(ctx, pcm, (size_t)n_in * desc->channels, desc->flags, false);
+        const float *g = fm_front_end(ctx, *desc, d_pcm, *prm, ff, 1, (out_dev && out->grey) ? out->grey : nullptr);
         if (!out_dev && out->grey)
             CUDA_CHECK(cudaMemcpyAsync(out->grey, g, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
+        // the picture stage with a table of one chart: the caller's span
+        std::vector<FmTail> cs(1);
+        cs[0].g = g;
+        cs[0].n = n;
+        cs[0].from = from;
+        cs[0].image_end = image_end;
+        cs[0].fg = fg;
+        cs[0].picture = out->image != nullptr;
         uint8_t *d_img = nullptr;
         if (out->image && fg.rows_max > 0)
             d_img = out_dev ? out->image : (uint8_t *)ctx->out_raster.reserve((size_t)fg.rows_max * fg.W);
-        const FmPicture pic = fm_picture(ctx, g, n, from, image_end, fg, prm->fold_lines, sp, d_img);
-        if (!out_dev && d_img && pic.rows > 0)
-            CUDA_CHECK(cudaMemcpy(out->image, d_img, (size_t)pic.rows * fg.W, cudaMemcpyDeviceToHost));
-        if (out->rows) *out->rows = pic.rows;
+        const long long bytes = fm_tail(ctx, cs, prm->fold_lines, sp, d_img);
+        if (!out_dev && bytes > 0)
+            CUDA_CHECK(cudaMemcpyAsync(out->image, d_img, (size_t)bytes, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        if (out->rows) *out->rows = cs[0].rows;
         if (out->width) *out->width = fg.W;
-        if (out->line_start) *out->line_start = pic.line_start;
-        if (slant_out) *slant_out = pic.so;
+        if (out->line_start) *out->line_start = cs[0].line_start;
+        if (slant_out) *slant_out = cs[0].so;
     });
 }
 
 int wefax_decode_fm_charts(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
                            const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts, int *n_charts,
                            uint8_t *images, long long image_capacity, float *tone_scores, float *grey) {
+    if (ctx && desc && desc->n_recordings != 1)
+        return guarded(ctx, [] { WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument"); });
+    return wefax_decode_fm_charts_batch(ctx, desc, pcm, params, charts, max_charts, n_charts, images, image_capacity,
+                                        tone_scores, grey);
+}
+
+int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                                 const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts,
+                                 int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
+                                 float *grey) {
     if (!ctx) return WEFAX_ERR_INVALID;
     return guarded(ctx, [&] {
         if (!desc || !pcm || !params || !n_charts || max_charts < 0 || (max_charts > 0 && !charts) ||
-            desc->n_recordings != 1 || desc->n_frames < 64 || (desc->channels != 1 && desc->channels != 2) ||
+            desc->n_recordings < 1 || desc->n_frames < 64 || (desc->channels != 1 && desc->channels != 2) ||
             desc->sample_rate < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
         const wefax_fm_params &prm = params->fm;
@@ -1624,89 +1744,137 @@ int wefax_decode_fm_charts(wefax_ctx *ctx, const wefax_batch_desc *desc, const i
         }
         use_device(ctx);
         cudaStream_t st = ctx->stream;
+        const int nrec = desc->n_recordings, ch = desc->channels;
         const long long n_in = desc->n_frames;
-        const long long n = desc->sample_rate != WEFAX_TARGET_RATE ? wefax_resampled_length(n_in, desc->sample_rate) : n_in;
+        const bool resample = desc->sample_rate != WEFAX_TARGET_RATE;
+        const long long n = resample ? wefax_resampled_length(n_in, desc->sample_rate) : n_in;
         if (n < 64) WEFAX_THROW(WEFAX_ERR_INVALID, "recording too short");
-        const bool out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE;
-        const float *g = fm_front_end(ctx, *desc, pcm, prm, n, (out_dev && grey) ? grey : nullptr);
-        if (!out_dev && grey)
-            CUDA_CHECK(cudaMemcpyAsync(grey, g, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
-
-        // tone windows -> charts
+        const bool out_dev = desc->flags & WEFAX_F_OUT_ON_DEVICE, pcm_dev = desc->flags & WEFAX_F_PCM_ON_DEVICE;
         const long long nw = n / WEFAX_FM_TONE_WINDOW;
-        const size_t tone_bytes = (size_t)nw * sizeof(float4);
-        float4 *d_tone = (float4 *)ctx->work_misc.reserve(tone_bytes + 16);
-        launch_fm_tone(ctx, g, nw, d_tone);
-        if (out_dev && tone_scores && nw > 0)
-            CUDA_CHECK(cudaMemcpyAsync(tone_scores, d_tone, tone_bytes, cudaMemcpyDeviceToDevice, st));
-        float *h_tone = (float *)pinned(ctx, tone_bytes + 16);
-        if (nw > 0) CUDA_CHECK(cudaMemcpyAsync(h_tone, d_tone, tone_bytes, cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaStreamSynchronize(st));
-        if (!out_dev && tone_scores && nw > 0) memcpy(tone_scores, h_tone, tone_bytes);
-        std::vector<int> cls((size_t)nw);
-        for (long long k = 0; k < nw; ++k) cls[k] = tone_class(h_tone + 4 * k);
-        std::vector<wefax_fm_chart> found = find_charts(cls, n);
-        *n_charts = (int)found.size();
-        const int nc = (int)std::min<long long>((long long)found.size(), max_charts);
+        const size_t tone_row = (size_t)nw * 4;   // floats of one recording's tone scores
+        const FmFront ff = fm_front_plan(ctx, n);
 
-        // LPM of each chart from its phasing lines (one launch for all charts and candidates)
-        for (int i = 0; i < nc; ++i) {
-            found[i].lpm = prm.lpm;
-            if (prm.ioc > 0) found[i].ioc = prm.ioc;
-        }
-        if (!(prm.lpm > 0.0) && nc > 0) {
-            std::vector<long long> from(nc);
-            for (int i = 0; i < nc; ++i) from[i] = std::min<long long>(found[i].search_from, n - 1);
-            char *buf = (char *)ctx->work_misc.reserve((size_t)nc * sizeof(long long) + (size_t)nc * n_cand * sizeof(double));
-            long long *d_from = (long long *)buf;
-            double *d_score = (double *)(buf + (size_t)nc * sizeof(long long));
-            CUDA_CHECK(cudaMemcpyAsync(d_from, from.data(), (size_t)nc * sizeof(long long), cudaMemcpyHostToDevice, st));
-            launch_fm_lpm(ctx, g, n, d_from, nc, cand, prm.fold_lines, d_score);
-            double *h_score = (double *)pinned(ctx, (size_t)nc * n_cand * sizeof(double));
-            CUDA_CHECK(cudaMemcpyAsync(h_score, d_score, (size_t)nc * n_cand * sizeof(double), cudaMemcpyDeviceToHost, st));
+        // waves: the front end's buffers, the grey streams and the pictures of every recording of a wave stay resident
+        const long long per_rec = (pcm_dev ? 0 : n_in * ch * 2) + (resample ? n_in * 4 + (n_in + n) * 4 : 0) +
+                                  ff.npad * 8 + ff.zs * 8 + nw * 16 + n + 4096;
+        int wave = (int)std::max<long long>(1, std::min<long long>(nrec, ctx->workspace_limit / per_rec));
+        wave = std::min(wave, 32768);
+
+        long long need = 0, img_off = 0;
+        bool too_small = false;
+        for (int w0 = 0; w0 < nrec; w0 += wave) {
+            const int gw = std::min(wave, nrec - w0);
+            // ---- front end and tone windows of the whole wave -----------------------------------------------------
+            const void *d_pcm = upload_pcm(ctx, pcm + (size_t)w0 * n_in * ch, (size_t)gw * n_in * ch, desc->flags, false);
+            float *grey_w = grey ? grey + (size_t)w0 * n : nullptr;
+            const float *g = fm_front_end(ctx, *desc, d_pcm, prm, ff, gw, out_dev ? grey_w : nullptr);
+            if (!out_dev && grey_w)
+                CUDA_CHECK(cudaMemcpyAsync(grey_w, g, (size_t)gw * n * sizeof(float), cudaMemcpyDeviceToHost, st));
+            const size_t tone_bytes = (size_t)gw * tone_row * sizeof(float);
+            float4 *d_tone = (float4 *)ctx->work_misc.reserve(tone_bytes + 16);
+            launch_fm_tone(ctx, g, n, nw, gw, d_tone);
+            if (out_dev && tone_scores && nw > 0)
+                CUDA_CHECK(cudaMemcpyAsync(tone_scores + (size_t)w0 * tone_row, d_tone, tone_bytes,
+                                           cudaMemcpyDeviceToDevice, st));
+            float *h_tone = (float *)pinned(ctx, tone_bytes + 16);
+            if (nw > 0) CUDA_CHECK(cudaMemcpyAsync(h_tone, d_tone, tone_bytes, cudaMemcpyDeviceToHost, st));
             CUDA_CHECK(cudaStreamSynchronize(st));
-            for (int i = 0; i < nc; ++i) {
-                int best = 0;
-                for (int c = 1; c < n_cand; ++c)
-                    if (h_score[(size_t)i * n_cand + c] > h_score[(size_t)i * n_cand + best]) best = c;
-                found[i].lpm = cand_lpm[best];
-                found[i].lpm_score = h_score[(size_t)i * n_cand + best];
-                if (found[i].lpm_score < WEFAX_FM_LPM_MIN_SCORE) found[i].status = WEFAX_FM_CHART_NO_LPM;
-            }
-        }
+            if (!out_dev && tone_scores && nw > 0) memcpy(tone_scores + (size_t)w0 * tone_row, h_tone, tone_bytes);
 
-        // each chart's picture: the tail of the single-picture decode on the shared grey stream
-        std::vector<FmGeometry> geo(nc);
-        long long need = 0;
-        for (int i = 0; i < nc; ++i) {
-            wefax_fm_chart &ch = found[i];
-            const long long from = std::min<long long>(ch.search_from, n - 1);
-            geo[i] = fm_geometry(ch.lpm, ch.ioc, sp, from, ch.image_end);
-            ch.width = geo[i].W;
-            if (ch.status == WEFAX_FM_CHART_OK) need += (long long)geo[i].rows_max * geo[i].W;
+            // ---- charts of each recording; the LPM of every chart of the wave in one launch ------------------------
+            std::vector<std::vector<wefax_fm_chart>> found(gw);
+            std::vector<FmChartJob> lpm_tab;
+            std::vector<int> cls((size_t)nw);
+            for (int r = 0; r < gw; ++r) {
+                for (long long k = 0; k < nw; ++k) cls[k] = tone_class(h_tone + (size_t)r * tone_row + 4 * k);
+                found[r] = find_charts(cls, n);
+                n_charts[w0 + r] = (int)found[r].size();
+                found[r].resize(std::min<size_t>(found[r].size(), (size_t)max_charts));
+                for (wefax_fm_chart &c : found[r]) {
+                    c.lpm = prm.lpm;
+                    if (prm.ioc > 0) c.ioc = prm.ioc;
+                    if (prm.lpm > 0.0) continue;
+                    FmChartJob j;
+                    memset(&j, 0, sizeof(j));
+                    j.g = g + (size_t)r * n;
+                    j.n = n;
+                    j.from = std::min<long long>(c.search_from, n - 1);
+                    lpm_tab.push_back(j);
+                }
+            }
+            if (!lpm_tab.empty()) {
+                const int nl = (int)lpm_tab.size();
+                const size_t tab_bytes = ((size_t)nl * sizeof(FmChartJob) + 255) / 256 * 256;
+                char *buf = (char *)ctx->work_misc.reserve(tab_bytes + (size_t)nl * n_cand * sizeof(double));
+                FmChartJob *d_tab = (FmChartJob *)buf;
+                double *d_score = (double *)(buf + tab_bytes);
+                CUDA_CHECK(cudaMemcpyAsync(d_tab, lpm_tab.data(), (size_t)nl * sizeof(FmChartJob), cudaMemcpyHostToDevice, st));
+                launch_fm_lpm(ctx, d_tab, nl, cand, prm.fold_lines, d_score);
+                double *h_score = (double *)pinned(ctx, (size_t)nl * n_cand * sizeof(double));
+                CUDA_CHECK(cudaMemcpyAsync(h_score, d_score, (size_t)nl * n_cand * sizeof(double), cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaStreamSynchronize(st));
+                int t = 0;
+                for (auto &rec : found)
+                    for (wefax_fm_chart &c : rec) {
+                        const double *sc = h_score + (size_t)(t++) * n_cand;
+                        int best = 0;
+                        for (int k = 1; k < n_cand; ++k)
+                            if (sc[k] > sc[best]) best = k;
+                        c.lpm = cand_lpm[best];
+                        c.lpm_score = sc[best];
+                        if (c.lpm_score < WEFAX_FM_LPM_MIN_SCORE) c.status = WEFAX_FM_CHART_NO_LPM;
+                    }
+            }
+
+            // ---- every picture of the wave: one table, packed from img_off on --------------------------------------
+            std::vector<FmTail> cs;
+            long long wave_need = 0;
+            for (int r = 0; r < gw; ++r)
+                for (wefax_fm_chart &c : found[r]) {
+                    const long long from = std::min<long long>(c.search_from, n - 1);
+                    const FmGeometry fg = fm_geometry(c.lpm, c.ioc, sp, from, c.image_end);
+                    c.width = fg.W;
+                    if (c.status != WEFAX_FM_CHART_OK) continue;
+                    wave_need += (long long)fg.rows_max * fg.W;
+                    if (!images) continue;
+                    FmTail t;
+                    t.g = g + (size_t)r * n;
+                    t.n = n;
+                    t.from = from;
+                    t.image_end = c.image_end;
+                    t.fg = fg;
+                    t.picture = true;
+                    cs.push_back(t);
+                }
+            need += wave_need;
+            if (images && need > image_capacity) too_small = true;   // (the remaining waves still count what they need)
+            long long bytes = 0;
+            if (!too_small && !cs.empty()) {
+                uint8_t *d_img = out_dev ? images + img_off : (uint8_t *)ctx->out_raster.reserve((size_t)wave_need + 1);
+                bytes = fm_tail(ctx, cs, prm.fold_lines, sp, d_img);
+                if (!out_dev && bytes > 0)
+                    CUDA_CHECK(cudaMemcpyAsync(images + img_off, d_img, (size_t)bytes, cudaMemcpyDeviceToHost, st));
+            }
+            CUDA_CHECK(cudaStreamSynchronize(st));
+            size_t t = 0;
+            long long off = img_off;
+            for (int r = 0; r < gw; ++r)
+                for (size_t i = 0; i < found[r].size(); ++i) {
+                    wefax_fm_chart &c = found[r][i];
+                    c.image_offset = off;
+                    if (images && c.status == WEFAX_FM_CHART_OK && !too_small) {
+                        const FmTail &p = cs[t++];
+                        c.image_offset = img_off + p.offset;
+                        c.rows = p.rows;
+                        c.line_start = p.line_start;
+                        c.slant = p.so;
+                        off = c.image_offset + (long long)p.rows * p.fg.W;
+                    }
+                    charts[(size_t)(w0 + r) * max_charts + i] = c;
+                }
+            img_off += bytes;
         }
-        if (images && need > image_capacity)
-            WEFAX_THROW(WEFAX_ERR_INVALID, "image_capacity %lld too small (need %lld)", image_capacity, need);
-        long long offset = 0;
-        for (int i = 0; i < nc; ++i) {
-            wefax_fm_chart &ch = found[i];
-            ch.image_offset = offset;
-            if (!images || ch.status != WEFAX_FM_CHART_OK) continue;
-            const FmGeometry &fg = geo[i];
-            uint8_t *d_img = nullptr;
-            if (fg.rows_max > 0)
-                d_img = out_dev ? images + offset : (uint8_t *)ctx->out_raster.reserve((size_t)fg.rows_max * fg.W);
-            const long long from = std::min<long long>(ch.search_from, n - 1);
-            const FmPicture pic = fm_picture(ctx, g, n, from, ch.image_end, fg, prm.fold_lines, sp, d_img);
-            if (!out_dev && d_img && pic.rows > 0)
-                CUDA_CHECK(cudaMemcpy(images + offset, d_img, (size_t)pic.rows * fg.W, cudaMemcpyDeviceToHost));
-            ch.rows = pic.rows;
-            ch.line_start = pic.line_start;
-            ch.slant = pic.so;
-            offset += (long long)pic.rows * fg.W;
-        }
-        CUDA_CHECK(cudaStreamSynchronize(st));
-        for (int i = 0; i < nc; ++i) charts[i] = found[i];
+        if (too_small) WEFAX_THROW(WEFAX_ERR_INVALID, "image_capacity %lld too small (need %lld)", image_capacity, need);
     });
 }
 

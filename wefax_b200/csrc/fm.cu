@@ -56,11 +56,15 @@ FirParams make_bandpass_fir(double lo_hz, double hi_hz, double fs, int taps) {
     return fp;
 }
 
-// grey[i] = (f_inst - black) / (white - black), f_inst from the phase step z[i] * conj(z[i-1])
+// grey[i] = (f_inst - black) / (white - black), f_inst from the phase step z[i] * conj(z[i-1]); blockIdx.y = recording
 __global__ void __launch_bounds__(256)
-fm_grey_kernel(const float *x, const float *y, float *g, long long n, float hz_per_rad, float black, float inv_span) {
+fm_grey_kernel(const float *x, const float *y, size_t xs, float *g, long long n, float hz_per_rad, float black,
+               float inv_span) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    x += blockIdx.y * xs;
+    y += blockIdx.y * xs;
+    g += blockIdx.y * (size_t)n;
     const long long j = i > 0 ? i - 1 : 0, k = i > 0 ? i : 1;   // sample 0 repeats the first step
     const float xr = __ldg(x + k), yr = __ldg(y + k), xp = __ldg(x + j), yp = __ldg(y + j);
     const float re = fmaf(xr, xp, yr * yp), im = fmaf(yr, xp, -xr * yp);
@@ -71,11 +75,18 @@ fm_grey_kernel(const float *x, const float *y, float *g, long long n, float hz_p
 __device__ __forceinline__ float clip01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
 
 // P[o] = sum over lines of clip(grey[from + floor(l * Ls + o)]), o < Lc = ceil(Ls); l * Ls and the sum each rounded
-// (no fused multiply-add: at a line length that is not a binary fraction the fused form can pick the next sample)
+// (no fused multiply-add: at a line length that is not a binary fraction the fused form can pick the next sample).
+// blockIdx.y = chart of the table (charts with phase = 0 are skipped), P of chart c at P + c * ps
 __global__ void __launch_bounds__(256)
-fm_fold_kernel(const float *g, long long n, long long from, double Ls, int lines, int Lc, float *P) {
+fm_fold_kernel(const FmChartJob *tab, int lines, float *P, int ps) {
+    const FmChartJob &job = tab[blockIdx.y];
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    if (o >= Lc) return;
+    const int Lc = job.Lc;
+    if (!job.phase || o >= Lc) return;
+    const float *g = job.g;
+    const long long n = job.n, from = job.from;
+    const double Ls = job.Ls;
+    P += (size_t)blockIdx.y * ps;
     float acc = 0.f;
     for (int l = 0; l < lines; ++l) {
         const long long i = from + (long long)floor(__dadd_rn(__dmul_rn((double)l, Ls), (double)o));
@@ -84,12 +95,18 @@ fm_fold_kernel(const float *g, long long n, long long from, double Ls, int lines
     P[o] = acc;
 }
 
-// line start = from + arg max_o sum_{j < wb} P[(o + j) mod Lc]  (smallest o on ties); one CTA
+// line start = from + arg max_o sum_{j < wb} P[(o + j) mod Lc]  (smallest o on ties); one CTA per chart with phase = 1
 __global__ void __launch_bounds__(1024)
-fm_phase_kernel(const float *P, int Lc, int wb, long long from, long long *line_start) {
+fm_phase_kernel(const FmChartJob *tab, const float *P, int ps, long long *line_start) {
     extern __shared__ double pre[];    // pre[i] = sum_{j < i} P[j mod Lc], i <= 2*Lc (two periods: circular boxcar)
     __shared__ double s_part[1024];
     __shared__ unsigned long long s_best[32];
+    const FmChartJob &job = tab[blockIdx.x];
+    if (!job.phase) return;
+    const int Lc = job.Lc, wb = job.wb;
+    const long long from = job.from;
+    P += (size_t)blockIdx.x * ps;
+    line_start += blockIdx.x;
     const int tid = threadIdx.x, nt = blockDim.x, total = 2 * Lc;
     // chunked scan: each thread sums a contiguous chunk, thread 0 scans the chunk totals
     const int chunk = (total + nt - 1) / nt;
@@ -136,13 +153,19 @@ fm_phase_kernel(const float *P, int Lc, int wb, long long from, long long *line_
 
 // pixel (r, p): box average of clip(grey) over [a, a + Ls / W), a = line_start + r * Ls + p * Ls / W.
 // rows = min(rows_max, floor((image_end - line_start) / Ls)), the host's expression (wefax_decode_fm_slant), so
-// every row the caller is told about is written; grid.y strides over the rows (it is capped at 65535)
+// every row the caller is told about is written; grid.y strides over the rows (it is capped at 65535), grid.z is the
+// chart of the table, grid.x covers the widest picture
 __global__ void __launch_bounds__(256)
-fm_image_kernel(const float *g, long long n, const long long *line_start, double Ls, int W, int rows_max,
-                long long image_end, uint8_t *img) {
+fm_image_kernel(const FmChartJob *tab, const long long *line_start, uint8_t *img) {
+    const FmChartJob &job = tab[blockIdx.z];
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= W) return;
-    const long long ls_i = *line_start;
+    const int W = job.W, rows_max = job.rows_max;
+    if (p >= W || rows_max <= 0) return;
+    const float *g = job.g;
+    const long long n = job.n, image_end = job.image_end;
+    const double Ls = job.Ls;
+    img += job.out;
+    const long long ls_i = line_start[blockIdx.z];
     const double ls = (double)ls_i;
     const long long rows = min((long long)rows_max, (long long)floor(__ddiv_rn((double)(image_end - ls_i), Ls)));
     const double step = Ls / (double)W;
@@ -162,10 +185,18 @@ fm_image_kernel(const float *g, long long n, const long long *line_start, double
 
 // ---- slant: the sample-clock error measured from the white line pulses (DESIGN.md §4.7a) ----
 
-// Q[l][b] = mean of clip(grey) over [from + floor(l * Ls) + b * D, +D); samples at or past n count as 0.  One CTA per line.
+// Q[l][b] = mean of clip(grey) over [from + floor(l * Ls) + b * D, +D); samples at or past n count as 0.  One CTA per
+// (line, chart), Ls = the chart's sLs, lines l < q_lines
 __global__ void __launch_bounds__(256)
-fm_slant_profile_kernel(const float *g, long long n, long long from, double Ls, int D, int Bn, float *Q) {
+fm_slant_profile_kernel(const FmChartJob *tab, float *Q) {
+    const FmChartJob &job = tab[blockIdx.y];
     const int l = blockIdx.x;
+    if (l >= job.q_lines) return;
+    const float *g = job.g;
+    const long long n = job.n, from = job.from;
+    const double Ls = job.sLs;
+    const int D = job.D, Bn = job.Bn;
+    Q += job.q_off;
     const long long base = from + (long long)floor((double)l * Ls);
     for (int b = threadIdx.x; b < Bn; b += blockDim.x) {
         const long long i0 = base + (long long)b * D;
@@ -181,11 +212,17 @@ __device__ __forceinline__ int floor_div(int a, int b) { return a / b - ((a % b 
 // One CTA per candidate c of the total shift k over `lines` lines (c = 0, 1, 2, 3, 4, ... -> k = 0, -2, +2, -4, +4, ...):
 // S_k[b] = sum_l Q[l][(b + round(l * k / lines)) mod Bn], circular boxcar of wbb bins, arg max over (c, b) into *best as
 // (score bits << 32) | (0x7fffffff - (c * Bn + b)): the highest score wins, then the smallest |k|, then the smallest b.
+// blockIdx.y = chart (lines = q_lines, candidates c < n_cand), its key into best[chart]
 __global__ void __launch_bounds__(1024)
-fm_slant_fold_kernel(const float *Q, int lines, int Bn, int wbb, unsigned long long *best) {
+fm_slant_fold_kernel(const FmChartJob *tab, const float *Q, unsigned long long *best) {
     extern __shared__ float S[];
     __shared__ unsigned long long s_best[32];
+    const FmChartJob &job = tab[blockIdx.y];
     const int c = blockIdx.x, tid = threadIdx.x;
+    if (c >= job.n_cand) return;
+    const int lines = job.q_lines, Bn = job.Bn, wbb = job.wbb;
+    Q += job.q_off;
+    best += blockIdx.y;
     const int k = c == 0 ? 0 : ((c + 1) / 2) * 2 * ((c & 1) ? -1 : 1);
     for (int b = tid; b < Bn; b += blockDim.x) {
         float acc = 0.f;
@@ -221,12 +258,20 @@ fm_slant_fold_kernel(const float *Q, int lines, int Bn, int wbb, unsigned long l
 // One warp per line l < lines: the pulse is the arg max over x in [c - R, c + R], c = floor(a + l * s + 0.5), of the
 // width-wb boxcar of clip(grey) (smallest x on ties); contrast = boxcar mean - mean of the guard bands [x - wb, x) and
 // [x + wb, x + 2 wb).  pos[l] = x when the contrast reaches min_contrast, else -1 (also when the window leaves the
-// recording).  Boxcars from float64 prefix sums of the window in shared memory.
+// recording).  Boxcars from float64 prefix sums of the window in shared memory.  blockIdx.y = chart (a, s, wb = swb,
+// R; lines l < track_lines), pos / contrast from its pos_off.
 __global__ void __launch_bounds__(32)
-fm_slant_track_kernel(const float *g, long long n, double a, double s, int wb, int R, double min_contrast,
-                      long long *pos, float *contrast) {
+fm_slant_track_kernel(const FmChartJob *tab, double min_contrast, long long *pos, float *contrast) {
     extern __shared__ double pre[];    // pre[i] = sum_{j < i} clip(g[lo + j]), i <= span
+    const FmChartJob &job = tab[blockIdx.y];
     const int l = blockIdx.x, lane = threadIdx.x;
+    if (l >= job.track_lines) return;
+    const float *g = job.g;
+    const long long n = job.n;
+    const double a = job.a, s = job.s;
+    const int wb = job.swb, R = job.R;
+    pos += job.pos_off;
+    contrast += job.pos_off;
     const long long c = (long long)floor(a + (double)l * s + 0.5);
     const long long lo = c - R - wb;
     const int span = 2 * R + 3 * wb;
@@ -313,12 +358,12 @@ __device__ __forceinline__ void block_sum(double (&v)[K], double *s) {
 // (f * j) mod 11025, r_f = 2 |C_f|^2 / (T^2 V) (0 when V = 0).  out[k] = (r_300, r_450, r_675, V)
 constexpr int kToneThreads = 256;
 __global__ void __launch_bounds__(kToneThreads)
-fm_tone_kernel(const float *g, float4 *out) {
+fm_tone_kernel(const float *g, long long n, long long nw, float4 *out) {
     constexpr int T = WEFAX_FM_TONE_WINDOW;
     constexpr int F[3] = {300, 450, 675};
     __shared__ float u[T];
     __shared__ double s_red[32 * 7];
-    const float *w = g + (size_t)blockIdx.x * T;
+    const float *w = g + blockIdx.y * (size_t)n + (size_t)blockIdx.x * T;   // blockIdx.y = recording
     double m[1] = {0.0};
     for (int j = threadIdx.x; j < T; j += blockDim.x) {
         const float v = clip01(__ldg(w + j));
@@ -346,21 +391,22 @@ fm_tone_kernel(const float *g, float4 *out) {
         for (int f = 0; f < 3; ++f)
             r[f] = a[0] > 0.0 ? (float)(2.0 * (a[1 + 2 * f] * a[1 + 2 * f] + a[2 + 2 * f] * a[2 + 2 * f]) / ((double)T * a[0]))
                               : 0.f;
-        out[blockIdx.x] = make_float4(r[0], r[1], r[2], (float)(a[0] / T));
+        out[blockIdx.y * (size_t)nw + blockIdx.x] = make_float4(r[0], r[1], r[2], (float)(a[0] / T));
     }
 }
 
 // One CTA per (chart, candidate): the phasing fold of fm_fold_kernel (same index, same float32 sums in line order) for
-// the candidate's line length from the chart's search_from, kept in shared memory, then
+// the candidate's line length from the chart's `from` in its grey stream, kept in shared memory, then
 // score = max_o sum_{j < wb} P[(o + j) mod Lc] / (wb * lines) - mean(P) / lines  (boxcar sums in float64)
 __global__ void __launch_bounds__(1024)
-fm_lpm_kernel(const float *g, long long n, const long long *from, LpmCandidates cand, int lines, double *score) {
+fm_lpm_kernel(const FmChartJob *tab, LpmCandidates cand, int lines, double *score) {
     __shared__ float P[kLpmMaxLine];
     __shared__ double s_red[32 * 2];
     const int chart = blockIdx.x / cand.n, c = blockIdx.x % cand.n, tid = threadIdx.x, nt = blockDim.x;
     const double Ls = cand.Ls[c];
     const int Lc = cand.Lc[c], wb = cand.wb[c];
-    const long long f0 = from[chart];
+    const float *g = tab[chart].g;
+    const long long n = tab[chart].n, f0 = tab[chart].from;
     double tot[1] = {0.0};
     for (int o = tid; o < Lc; o += nt) {
         float acc = 0.f;
@@ -394,39 +440,41 @@ fm_lpm_kernel(const float *g, long long n, const long long *from, LpmCandidates 
     }
 }
 
-void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n_windows, float4 *out) {
-    if (n_windows <= 0) return;
+void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n, long long n_windows, int batch, float4 *out) {
+    if (n_windows <= 0 || batch <= 0) return;
     StageTimer timer(ctx, "fm_tone");
-    fm_tone_kernel<<<(unsigned)n_windows, kToneThreads, 0, ctx->stream>>>(g, out);
+    fm_tone_kernel<<<dim3((unsigned)n_windows, batch), kToneThreads, 0, ctx->stream>>>(g, n, n_windows, out);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_lpm(wefax_ctx *ctx, const float *g, long long n, const long long *d_from, int n_charts,
-                   const LpmCandidates &cand, int lines, double *d_score) {
+void launch_fm_lpm(wefax_ctx *ctx, const FmChartJob *d_tab, int n_charts, const LpmCandidates &cand, int lines,
+                   double *d_score) {
     if (n_charts <= 0) return;
     StageTimer timer(ctx, "fm_lpm");
-    fm_lpm_kernel<<<(unsigned)(n_charts * cand.n), 1024, 0, ctx->stream>>>(g, n, d_from, cand, lines, d_score);
+    fm_lpm_kernel<<<(unsigned)(n_charts * cand.n), 1024, 0, ctx->stream>>>(d_tab, cand, lines, d_score);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, float *g, long long n, double black_hz,
-                    double white_hz) {
+void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, size_t xs, float *g, long long n, int batch,
+                    double black_hz, double white_hz) {
     StageTimer timer(ctx, "fm_grey");
     const float hz_per_rad = (float)((double)WEFAX_TARGET_RATE / (2.0 * M_PI));
-    fm_grey_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(x, y, g, n, hz_per_rad, (float)black_hz,
-                                                                       (float)(1.0 / (white_hz - black_hz)));
+    fm_grey_kernel<<<dim3((unsigned)((n + 255) / 256), batch), 256, 0, ctx->stream>>>(
+        x, y, xs, g, n, hz_per_rad, (float)black_hz, (float)(1.0 / (white_hz - black_hz)));
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_phasing(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int lines, float *P,
-                       long long *d_line_start) {
+void launch_fm_phasing(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts, int lines,
+                       float *P, long long *d_line_start) {
+    int Lc = 0;
+    for (int c = 0; c < n_charts; ++c)
+        if (h_tab[c].phase) Lc = std::max(Lc, h_tab[c].Lc);
+    if (Lc == 0) return;
     StageTimer timer(ctx, "fm_phasing");
-    const int Lc = (int)ceil(Ls);
-    const int wb = std::max(1, (int)llround(0.05 * Ls));
-    fm_fold_kernel<<<(Lc + 255) / 256, 256, 0, ctx->stream>>>(g, n, from, Ls, lines, Lc, P);
+    fm_fold_kernel<<<dim3((Lc + 255) / 256, n_charts), 256, 0, ctx->stream>>>(d_tab, lines, P, Lc);
     const size_t smem = (size_t)(2 * Lc + 1) * sizeof(double);
     if (smem > 200 * 1024) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "line of %d samples is too long for the phasing search", Lc);
     const void *fn = (const void *)fm_phase_kernel;
@@ -434,48 +482,73 @@ void launch_fm_phasing(wefax_ctx *ctx, const float *g, long long n, long long fr
         CUDA_CHECK(cudaFuncSetAttribute(fm_phase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         ctx->smem_configured[fn] = 1;
     }
-    fm_phase_kernel<<<1, 1024, smem, ctx->stream>>>(P, Lc, wb, from, d_line_start);
+    fm_phase_kernel<<<n_charts, 1024, smem, ctx->stream>>>(d_tab, P, Lc, d_line_start);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches += 2;
 }
 
-void launch_fm_image(wefax_ctx *ctx, const float *g, long long n, const long long *d_line_start, double Ls, int W,
-                     int rows_max, long long image_end, uint8_t *img) {
-    if (rows_max <= 0) return;
+void launch_fm_image(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
+                     const long long *d_line_start, uint8_t *img) {
+    int W = 0, rows = 0;
+    for (int c = 0; c < n_charts; ++c)
+        if (h_tab[c].rows_max > 0) {
+            W = std::max(W, h_tab[c].W);
+            rows = std::max(rows, h_tab[c].rows_max);
+        }
+    if (rows <= 0 || W <= 0) return;
     StageTimer timer(ctx, "fm_image");
-    dim3 grid((W + 255) / 256, std::min(rows_max, 65535));
-    fm_image_kernel<<<grid, 256, 0, ctx->stream>>>(g, n, d_line_start, Ls, W, rows_max, image_end, img);
+    dim3 grid((W + 255) / 256, std::min(rows, 65535), n_charts);
+    fm_image_kernel<<<grid, 256, 0, ctx->stream>>>(d_tab, d_line_start, img);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_slant_profile(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int D, int Bn,
-                             int lines, float *Q) {
+void launch_fm_slant_profile(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts, float *Q) {
+    int lines = 0;
+    for (int c = 0; c < n_charts; ++c) lines = std::max(lines, h_tab[c].q_lines);
+    if (lines <= 0) return;
     StageTimer timer(ctx, "fm_slant_profile");
-    fm_slant_profile_kernel<<<lines, 256, 0, ctx->stream>>>(g, n, from, Ls, D, Bn, Q);
+    fm_slant_profile_kernel<<<dim3(lines, n_charts), 256, 0, ctx->stream>>>(d_tab, Q);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_slant_fold(wefax_ctx *ctx, const float *Q, int lines, int Bn, int wbb, int n_cand,
-                          unsigned long long *d_best) {
+void launch_fm_slant_fold(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
+                          const float *Q, unsigned long long *d_best) {
+    int Bn = 0, n_cand = 0;
+    for (int c = 0; c < n_charts; ++c) {
+        const FmChartJob &j = h_tab[c];
+        if (j.q_lines <= 0) continue;
+        if (j.Bn > 8192 || (long long)j.n_cand * j.Bn > 0x7fffffffLL)
+            WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "slant search of %d bins x %d candidates is too large", j.Bn, j.n_cand);
+        Bn = std::max(Bn, j.Bn);
+        n_cand = std::max(n_cand, j.n_cand);
+    }
+    CUDA_CHECK(cudaMemsetAsync(d_best, 0, (size_t)n_charts * sizeof(unsigned long long), ctx->stream));
+    if (n_cand <= 0) return;
     StageTimer timer(ctx, "fm_slant_fold");
-    if (Bn > 8192 || (long long)n_cand * Bn > 0x7fffffffLL)
-        WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "slant search of %d bins x %d candidates is too large", Bn, n_cand);
     const int threads = std::min(1024, (Bn + 31) / 32 * 32);
-    CUDA_CHECK(cudaMemsetAsync(d_best, 0, sizeof(unsigned long long), ctx->stream));
-    fm_slant_fold_kernel<<<n_cand, threads, (size_t)Bn * sizeof(float), ctx->stream>>>(Q, lines, Bn, wbb, d_best);
+    fm_slant_fold_kernel<<<dim3(n_cand, n_charts), threads, (size_t)Bn * sizeof(float), ctx->stream>>>(d_tab, Q, d_best);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }
 
-void launch_fm_slant_track(wefax_ctx *ctx, const float *g, long long n, double a, double s, int lines, int wb, int R,
+void launch_fm_slant_track(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
                            double min_contrast, long long *pos, float *contrast) {
+    int lines = 0;
+    size_t smem = 0;
+    for (int c = 0; c < n_charts; ++c) {
+        const FmChartJob &j = h_tab[c];
+        if (j.track_lines <= 0) continue;
+        lines = std::max(lines, j.track_lines);
+        const size_t sm = (size_t)(2 * j.R + 3 * j.swb + 1) * sizeof(double);
+        if (sm > 48 * 1024)
+            WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "line pulse of %d samples is too long for the slant search", j.swb);
+        smem = std::max(smem, sm);
+    }
     if (lines <= 0) return;
     StageTimer timer(ctx, "fm_slant_track");
-    const size_t smem = (size_t)(2 * R + 3 * wb + 1) * sizeof(double);
-    if (smem > 48 * 1024) WEFAX_THROW(WEFAX_ERR_UNSUPPORTED, "line pulse of %d samples is too long for the slant search", wb);
-    fm_slant_track_kernel<<<lines, 32, smem, ctx->stream>>>(g, n, a, s, wb, R, min_contrast, pos, contrast);
+    fm_slant_track_kernel<<<dim3(lines, n_charts), 32, smem, ctx->stream>>>(d_tab, min_contrast, pos, contrast);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches++;
 }

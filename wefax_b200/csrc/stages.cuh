@@ -130,23 +130,43 @@ void launch_tone_peaks(wefax_ctx *ctx, const float2 *X, size_t xs, long long pac
 
 // ---- N4 extension: FM-discriminator demodulation and IOC pixel columns (fm.cu) ----
 FirParams make_bandpass_fir(double lo_hz, double hi_hz, double fs, int taps);
-void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, float *g, long long n, double black_hz,
-                    double white_hz);
-void launch_fm_phasing(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int lines, float *P,
-                       long long *d_line_start);
-void launch_fm_image(wefax_ctx *ctx, const float *g, long long n, const long long *d_line_start, double Ls, int W,
-                     int rows_max, long long image_end, uint8_t *img);
-// slant search (DESIGN.md §4.7a): Q = lines x Bn bin means of D samples from `from` on lines of Ls samples
-void launch_fm_slant_profile(wefax_ctx *ctx, const float *g, long long n, long long from, double Ls, int D, int Bn,
-                             int lines, float *Q);
-// sheared folds of Q for n_cand candidate total shifts, best (score, candidate, bin) key into d_best (device)
-void launch_fm_slant_fold(wefax_ctx *ctx, const float *Q, int lines, int Bn, int wbb, int n_cand,
-                          unsigned long long *d_best);
-// pulse position (or -1) and contrast of lines [0, lines) around a + l * s, +-R samples, pulse width wb
-void launch_fm_slant_track(wefax_ctx *ctx, const float *g, long long n, double a, double s, int lines, int wb, int R,
+// grey of `batch` recordings: x / y rows of stride xs, g rows of n samples
+void launch_fm_grey(wefax_ctx *ctx, const float *x, const float *y, size_t xs, float *g, long long n, int batch,
+                    double black_hz, double white_hz);
+// One chart of the FM decode's picture stage, which runs once over a table of charts (DESIGN.md §4.7c): where its grey
+// stream lies, its span, the phasing fold and picture geometry, its output offset, and its slant search state
+struct FmChartJob {
+    const float *g;         // grey stream of the chart's recording, n samples
+    long long n, from, image_end;
+    double Ls;              // line length of the phasing fold and of the picture
+    int Lc, wb;             // phasing fold: ceil(Ls) offsets, boxcar of wb samples
+    int phase;              // 1: line start from the phasing fold; 0: given (the slant fit)
+    int W, rows_max;        // picture: W pixels per row, rows_max rows at most (0: no picture)
+    long long out;          // offset (bytes) of the picture in the output
+    // slant search (AUTO): profile of q_lines lines of the nominal line sLs in Bn bins of D samples (Q from q_off),
+    // n_cand sheared folds; pulse tracking of track_lines lines around a + l * s (pos / contrast from pos_off)
+    double sLs, a, s;
+    int D, Bn, wbb, R, swb, q_lines, n_cand, track_lines;
+    long long q_off, pos_off;
+};
+// line start of every chart with phase = 1 into d_line_start[chart]: the fold of `lines` lines (P: max Lc floats per chart)
+void launch_fm_phasing(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts, int lines,
+                       float *P, long long *d_line_start);
+// every chart's picture (rows_max > 0) into img + out
+void launch_fm_image(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
+                     const long long *d_line_start, uint8_t *img);
+// slant search (DESIGN.md §4.7a), per chart with q_lines > 0: Q = q_lines x Bn bin means of D samples from `from`
+void launch_fm_slant_profile(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts, float *Q);
+// sheared folds of each chart's Q for its n_cand candidate total shifts, best (score, candidate, bin) key into
+// d_best[chart] (device)
+void launch_fm_slant_fold(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
+                          const float *Q, unsigned long long *d_best);
+// pulse position (or -1) and contrast of lines [0, track_lines) of each chart around a + l * s, +-R samples, pulse width swb
+void launch_fm_slant_track(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
                            double min_contrast, long long *pos, float *contrast);
-// charts (DESIGN.md §4.7b): (r_300, r_450, r_675, V) of each whole WEFAX_FM_TONE_WINDOW window of g into out
-void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n_windows, float4 *out);
+// charts (DESIGN.md §4.7b): (r_300, r_450, r_675, V) of each whole WEFAX_FM_TONE_WINDOW window of g into out, for
+// `batch` recordings of n samples (g) and n_windows windows (out) each
+void launch_fm_tone(wefax_ctx *ctx, const float *g, long long n, long long n_windows, int batch, float4 *out);
 // the LPM candidates' line lengths Ls = 60 / lpm * 11025, Lc = ceil(Ls) <= kLpmMaxLine, boxcars wb = max(1, round(0.05 Ls))
 constexpr int kLpmMaxLine = 11025;
 struct LpmCandidates {
@@ -154,8 +174,9 @@ struct LpmCandidates {
     double Ls[WEFAX_FM_MAX_LPM_CANDIDATES];
     int Lc[WEFAX_FM_MAX_LPM_CANDIDATES], wb[WEFAX_FM_MAX_LPM_CANDIDATES];
 };
-// phasing score of every (chart, candidate), chart-major, folding `lines` lines from d_from[chart] (device)
-void launch_fm_lpm(wefax_ctx *ctx, const float *g, long long n, const long long *d_from, int n_charts,
-                   const LpmCandidates &cand, int lines, double *d_score);
+// phasing score of every (chart, candidate), chart-major, folding `lines` lines from each chart's `from` in its grey
+// stream (d_tab: g, n, from)
+void launch_fm_lpm(wefax_ctx *ctx, const FmChartJob *d_tab, int n_charts, const LpmCandidates &cand, int lines,
+                   double *d_score);
 
 }  // namespace wefax

@@ -10,7 +10,8 @@ and has no reference parity; see ``oracle/fm_oracle.py`` and ``tests/test_gpu_fm
 :func:`decode_fm` decodes one picture whose LPM and IOC the caller knows.  Its default span comes from the AM path's
 tone test (:func:`image_span`), which finds only the first IOC 576 chart of a recording.  :func:`decode_fm_charts`
 finds every chart of a recording in the FM grey stream itself (start tones at 300 / 675 Hz, stop tone at 450 Hz),
-measures each chart's LPM from its phasing lines and decodes them all from one front end (``wefax_decode_fm_charts``).
+measures each chart's LPM from its phasing lines and decodes them all from one front end (``wefax_decode_fm_charts``);
+:func:`decode_fm_charts_batch` does the same for a batch of equal-length recordings in one call.
 """
 from __future__ import annotations
 
@@ -186,6 +187,37 @@ def chart_params(lpm=None, ioc=None, lpm_candidates=None, slant=None, max_slant_
     return N.FmChartParams(prm, sp, len(cands), arr)
 
 
+def _max_charts(max_charts):
+    if isinstance(max_charts, bool) or not isinstance(max_charts, numbers.Integral) or max_charts < 0:
+        raise ValueError(f"max_charts must be a non-negative integer, not {max_charts!r}")
+    return int(max_charts)
+
+
+def _image_bound(prm, lpm, ioc, n_out: int) -> int:
+    """Bytes that hold the pictures of any recording of n_out samples (at 11025 Hz): the charts' spans are disjoint,
+    so ceil(n_out / shortest line) rows of the widest picture hold them all."""
+    ls_min = 60.0 / (float(lpm) if lpm else max(prm.lpm_candidates[: prm.n_lpm_candidates])) * N.TARGET_RATE
+    sp = prm.slant
+    if sp.mode != N.FM_SLANT_OFF:
+        ls_min = ls_min / (1.0 + (sp.max_ppm if sp.mode == N.FM_SLANT_AUTO else max(sp.ppm, 0.0)) * 1e-6)
+    w_max = int(round(math.pi * (ioc if ioc else 576)))
+    return int(math.ceil(n_out / ls_min)) * w_max
+
+
+def _charts(out, n_found: int, max_charts: int, img, prm) -> list:
+    """FmChart of the native chart entries ``out`` (pictures cut from ``img``, None when pictures were not asked for)."""
+    charts = []
+    for c in out[: min(n_found, max_charts)]:
+        decoded = img is not None and c.status == N.FM_CHART_OK
+        picture = img[c.image_offset: c.image_offset + c.rows * c.width].reshape(c.rows, c.width) if decoded else None
+        so = FmSlant(**{name: getattr(c.slant, name) for name, _ in N.FmSlantOut._fields_}) \
+            if (decoded and prm.slant.mode != N.FM_SLANT_OFF) else None
+        charts.append(FmChart(int(c.tone_begin), int(c.search_from), int(c.image_end), bool(c.stop_found), int(c.ioc),
+                              float(c.lpm), float(c.lpm_score), int(c.status), int(c.width), int(c.line_start),
+                              picture, so))
+    return charts
+
+
 def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_candidates=None, slant=None,
                      max_slant_ppm: float = 300.0, max_charts: int = 64, fold_lines: int = 20,
                      black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0), fir_taps: int = 63,
@@ -200,19 +232,12 @@ def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_can
     search_from and image_end.  ``want_images=False`` returns the chart list only; ``image_capacity`` overrides the
     size of the picture buffer (bytes; default: enough for any recording of this length)."""
     prm = chart_params(lpm, ioc, lpm_candidates, slant, max_slant_ppm, fold_lines, black_hz, white_hz, band, fir_taps)
-    if isinstance(max_charts, bool) or not isinstance(max_charts, numbers.Integral) or max_charts < 0:
-        raise ValueError(f"max_charts must be a non-negative integer, not {max_charts!r}")
+    max_charts = _max_charts(max_charts)
     pcm = np.ascontiguousarray(pcm, dtype=np.int16)
     n_in, ch = int(pcm.shape[0]), (1 if pcm.ndim == 1 else int(pcm.shape[1]))
     n_out = n_in if sample_rate == N.TARGET_RATE else N.resampled_length(n_in, sample_rate)
     if image_capacity is None:
-        # the charts' spans are disjoint: ceil(n_out / shortest line) rows of the widest picture hold them all
-        ls_min = 60.0 / (float(lpm) if lpm else max(prm.lpm_candidates[: prm.n_lpm_candidates])) * N.TARGET_RATE
-        sp = prm.slant
-        if sp.mode != N.FM_SLANT_OFF:
-            ls_min = ls_min / (1.0 + (sp.max_ppm if sp.mode == N.FM_SLANT_AUTO else max(sp.ppm, 0.0)) * 1e-6)
-        w_max = int(round(math.pi * (ioc if ioc else 576)))
-        image_capacity = int(math.ceil(n_out / ls_min)) * w_max if want_images else 0
+        image_capacity = _image_bound(prm, lpm, ioc, n_out) if want_images else 0
     img = np.zeros(max(1, image_capacity), dtype=np.uint8) if want_images else None
     grey = np.zeros(n_out, dtype=np.float32) if want_grey else None
     tones = np.zeros((n_out // N.FM_TONE_WINDOW, 4), dtype=np.float32) if want_tone_scores else None
@@ -223,17 +248,56 @@ def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_can
         decoder._h, C.byref(desc), C.c_void_p(pcm.ctypes.data), C.byref(prm), out, int(max_charts), C.byref(n_found),
         img.ctypes.data if want_images else None, int(image_capacity),
         tones.ctypes.data if want_tone_scores else None, grey.ctypes.data if want_grey else None))
-    charts = []
-    for c in out[: min(n_found.value, max_charts)]:
-        picture = None
-        if want_images and c.status == N.FM_CHART_OK:
-            picture = img[c.image_offset: c.image_offset + c.rows * c.width].reshape(c.rows, c.width)
-        so = FmSlant(**{name: getattr(c.slant, name) for name, _ in N.FmSlantOut._fields_}) \
-            if (want_images and c.status == N.FM_CHART_OK and prm.slant.mode != N.FM_SLANT_OFF) else None
-        charts.append(FmChart(int(c.tone_begin), int(c.search_from), int(c.image_end), bool(c.stop_found), int(c.ioc),
-                              float(c.lpm), float(c.lpm_score), int(c.status), int(c.width), int(c.line_start),
-                              picture, so))
-    return FmCharts(charts, int(n_found.value), grey, tones)
+    return FmCharts(_charts(out, n_found.value, max_charts, img, prm), int(n_found.value), grey, tones)
+
+
+def decode_fm_charts_batch(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_candidates=None, slant=None,
+                           max_slant_ppm: float = 300.0, max_charts: int = 64, fold_lines: int = 20,
+                           black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0),
+                           fir_taps: int = 63, want_images: bool = True, want_grey: bool = False,
+                           want_tone_scores: bool = False, image_capacity: int | None = None) -> list:
+    """:func:`decode_fm_charts` of R recordings of equal length in one call (``wefax_decode_fm_charts_batch``): one
+    FmCharts per recording, each what :func:`decode_fm_charts` returns for that recording alone.
+
+    ``pcm``: int16 ``(R, n)`` mono or ``(R, n, 2)`` stereo, as numpy (host) or as a CUDA torch tensor (read in place on
+    the device).  The outputs are numpy arrays on the host.  ``image_capacity`` is the byte size of the picture buffer
+    of the whole batch (default: R times the bound of :func:`decode_fm_charts`)."""
+    prm = chart_params(lpm, ioc, lpm_candidates, slant, max_slant_ppm, fold_lines, black_hz, white_hz, band, fir_taps)
+    max_charts = _max_charts(max_charts)
+    if isinstance(sample_rate, bool) or not isinstance(sample_rate, numbers.Integral) or sample_rate < 1:
+        raise ValueError(f"sample_rate must be a positive integer, not {sample_rate!r}")
+    flags, keep = 0, pcm
+    if type(pcm).__module__.startswith("torch"):
+        import torch
+        if not pcm.is_cuda or pcm.dtype != torch.int16:
+            raise ValueError(f"a torch pcm must be an int16 CUDA tensor, not {pcm.dtype} on {pcm.device}")
+        keep = pcm.contiguous()
+        ptr, shape, flags = keep.data_ptr(), tuple(keep.shape), N.F_PCM_ON_DEVICE
+    else:
+        keep = np.ascontiguousarray(pcm, dtype=np.int16)
+        ptr, shape = keep.ctypes.data, keep.shape
+    if not (len(shape) == 2 or (len(shape) == 3 and shape[2] == 2)) or shape[0] < 1 or shape[1] < 1:
+        raise ValueError(f"pcm must be (R, n) or (R, n, 2) with R, n >= 1, not {shape}")
+    R, n_in, ch = int(shape[0]), int(shape[1]), (1 if len(shape) == 2 else 2)
+    n_out = n_in if sample_rate == N.TARGET_RATE else N.resampled_length(n_in, sample_rate)
+    if image_capacity is None:
+        image_capacity = R * _image_bound(prm, lpm, ioc, n_out) if want_images else 0
+    img = np.zeros(max(1, image_capacity), dtype=np.uint8) if want_images else None
+    grey = np.zeros((R, n_out), dtype=np.float32) if want_grey else None
+    tones = np.zeros((R, n_out // N.FM_TONE_WINDOW, 4), dtype=np.float32) if want_tone_scores else None
+    out = (N.FmChart * max(1, R * max_charts))()
+    n_found = (C.c_int * R)()
+    desc = N.BatchDesc(R, n_in, ch, int(sample_rate), 0.0, 0.0, flags)
+    decoder._check(decoder._lib.wefax_decode_fm_charts_batch(
+        decoder._h, C.byref(desc), C.c_void_p(ptr), C.byref(prm), out, max_charts, n_found,
+        img.ctypes.data if want_images else None, int(image_capacity),
+        tones.ctypes.data if want_tone_scores else None, grey.ctypes.data if want_grey else None))
+    res = []
+    for r in range(R):
+        entries = out[r * max_charts: (r + 1) * max_charts]
+        res.append(FmCharts(_charts(entries, n_found[r], max_charts, img, prm), int(n_found[r]),
+                            None if grey is None else grey[r], None if tones is None else tones[r]))
+    return res
 
 
 def _pcm16(data: np.ndarray) -> np.ndarray:

@@ -328,16 +328,18 @@ class Decoder:
                                              x.ctypes.data, y.ctypes.data))
         return y
 
-    def digitalize(self, envelope: np.ndarray):
+    def digitalize(self, envelope: np.ndarray, demodulated: bool = True):
         """median-5 + percentile stretch + rounding of a raw |hilbert| envelope
-        (wefax.py:175,196-216).  Returns ``(demodulated, digitalized, low_high, status)``."""
+        (wefax.py:175,196-216).  Returns ``(demodulated, digitalized, low_high, status)``;
+        ``demodulated=False`` skips the median-5 output (returned as None) and its host buffer."""
         e = np.ascontiguousarray(envelope, dtype=np.float32)
         batch = int(np.prod(e.shape[:-1])) if e.ndim > 1 else 1
-        dem = np.empty_like(e)
+        dem = np.empty_like(e) if demodulated else None
         dig = np.empty(e.shape, dtype=np.uint8)
         lh = np.zeros((batch, 2), dtype=np.float64)
         st = np.zeros(batch, dtype=np.int32)
-        self._check(self._lib.wefax_digitalize(self._h, e.shape[-1], batch, e.ctypes.data, dem.ctypes.data,
+        self._check(self._lib.wefax_digitalize(self._h, e.shape[-1], batch, e.ctypes.data,
+                                               C.c_void_p(dem.ctypes.data if dem is not None else None),
                                                dig.ctypes.data, lh.ctypes.data, st.ctypes.data))
         return dem, dig, lh, st
 

@@ -432,6 +432,45 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
                                  int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
                                  float *grey);
 
+/* ---- tuning offset of each chart from its phasing lines (DESIGN.md 4.7d) --------------------------------------------
+ * A receiver mistuned by D Hz moves every grey value by D / (white_hz - black_hz).  For each chart with a picture, with
+ * s its line start, Ls its line length (the slant fit's under AUTO slant), wb = max(1, round(0.05 Ls)), e = ceil(wb / 4)
+ * and end = min(n_out, image_end), the samples i = s + floor(l * Ls + o) of lines l < fold_lines that lie in [0, end)
+ * form two sets: the pulse, o in [e, wb - e), and the body, o in [wb + e, floor(Ls) - e).  b and w are the lower
+ * medians (element floor((m - 1) / 2) in ascending order) of the unclipped grey over the body and the pulse; d = (b +
+ * w) / 2 - 0.5.  Status OK when both sets hold samples, w - b is within [0.75, 1.25] and |d (white_hz - black_hz)| <=
+ * max_offset_hz: the picture is then made of clip(grey - (float)d), a shift with no stretch (the discriminator's scale
+ * is exact; noise pulls the measured levels toward the band centre, so the span is not a measure of it).  Otherwise the
+ * picture is the uncorrected one.  The grey stream and the tone scores are never corrected. */
+#define WEFAX_FM_LEVELS_OFF 0
+#define WEFAX_FM_LEVELS_AUTO 1
+#define WEFAX_FM_LEVELS_OK 0
+#define WEFAX_FM_LEVELS_NOT_FOUND 1      /* measured, failed the checks: picture uncorrected */
+#define WEFAX_FM_LEVELS_NOT_MEASURED 2   /* mode OFF, or the chart got no picture            */
+#define WEFAX_FM_LEVELS_MAX_OFFSET_HZ 300.0
+
+typedef struct {
+    int mode;                 /* WEFAX_FM_LEVELS_*                                                                */
+    double max_offset_hz;     /* largest offset corrected, (0, WEFAX_FM_LEVELS_MAX_OFFSET_HZ]; 0 = 200          */
+} wefax_fm_levels;
+
+typedef struct {
+    double black_hz, white_hz, offset_hz;   /* measured (NaN from an empty set); offset_hz is applied only when status
+                                               is OK; all 0 when not measured                                   */
+    int64_t black_samples, white_samples;   /* samples in the body and the pulse set                              */
+    int32_t status;                         /* WEFAX_FM_LEVELS_*                                                  */
+} wefax_fm_levels_out;
+
+/* wefax_decode_fm_charts_batch with the tuning offset measured and corrected per chart (levels: HOST pointer, not
+ * NULL; a bad mode or max_offset_hz is WEFAX_ERR_INVALID).  levels_out: HOST array laid out like charts
+ * (n_recordings x max_charts), or NULL.  With mode OFF every output equals wefax_decode_fm_charts_batch's, which is
+ * this call with mode OFF and levels_out NULL.  AUTO adds one launch per wave with pictures and no synchronisation. */
+int wefax_decode_fm_charts_levels(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                                  const wefax_fm_chart_params *params, const wefax_fm_levels *levels,
+                                  wefax_fm_chart *charts, wefax_fm_levels_out *levels_out, int max_charts,
+                                  int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
+                                  float *grey);
+
 #ifdef __cplusplus
 }
 #endif

@@ -30,7 +30,7 @@ EXPORTED_SYMBOLS = (
     "wefax_segment_envelope", "wefax_segment_histogram", "wefax_segment_quantise", "wefax_segment_sync",
     "wefax_segment_raster", "wefax_sync_pulse_scan", "wefax_segment_select_init", "wefax_segment_histogram_dev",
     "wefax_segment_select_dev", "wefax_segment_quantise_dev", "wefax_decode_fm_slant", "wefax_decode_fm_charts",
-    "wefax_decode_fm_charts_batch",
+    "wefax_decode_fm_charts_batch", "wefax_decode_fm_charts_levels",
 )
 ABI_VERSION = 5
 
@@ -117,6 +117,20 @@ class FmChart(C.Structure):
                 ("image_offset", C.c_int64), ("slant", FmSlantOut)]
 
 
+FM_LEVELS_OFF, FM_LEVELS_AUTO = 0, 1
+FM_LEVELS_OK, FM_LEVELS_NOT_FOUND, FM_LEVELS_NOT_MEASURED = 0, 1, 2
+FM_LEVELS_MAX_OFFSET_HZ = 300.0
+
+
+class FmLevels(C.Structure):
+    _fields_ = [("mode", C.c_int), ("max_offset_hz", C.c_double)]
+
+
+class FmLevelsOut(C.Structure):
+    _fields_ = [("black_hz", C.c_double), ("white_hz", C.c_double), ("offset_hz", C.c_double),
+                ("black_samples", C.c_int64), ("white_samples", C.c_int64), ("status", C.c_int32)]
+
+
 class NativeLibraryMissing(RuntimeError):
     pass
 
@@ -195,6 +209,9 @@ def load():
     lib.wefax_decode_fm_charts_batch.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmChartParams), vp, i, vp,
                                                  vp, ll, vp, vp]
     lib.wefax_decode_fm_charts_batch.restype = i
+    lib.wefax_decode_fm_charts_levels.argtypes = [vp, C.POINTER(BatchDesc), vp, C.POINTER(FmChartParams),
+                                                  C.POINTER(FmLevels), vp, vp, i, vp, vp, ll, vp, vp]
+    lib.wefax_decode_fm_charts_levels.restype = i
     lib.wefax_segment_envelope.argtypes = [vp, C.POINTER(BatchDesc), vp, ll, ll, ll, ll]
     lib.wefax_segment_envelope.restype = i
     lib.wefax_segment_histogram.argtypes = [vp, i, C.POINTER(C.c_uint32 * 4), vp]

@@ -543,24 +543,31 @@ struct FmTail {
     int rows = 0;
     long long offset = 0;      // of its picture from d_img (fm_tail)
     wefax_fm_slant_out so;
+    wefax_fm_levels_out lv;    // tuning offset (NOT_MEASURED unless the levels mode is AUTO)
 };
 
 // The picture stage of every chart in cs, each launch once over one chart table (DESIGN.md §4.7c):
 //   AUTO: coarse sheared fold of each chart's first Lc lines, per-line pulse tracking, robust line fit (twice: Lc
 //         lines, then all L lines from the first fit), three synchronisations for all charts together; a chart whose
 //         search finds too few pulses or leaves +-max_ppm keeps its phasing line start (status NOT_FOUND);
-//   the phasing fold of every chart without a fitted line; one synchronisation for all line starts;
-//   packed picture offsets from d_img on (rows * W bytes each); one image launch.
+//   the phasing fold of every chart without a fitted line; levels AUTO: every chart's black and white levels from its
+//   line start (DESIGN.md §4.7d); one synchronisation for all line starts and levels;
+//   packed picture offsets from d_img on (rows * W bytes each), each chart's tuning shift; one image launch.
 // Returns the bytes of pictures written to d_img (device); the image launch may still be running.
-long long fm_tail(wefax_ctx *ctx, std::vector<FmTail> &cs, int fold_lines, const wefax_fm_slant &sp, uint8_t *d_img) {
+long long fm_tail(wefax_ctx *ctx, std::vector<FmTail> &cs, const wefax_fm_params &prm, const wefax_fm_slant &sp,
+                  const wefax_fm_levels &lv, uint8_t *d_img) {
     cudaStream_t st = ctx->stream;
     const int nc = (int)cs.size();
     if (nc == 0) return 0;
+    const int fold_lines = prm.fold_lines;
+    const bool levels = lv.mode == WEFAX_FM_LEVELS_AUTO;
     std::vector<FmChartJob> tab(nc);
     int max_lc = 0;
     for (int i = 0; i < nc; ++i) {
         FmTail &c = cs[i];
         FmChartJob &j = tab[i];
+        memset(&c.lv, 0, sizeof(c.lv));
+        c.lv.status = WEFAX_FM_LEVELS_NOT_MEASURED;
         memset(&j, 0, sizeof(j));
         j.g = c.g;
         j.n = c.n;
@@ -576,11 +583,14 @@ long long fm_tail(wefax_ctx *ctx, std::vector<FmTail> &cs, int fold_lines, const
     }
     const size_t tab_bytes = ((size_t)nc * sizeof(FmChartJob) + 255) / 256 * 256;
     const size_t key_bytes = ((size_t)nc * sizeof(long long) + 255) / 256 * 256;
-    char *dev = (char *)ctx->out_small.reserve(tab_bytes + 2 * key_bytes + (size_t)nc * max_lc * sizeof(float));
+    const size_t lev_bytes = ((size_t)2 * nc * sizeof(FmLevel) + 255) / 256 * 256;
+    char *dev = (char *)ctx->out_small.reserve(tab_bytes + 2 * key_bytes + lev_bytes +
+                                               (size_t)nc * max_lc * sizeof(float));
     FmChartJob *d_tab = (FmChartJob *)dev;
     long long *d_ls = (long long *)(dev + tab_bytes);
     unsigned long long *d_best = (unsigned long long *)(dev + tab_bytes + key_bytes);
-    float *P = (float *)(dev + tab_bytes + 2 * key_bytes);
+    FmLevel *d_lev = (FmLevel *)(dev + tab_bytes + 2 * key_bytes);
+    float *P = (float *)(dev + tab_bytes + 2 * key_bytes + lev_bytes);
     // (pageable source: the copy is staged before the call returns, so the host table may change right after it)
     auto upload = [&] {
         CUDA_CHECK(cudaMemcpyAsync(d_tab, tab.data(), (size_t)nc * sizeof(FmChartJob), cudaMemcpyHostToDevice, st));
@@ -688,15 +698,33 @@ long long fm_tail(wefax_ctx *ctx, std::vector<FmTail> &cs, int fold_lines, const
     upload();
     CUDA_CHECK(cudaMemcpyAsync(d_ls, ls0.data(), (size_t)nc * sizeof(long long), cudaMemcpyHostToDevice, st));
     launch_fm_phasing(ctx, d_tab, tab.data(), nc, fold_lines, P, d_ls);
-    long long *h_ls = (long long *)pinned(ctx, (size_t)nc * sizeof(long long) + 64);
+    if (levels) launch_fm_levels(ctx, d_tab, nc, fold_lines, d_ls, d_lev);
+    long long *h_ls = (long long *)pinned(ctx, (size_t)nc * sizeof(long long) + (size_t)2 * nc * sizeof(FmLevel) + 64);
+    FmLevel *h_lev = (FmLevel *)(h_ls + nc);
     CUDA_CHECK(cudaMemcpyAsync(h_ls, d_ls, (size_t)nc * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    if (levels) CUDA_CHECK(cudaMemcpyAsync(h_lev, d_lev, (size_t)2 * nc * sizeof(FmLevel), cudaMemcpyDeviceToHost, st));
     CUDA_CHECK(cudaStreamSynchronize(st));
 
-    // rows and packed offsets, then every picture in one launch
+    // rows, packed offsets and tuning shifts, then every picture in one launch
+    const double span = prm.white_hz - prm.black_hz;
     long long off = 0;
     for (int i = 0; i < nc; ++i) {
         FmTail &c = cs[i];
         const double line_length = tab[i].Ls;
+        if (levels) {
+            const FmLevel &body = h_lev[2 * i], &pulse = h_lev[2 * i + 1];
+            const double b = body.value, w = pulse.value, delta = (b + w) / 2.0 - 0.5;
+            wefax_fm_levels_out &o = c.lv;
+            o.black_hz = prm.black_hz + b * span;
+            o.white_hz = prm.black_hz + w * span;
+            o.offset_hz = delta * span;
+            o.black_samples = body.count;
+            o.white_samples = pulse.count;
+            const bool ok = body.count > 0 && pulse.count > 0 && w - b >= 0.75 && w - b <= 1.25 &&
+                            fabs(o.offset_hz) <= lv.max_offset_hz;
+            o.status = ok ? WEFAX_FM_LEVELS_OK : WEFAX_FM_LEVELS_NOT_FOUND;
+            if (ok) tab[i].shift = (float)delta;
+        }
         c.line_start = h_ls[i];
         c.rows = (int)std::min<long long>(
             c.fg.rows_max, std::max<long long>(0, (long long)floor((double)(c.image_end - c.line_start) / line_length)));
@@ -1693,7 +1721,8 @@ int wefax_decode_fm_slant(wefax_ctx *ctx, const wefax_batch_desc *desc, const in
         uint8_t *d_img = nullptr;
         if (out->image && fg.rows_max > 0)
             d_img = out_dev ? out->image : (uint8_t *)ctx->out_raster.reserve((size_t)fg.rows_max * fg.W);
-        const long long bytes = fm_tail(ctx, cs, prm->fold_lines, sp, d_img);
+        const wefax_fm_levels off = {WEFAX_FM_LEVELS_OFF, 200.0};
+        const long long bytes = fm_tail(ctx, cs, *prm, sp, off, d_img);
         if (!out_dev && bytes > 0)
             CUDA_CHECK(cudaMemcpyAsync(out->image, d_img, (size_t)bytes, cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaStreamSynchronize(st));
@@ -1717,9 +1746,19 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
                                  const wefax_fm_chart_params *params, wefax_fm_chart *charts, int max_charts,
                                  int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
                                  float *grey) {
+    const wefax_fm_levels off = {WEFAX_FM_LEVELS_OFF, 0.0};
+    return wefax_decode_fm_charts_levels(ctx, desc, pcm, params, &off, charts, nullptr, max_charts, n_charts, images,
+                                         image_capacity, tone_scores, grey);
+}
+
+int wefax_decode_fm_charts_levels(wefax_ctx *ctx, const wefax_batch_desc *desc, const int16_t *pcm,
+                                  const wefax_fm_chart_params *params, const wefax_fm_levels *levels,
+                                  wefax_fm_chart *charts, wefax_fm_levels_out *levels_out, int max_charts,
+                                  int *n_charts, uint8_t *images, long long image_capacity, float *tone_scores,
+                                  float *grey) {
     if (!ctx) return WEFAX_ERR_INVALID;
     return guarded(ctx, [&] {
-        if (!desc || !pcm || !params || !n_charts || max_charts < 0 || (max_charts > 0 && !charts) ||
+        if (!desc || !pcm || !params || !levels || !n_charts || max_charts < 0 || (max_charts > 0 && !charts) ||
             desc->n_recordings < 1 || desc->n_frames < 64 || (desc->channels != 1 && desc->channels != 2) ||
             desc->sample_rate < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad argument");
@@ -1727,6 +1766,12 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
         if (!(prm.lpm >= 0.0) || prm.ioc < 0 || !(prm.white_hz > prm.black_hz) || prm.fold_lines < 1)
             WEFAX_THROW(WEFAX_ERR_INVALID, "bad FM parameters");
         const wefax_fm_slant sp = checked_slant(params->slant);
+        wefax_fm_levels lv = *levels;
+        if (lv.mode != WEFAX_FM_LEVELS_OFF && lv.mode != WEFAX_FM_LEVELS_AUTO)
+            WEFAX_THROW(WEFAX_ERR_INVALID, "unknown levels mode %d", lv.mode);
+        if (lv.max_offset_hz == 0.0) lv.max_offset_hz = 200.0;
+        if (!(lv.max_offset_hz > 0.0 && lv.max_offset_hz <= WEFAX_FM_LEVELS_MAX_OFFSET_HZ))
+            WEFAX_THROW(WEFAX_ERR_INVALID, "max_offset_hz must be in (0, %g]", WEFAX_FM_LEVELS_MAX_OFFSET_HZ);
         static const double kStandardLpm[] = {60.0, 90.0, 100.0, 120.0, 180.0, 240.0};
         const int n_cand = params->n_lpm_candidates ? params->n_lpm_candidates : 6;
         const double *cand_lpm = params->n_lpm_candidates ? params->lpm_candidates : kStandardLpm;
@@ -1851,7 +1896,7 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
             long long bytes = 0;
             if (!too_small && !cs.empty()) {
                 uint8_t *d_img = out_dev ? images + img_off : (uint8_t *)ctx->out_raster.reserve((size_t)wave_need + 1);
-                bytes = fm_tail(ctx, cs, prm.fold_lines, sp, d_img);
+                bytes = fm_tail(ctx, cs, prm, sp, lv, d_img);
                 if (!out_dev && bytes > 0)
                     CUDA_CHECK(cudaMemcpyAsync(images + img_off, d_img, (size_t)bytes, cudaMemcpyDeviceToHost, st));
             }
@@ -1861,6 +1906,9 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
             for (int r = 0; r < gw; ++r)
                 for (size_t i = 0; i < found[r].size(); ++i) {
                     wefax_fm_chart &c = found[r][i];
+                    wefax_fm_levels_out lo;
+                    memset(&lo, 0, sizeof(lo));
+                    lo.status = WEFAX_FM_LEVELS_NOT_MEASURED;
                     c.image_offset = off;
                     if (images && c.status == WEFAX_FM_CHART_OK && !too_small) {
                         const FmTail &p = cs[t++];
@@ -1868,9 +1916,11 @@ int wefax_decode_fm_charts_batch(wefax_ctx *ctx, const wefax_batch_desc *desc, c
                         c.rows = p.rows;
                         c.line_start = p.line_start;
                         c.slant = p.so;
+                        lo = p.lv;
                         off = c.image_offset + (long long)p.rows * p.fg.W;
                     }
                     charts[(size_t)(w0 + r) * max_charts + i] = c;
+                    if (levels_out) levels_out[(size_t)(w0 + r) * max_charts + i] = lo;
                 }
             img_off += bytes;
         }

@@ -18,6 +18,8 @@
 //                one thread per pixel: demod -> grey map -> line resample in one pass over x, y
 //   slant        (optional) the recording's true line length from the white line pulses: sheared folds of a
 //                binned profile, per-line pulse tracking, a line fit on the host (api.cu; DESIGN.md §4.7a)
+//   levels       (optional) each chart's tuning offset: lower medians of the grey over the phasing lines' body and
+//                pulse, the picture shifted by their midpoint's distance from 0.5 (DESIGN.md §4.7d)
 #include <cmath>
 #include <vector>
 
@@ -151,10 +153,10 @@ fm_phase_kernel(const FmChartJob *tab, const float *P, int ps, long long *line_s
     }
 }
 
-// pixel (r, p): box average of clip(grey) over [a, a + Ls / W), a = line_start + r * Ls + p * Ls / W.
+// pixel (r, p): box average of clip(grey - shift) over [a, a + Ls / W), a = line_start + r * Ls + p * Ls / W.
 // rows = min(rows_max, floor((image_end - line_start) / Ls)), the host's expression (wefax_decode_fm_slant), so
 // every row the caller is told about is written; grid.y strides over the rows (it is capped at 65535), grid.z is the
-// chart of the table, grid.x covers the widest picture
+// chart of the table, grid.x covers the widest picture.  shift = 0 leaves every grey value as it is (g - 0.f == g).
 __global__ void __launch_bounds__(256)
 fm_image_kernel(const FmChartJob *tab, const long long *line_start, uint8_t *img) {
     const FmChartJob &job = tab[blockIdx.z];
@@ -162,6 +164,7 @@ fm_image_kernel(const FmChartJob *tab, const long long *line_start, uint8_t *img
     const int W = job.W, rows_max = job.rows_max;
     if (p >= W || rows_max <= 0) return;
     const float *g = job.g;
+    const float shift = job.shift;
     const long long n = job.n, image_end = job.image_end;
     const double Ls = job.Ls;
     img += job.out;
@@ -176,10 +179,104 @@ fm_image_kernel(const FmChartJob *tab, const long long *line_start, uint8_t *img
         for (long long i = i0; i < i1; ++i) {
             const double lo = fmax(a, (double)i), hi = fmin(b, (double)(i + 1));
             const float wgt = (float)(hi - lo);
-            if (i >= 0 && i < n && wgt > 0.f) acc = fmaf(wgt, clip01(__ldg(g + i)), acc);
+            if (i >= 0 && i < n && wgt > 0.f) acc = fmaf(wgt, clip01(__ldg(g + i) - shift), acc);
         }
         const float v = rintf(255.f * acc / (float)step);
         img[(size_t)r * W + p] = (uint8_t)fminf(fmaxf(v, 0.f), 255.f);
+    }
+}
+
+// ---- tuning offset: the black and white levels of the phasing lines (DESIGN.md §4.7d) ----
+
+// order-preserving key: a < b as floats <=> key(a) < key(b) as unsigned integers (NaN aside)
+__device__ __forceinline__ unsigned int float_key(float v) {
+    const unsigned int u = __float_as_uint(v);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key_float(unsigned int k) {
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// One CTA per (set, chart): blockIdx.x = 0 is the body set, offsets o in [wb + e, floor(Ls) - e); 1 is the pulse set,
+// o in [e, wb - e); e = ceil(wb / 4).  Its samples are i = s + floor(l * Ls + o) for lines l < lines (fm_fold_kernel's
+// rounding), s = line_start[chart], kept where 0 <= i < min(n, image_end).  Out: the lower median of their unclipped
+// grey (element floor((m - 1) / 2) of the m values in ascending order) and m.  The median is an exact radix select
+// over the order-preserving keys, 11, 11 and 10 bits, each pass walking the set again (it is read from L2).
+constexpr int kLevelsThreads = 1024;
+__global__ void __launch_bounds__(kLevelsThreads)
+fm_levels_kernel(const FmChartJob *tab, int lines, const long long *line_start, FmLevel *lev) {
+    __shared__ unsigned int hist[2048];
+    __shared__ unsigned int s_warp[kLevelsThreads / 32];
+    __shared__ unsigned int s_prefix, s_rank;
+    const FmChartJob &job = tab[blockIdx.y];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *g = job.g;
+    const double Ls = job.Ls;
+    const int wb = job.wb, e = (wb + 3) / 4;
+    const int o0 = blockIdx.x == 0 ? wb + e : e;
+    const int o1 = blockIdx.x == 0 ? (int)floor(Ls) - e : wb - e;
+    const long long s = line_start[blockIdx.y], end = min(job.n, job.image_end);
+    // line l starts at or after s + l * Ls - 1: the lines past this bound hold no sample below end
+    const long long ln = end > s ? min((long long)lines, (long long)floor((double)(end - s) / Ls) + 2) : 0;
+    lev += 2 * (size_t)blockIdx.y + blockIdx.x;
+    unsigned int prefix = 0u, rank = 0u, count = 0u;
+    for (int pass = 0; pass < 3; ++pass) {
+        const int shift = pass == 0 ? 21 : (pass == 1 ? 10 : 0);
+        const unsigned int digit = pass == 2 ? 0x3ffu : 0x7ffu;
+        const unsigned int chosen = pass == 0 ? 0u : (pass == 1 ? 0xffe00000u : 0xfffffc00u);   // bits already found
+        for (int b = tid; b < 2048; b += kLevelsThreads) hist[b] = 0u;
+        __syncthreads();
+        for (long long l = 0; l < ln; ++l) {
+            const double base = __dmul_rn((double)l, Ls);
+            for (int o = o0 + tid; o < o1; o += kLevelsThreads) {
+                const long long i = s + (long long)floor(__dadd_rn(base, (double)o));
+                if (i < 0 || i >= end) continue;
+                const unsigned int k = float_key(__ldg(g + i));
+                if ((k & chosen) == prefix) atomicAdd(&hist[(k >> shift) & digit], 1u);
+            }
+        }
+        __syncthreads();
+        // exclusive scan of the bins, two per thread: the bin holding the rank extends the prefix
+        const unsigned int h0 = hist[2 * tid], h1 = hist[2 * tid + 1], mine = h0 + h1;
+        unsigned int incl = mine;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const unsigned int v = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += v;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            unsigned int w = s_warp[lane];
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const unsigned int v = __shfl_up_sync(0xffffffffu, w, d);
+                if (lane >= d) w += v;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        if (pass == 0) {
+            count = s_warp[kLevelsThreads / 32 - 1];
+            if (count == 0u) break;     // (every thread sees the same count)
+            rank = (count - 1u) / 2u;
+        }
+        const unsigned int start = (warp ? s_warp[warp - 1] : 0u) + incl - mine;
+        if (rank >= start && rank < start + h0) {
+            s_prefix = prefix | ((unsigned int)(2 * tid) << shift);
+            s_rank = rank - start;
+        } else if (rank >= start + h0 && rank < start + mine) {
+            s_prefix = prefix | ((unsigned int)(2 * tid + 1) << shift);
+            s_rank = rank - start - h0;
+        }
+        __syncthreads();
+        prefix = s_prefix;
+        rank = s_rank;
+    }
+    if (tid == 0) {
+        lev->value = count ? key_float(prefix) : __int_as_float(0x7fc00000);
+        lev->pad = 0;
+        lev->count = (long long)count;
     }
 }
 
@@ -485,6 +582,15 @@ void launch_fm_phasing(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob
     fm_phase_kernel<<<n_charts, 1024, smem, ctx->stream>>>(d_tab, P, Lc, d_line_start);
     CUDA_CHECK(cudaGetLastError());
     ctx->launches += 2;
+}
+
+void launch_fm_levels(wefax_ctx *ctx, const FmChartJob *d_tab, int n_charts, int lines, const long long *d_line_start,
+                      FmLevel *lev) {
+    if (n_charts <= 0) return;
+    StageTimer timer(ctx, "fm_levels");
+    fm_levels_kernel<<<dim3(2, n_charts), kLevelsThreads, 0, ctx->stream>>>(d_tab, lines, d_line_start, lev);
+    CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
 }
 
 void launch_fm_image(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,

@@ -143,6 +143,7 @@ struct FmChartJob {
     int phase;              // 1: line start from the phasing fold; 0: given (the slant fit)
     int W, rows_max;        // picture: W pixels per row, rows_max rows at most (0: no picture)
     long long out;          // offset (bytes) of the picture in the output
+    float shift;            // picture of clip(grey - shift): the measured tuning offset in grey units (0: none)
     // slant search (AUTO): profile of q_lines lines of the nominal line sLs in Bn bins of D samples (Q from q_off),
     // n_cand sheared folds; pulse tracking of track_lines lines around a + l * s (pos / contrast from pos_off)
     double sLs, a, s;
@@ -152,6 +153,16 @@ struct FmChartJob {
 // line start of every chart with phase = 1 into d_line_start[chart]: the fold of `lines` lines (P: max Lc floats per chart)
 void launch_fm_phasing(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts, int lines,
                        float *P, long long *d_line_start);
+// tuning offset (DESIGN.md §4.7d): lower median of the unclipped grey over each chart's pulse and body sets of its first
+// `lines` lines from d_line_start[chart] (Ls, wb; samples below min(n, image_end)), one (value, count) per set
+struct FmLevel {
+    float value;            // the order statistic (NaN when the set is empty)
+    int pad;
+    long long count;        // samples in the set
+};
+// lev[2 * chart] = body (black), lev[2 * chart + 1] = pulse (white)
+void launch_fm_levels(wefax_ctx *ctx, const FmChartJob *d_tab, int n_charts, int lines, const long long *d_line_start,
+                      FmLevel *lev);
 // every chart's picture (rows_max > 0) into img + out
 void launch_fm_image(wefax_ctx *ctx, const FmChartJob *d_tab, const FmChartJob *h_tab, int n_charts,
                      const long long *d_line_start, uint8_t *img);

@@ -42,6 +42,21 @@ class FmSlant:
 
 
 @dataclass
+class FmLevels:
+    """A chart's tuning offset, measured from its phasing lines (``wefax_fm_levels_out``)."""
+    black_hz: float            # measured black level (NaN when the body set is empty)
+    white_hz: float            # measured white level (NaN when the pulse set is empty)
+    offset_hz: float           # (black_hz + white_hz) / 2 minus the centre of the grey scale (1900 Hz by default)
+    black_samples: int         # samples the black level is the lower median of
+    white_samples: int         # samples the white level is the lower median of
+    status: int                # N.FM_LEVELS_OK (picture corrected by offset_hz), N.FM_LEVELS_NOT_FOUND (uncorrected)
+
+    @property
+    def found(self) -> bool:
+        return self.status == N.FM_LEVELS_OK
+
+
+@dataclass
 class FmResult:
     image: np.ndarray          # (rows, width) uint8, 0 = black (1500 Hz), 255 = white (2300 Hz)
     line_start: int            # sample (at 11025 Hz) of the first image row
@@ -67,6 +82,7 @@ class FmChart:
     line_start: int            # sample of the first picture line (-1: no picture decoded)
     image: np.ndarray | None   # (rows, width) uint8; None when pictures were not asked for or status is not OK
     slant: FmSlant | None = None
+    levels: FmLevels | None = None      # with levels="auto", when the chart has a picture
 
 
 @dataclass
@@ -187,6 +203,17 @@ def chart_params(lpm=None, ioc=None, lpm_candidates=None, slant=None, max_slant_
     return N.FmChartParams(prm, sp, len(cands), arr)
 
 
+def levels_params(levels=None, max_offset_hz: float = 200.0):
+    """``N.FmLevels`` for ``levels`` = None (no correction) or ``"auto"`` (measure each chart's tuning offset from its
+    phasing lines and correct it when it is within +-``max_offset_hz``); ValueError for anything else."""
+    if levels is not None and levels != "auto":
+        raise ValueError(f"levels must be None or 'auto', not {levels!r}")
+    if isinstance(max_offset_hz, bool) or not isinstance(max_offset_hz, numbers.Real) or \
+            not 0.0 < float(max_offset_hz) <= N.FM_LEVELS_MAX_OFFSET_HZ:
+        raise ValueError(f"max_offset_hz must be in (0, {N.FM_LEVELS_MAX_OFFSET_HZ:g}], not {max_offset_hz!r}")
+    return N.FmLevels(N.FM_LEVELS_OFF if levels is None else N.FM_LEVELS_AUTO, float(max_offset_hz))
+
+
 def _max_charts(max_charts):
     if isinstance(max_charts, bool) or not isinstance(max_charts, numbers.Integral) or max_charts < 0:
         raise ValueError(f"max_charts must be a non-negative integer, not {max_charts!r}")
@@ -204,17 +231,20 @@ def _image_bound(prm, lpm, ioc, n_out: int) -> int:
     return int(math.ceil(n_out / ls_min)) * w_max
 
 
-def _charts(out, n_found: int, max_charts: int, img, prm) -> list:
-    """FmChart of the native chart entries ``out`` (pictures cut from ``img``, None when pictures were not asked for)."""
+def _charts(out, lev, n_found: int, max_charts: int, img, prm) -> list:
+    """FmChart of the native chart entries ``out`` and their levels ``lev`` (pictures cut from ``img``, None when
+    pictures were not asked for)."""
     charts = []
-    for c in out[: min(n_found, max_charts)]:
+    for c, lo in zip(out[: min(n_found, max_charts)], lev):
         decoded = img is not None and c.status == N.FM_CHART_OK
         picture = img[c.image_offset: c.image_offset + c.rows * c.width].reshape(c.rows, c.width) if decoded else None
         so = FmSlant(**{name: getattr(c.slant, name) for name, _ in N.FmSlantOut._fields_}) \
             if (decoded and prm.slant.mode != N.FM_SLANT_OFF) else None
+        lv = FmLevels(**{name: getattr(lo, name) for name, _ in N.FmLevelsOut._fields_}) \
+            if lo.status != N.FM_LEVELS_NOT_MEASURED else None
         charts.append(FmChart(int(c.tone_begin), int(c.search_from), int(c.image_end), bool(c.stop_found), int(c.ioc),
                               float(c.lpm), float(c.lpm_score), int(c.status), int(c.width), int(c.line_start),
-                              picture, so))
+                              picture, so, lv))
     return charts
 
 
@@ -222,7 +252,7 @@ def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_can
                      max_slant_ppm: float = 300.0, max_charts: int = 64, fold_lines: int = 20,
                      black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0), fir_taps: int = 63,
                      want_images: bool = True, want_grey: bool = False, want_tone_scores: bool = False,
-                     image_capacity: int | None = None) -> FmCharts:
+                     image_capacity: int | None = None, levels=None, max_offset_hz: float = 200.0) -> FmCharts:
     """Find and decode every chart of a recording (int16 numpy, mono ``(n,)`` or stereo ``(n, 2)``).
 
     Each chart starts at a start tone (300 Hz: IOC 576, 675 Hz: IOC 288) and ends at the stop tone, the next start
@@ -230,8 +260,11 @@ def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_can
     fold shows the sharpest line pulse.  ``lpm`` / ``ioc`` force a value for every chart.  ``slant`` as for
     :func:`decode_fm`, for every chart.  Each chart's picture equals ``decode_fm`` with that chart's lpm, ioc,
     search_from and image_end.  ``want_images=False`` returns the chart list only; ``image_capacity`` overrides the
-    size of the picture buffer (bytes; default: enough for any recording of this length)."""
+    size of the picture buffer (bytes; default: enough for any recording of this length).  ``levels="auto"`` measures
+    each decoded chart's tuning offset from its phasing lines (``chart.levels``) and, when it is found within
+    +-``max_offset_hz``, shifts the chart's grey levels by it (the grey stream and the tone scores stay uncorrected)."""
     prm = chart_params(lpm, ioc, lpm_candidates, slant, max_slant_ppm, fold_lines, black_hz, white_hz, band, fir_taps)
+    lvp = levels_params(levels, max_offset_hz)
     max_charts = _max_charts(max_charts)
     pcm = np.ascontiguousarray(pcm, dtype=np.int16)
     n_in, ch = int(pcm.shape[0]), (1 if pcm.ndim == 1 else int(pcm.shape[1]))
@@ -242,27 +275,31 @@ def decode_fm_charts(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_can
     grey = np.zeros(n_out, dtype=np.float32) if want_grey else None
     tones = np.zeros((n_out // N.FM_TONE_WINDOW, 4), dtype=np.float32) if want_tone_scores else None
     out = (N.FmChart * max(1, max_charts))()
+    lev = (N.FmLevelsOut * max(1, max_charts))()
     n_found = C.c_int(0)
     desc = N.BatchDesc(1, n_in, ch, int(sample_rate), 0.0, 0.0, 0)
-    decoder._check(decoder._lib.wefax_decode_fm_charts(
-        decoder._h, C.byref(desc), C.c_void_p(pcm.ctypes.data), C.byref(prm), out, int(max_charts), C.byref(n_found),
-        img.ctypes.data if want_images else None, int(image_capacity),
+    decoder._check(decoder._lib.wefax_decode_fm_charts_levels(
+        decoder._h, C.byref(desc), C.c_void_p(pcm.ctypes.data), C.byref(prm), C.byref(lvp), out, lev,
+        int(max_charts), C.byref(n_found), img.ctypes.data if want_images else None, int(image_capacity),
         tones.ctypes.data if want_tone_scores else None, grey.ctypes.data if want_grey else None))
-    return FmCharts(_charts(out, n_found.value, max_charts, img, prm), int(n_found.value), grey, tones)
+    return FmCharts(_charts(out, lev, n_found.value, max_charts, img, prm), int(n_found.value), grey, tones)
 
 
 def decode_fm_charts_batch(decoder, pcm, sample_rate: int, lpm=None, ioc=None, lpm_candidates=None, slant=None,
                            max_slant_ppm: float = 300.0, max_charts: int = 64, fold_lines: int = 20,
                            black_hz: float = 1500.0, white_hz: float = 2300.0, band=(1200.0, 2600.0),
                            fir_taps: int = 63, want_images: bool = True, want_grey: bool = False,
-                           want_tone_scores: bool = False, image_capacity: int | None = None) -> list:
+                           want_tone_scores: bool = False, image_capacity: int | None = None, levels=None,
+                           max_offset_hz: float = 200.0) -> list:
     """:func:`decode_fm_charts` of R recordings of equal length in one call (``wefax_decode_fm_charts_batch``): one
     FmCharts per recording, each what :func:`decode_fm_charts` returns for that recording alone.
 
     ``pcm``: int16 ``(R, n)`` mono or ``(R, n, 2)`` stereo, as numpy (host) or as a CUDA torch tensor (read in place on
     the device).  The outputs are numpy arrays on the host.  ``image_capacity`` is the byte size of the picture buffer
-    of the whole batch (default: R times the bound of :func:`decode_fm_charts`)."""
+    of the whole batch (default: R times the bound of :func:`decode_fm_charts`).  ``levels`` / ``max_offset_hz`` as
+    for :func:`decode_fm_charts`."""
     prm = chart_params(lpm, ioc, lpm_candidates, slant, max_slant_ppm, fold_lines, black_hz, white_hz, band, fir_taps)
+    lvp = levels_params(levels, max_offset_hz)
     max_charts = _max_charts(max_charts)
     if isinstance(sample_rate, bool) or not isinstance(sample_rate, numbers.Integral) or sample_rate < 1:
         raise ValueError(f"sample_rate must be a positive integer, not {sample_rate!r}")
@@ -286,16 +323,18 @@ def decode_fm_charts_batch(decoder, pcm, sample_rate: int, lpm=None, ioc=None, l
     grey = np.zeros((R, n_out), dtype=np.float32) if want_grey else None
     tones = np.zeros((R, n_out // N.FM_TONE_WINDOW, 4), dtype=np.float32) if want_tone_scores else None
     out = (N.FmChart * max(1, R * max_charts))()
+    lev = (N.FmLevelsOut * max(1, R * max_charts))()
     n_found = (C.c_int * R)()
     desc = N.BatchDesc(R, n_in, ch, int(sample_rate), 0.0, 0.0, flags)
-    decoder._check(decoder._lib.wefax_decode_fm_charts_batch(
-        decoder._h, C.byref(desc), C.c_void_p(ptr), C.byref(prm), out, max_charts, n_found,
+    decoder._check(decoder._lib.wefax_decode_fm_charts_levels(
+        decoder._h, C.byref(desc), C.c_void_p(ptr), C.byref(prm), C.byref(lvp), out, lev, max_charts, n_found,
         img.ctypes.data if want_images else None, int(image_capacity),
         tones.ctypes.data if want_tone_scores else None, grey.ctypes.data if want_grey else None))
     res = []
     for r in range(R):
         entries = out[r * max_charts: (r + 1) * max_charts]
-        res.append(FmCharts(_charts(entries, n_found[r], max_charts, img, prm), int(n_found[r]),
+        levs = lev[r * max_charts: (r + 1) * max_charts]
+        res.append(FmCharts(_charts(entries, levs, n_found[r], max_charts, img, prm), int(n_found[r]),
                             None if grey is None else grey[r], None if tones is None else tones[r]))
     return res
 
@@ -327,6 +366,10 @@ def main(argv=None) -> int:
     ap.add_argument("--slant", default=None, metavar="auto|PPM",
                     help="correct the sample-clock error: 'auto' measures it, a number gives it in ppm")
     ap.add_argument("--max-slant-ppm", type=float, default=300.0, help="largest error 'auto' searches (default 300)")
+    ap.add_argument("--levels", choices=["auto"], default=None,
+                    help="with --all: measure each chart's tuning offset from its phasing lines and correct its grey levels")
+    ap.add_argument("--max-offset-hz", type=float, default=200.0,
+                    help="largest tuning offset --levels auto corrects (default 200)")
     ap.add_argument("--device", type=int, default=0, help="CUDA device (default 0)")
     a = ap.parse_args(argv)
     slant = a.slant
@@ -335,8 +378,11 @@ def main(argv=None) -> int:
             slant = float(slant)
         except ValueError:
             ap.error(f"--slant takes 'auto' or a number, not {a.slant!r}")
+    if a.levels is not None and not a.all:
+        ap.error("--levels needs --all")
     try:
         slant_params(slant, a.max_slant_ppm)
+        levels_params(a.levels, a.max_offset_hz)
     except ValueError as e:
         ap.error(str(e))
 
@@ -374,7 +420,8 @@ def _main_all(a, slant, pcm, sample_rate, ap) -> int:
         ap.error(str(e))
     stem, ext = os.path.splitext(a.png)
     with Decoder(a.device) as dec:
-        res = decode_fm_charts(dec, pcm, sample_rate, lpm=a.lpm, ioc=a.ioc, slant=slant, max_slant_ppm=a.max_slant_ppm)
+        res = decode_fm_charts(dec, pcm, sample_rate, lpm=a.lpm, ioc=a.ioc, slant=slant, max_slant_ppm=a.max_slant_ppm,
+                               levels=a.levels, max_offset_hz=a.max_offset_hz)
     if res.n_found > len(res.charts):
         print(f"{res.n_found} charts found, the first {len(res.charts)} decoded")
     for k, c in enumerate(res.charts, 1):
@@ -388,6 +435,9 @@ def _main_all(a, slant, pcm, sample_rate, ap) -> int:
         line = f"{where}, LPM {c.lpm:g} (score {c.lpm_score:.2f}), {path}: {c.image.shape[0]} x {c.image.shape[1]}"
         if c.slant is not None:
             line += f", slant {c.slant.ppm:+.3f} ppm" if c.slant.found else ", slant not measured"
+        if a.levels is not None:
+            line += f", tuning offset {c.levels.offset_hz:+.1f} Hz" if (c.levels and c.levels.found) \
+                else ", tuning offset not measured"
         print(line)
     if not res.n_found:
         print("no chart found (no start tone of 2 s or more)")
